@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the AR scoring hot path (BASELINE.json metric: query windows/sec, 5-way 1-shot, T=16).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Headline workload (default, `--config cfg2`): a step = one pass of the hot path over one batch: BASELINE cfg2, 4096 synthetic
@@ -10,9 +10,9 @@ windows are independent and shard with no data-path collective; every step re-pr
 all-gathers the scores).  One JSON line (rank 0):
 
   value        device-timed (CUDA events on the launching stream, max over ranks), inputs resident in HBM, L2 flushed
-               between timed steps.  The timed region is `repeats` back-to-back blocks of EXACTLY K steps each (every
-               block bracketed by barrier + synchronize), enough blocks for >= 1 s of timed work; value = all windows / all
-               block times, so one scheduling hiccup in 8 ms of work no longer decides a scaling number.
+               between timed steps.  The timed region is EXACTLY K steps, bracketed by barrier + synchronize; value =
+               all windows / the summed step times.  At ~0.35 ms a step the default K=50 is ~17 ms of timed work, where
+               one scheduling hiccup can move the figure: for a stable number give K >= 3000 (>= 1 s).
   e2e          the same metric through the host-buffer C-ABI entry points, pinned H2D / D2H inside the timed region.
   sustained    >= 2 s of back-to-back steps over a ring of input batches larger than L2 (no flush), clocks sampled
                under load; attention roofline fraction against the SUSTAINED measured bf16 peak.
@@ -25,12 +25,16 @@ all-gathers the scores).  One JSON line (rank 0):
                box's host cores, bounded sample.
 
 `--impl reference` times that same CPU arm on the same config and prints the same line shape.
+
+`--dump-outputs DIR` (rank 0) writes what the last timed step returned to its caller -- the all-gathered logits (B*N, W)
+and is_true (B*N, 1) -- as DIR/logits.npy and DIR/is_true.npy (float32).  Inputs and weights come from fixed seeds, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import faulthandler
 import json
-import math
 import os
 import sys
 import threading
@@ -215,10 +219,14 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
-def teardown(torch, dist, world, graphs=()):
-    """CUDA graphs that captured NCCL kernels must be destroyed before the communicator; a teardown that still hangs (seen
-    once: destroy_process_group never returned after graph replays) must not turn a finished measurement into a timeout:
-    the result line is already printed and flushed, so a watchdog ends the process with exit code 0."""
+def teardown(torch, dist, world, graphs=(), models=()):
+    """Ends a run whose result line is printed: destroys the CUDA graphs (before the communicator: they captured NCCL
+    kernels) and the library handles (arx_destroy synchronises the device), then the process group, and returns, so the
+    process exits normally and its exit handlers run.  A hang must not turn the finished measurement into a timeout:
+    - during these steps (seen once: destroy_process_group never returned after graph replays) a timer thread ends the
+      process with exit code 0 after 20 s;
+    - during interpreter finalization a daemon thread can no longer run, so faulthandler's watchdog (a C thread) covers
+      it: after a further 30 s it prints every thread's stack to stderr and ends the process with exit code 1."""
     sys.stdout.flush()
     # (at N=1 too: one default run of round 2 printed its line and then never exited -- seen once in ~10 runs, not reproduced
     # under faulthandler; whatever finaliser it was, the measurement was complete)
@@ -228,6 +236,11 @@ def teardown(torch, dist, world, graphs=()):
     for g in graphs:
         try:
             g.reset()
+        except Exception:
+            pass
+    for m in models:
+        try:
+            m._release()
         except Exception:
             pass
     try:
@@ -240,9 +253,10 @@ def teardown(torch, dist, world, graphs=()):
             dist.destroy_process_group()
         except Exception:
             pass
+    t.cancel()
+    faulthandler.dump_traceback_later(30.0, exit=True)
     sys.stdout.flush()
     sys.stderr.flush()
-    os._exit(0)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -257,6 +271,26 @@ def timed_ms(torch, fn, reps, warm=2):
     b.record()
     torch.cuda.synchronize()
     return a.elapsed_time(b) / reps
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, per_rank):
+    """--dump-outputs: the last step's per-rank (logits, is_true) as d/logits.npy and d/is_true.npy, rows of all ranks in
+    rank order, float32.  Beyond DUMP_BYTES in all, both keep the same fixed, seeded sample of rows (in row order)."""
+    import numpy as np
+    import torch
+    arrays = {"logits": torch.cat([r[0] for r in per_rank]).cpu().numpy(),
+              "is_true": torch.cat([r[1] for r in per_rank]).cpu().numpy()}
+    n = arrays["logits"].shape[0]
+    row_bytes = 4 * sum(a.shape[1] for a in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def other_configs(torch, dev, peaks):
@@ -427,7 +461,7 @@ def cfg3_sharded(torch, dist, dev, world, rank, steps):
     return {"workload": f"60-way x 65536 windows, T=16 pairs, split contiguously over {world} rank(s); every step: support set on rank 0, NCCL "
                         "broadcast of the support tuple embeddings, shard scoring, all-gather of [logits | is_true]",
             "metric": "query windows/sec (60-way 1-shot, T=16)", "value": B / ms * 1e3, "ms_per_step": ms, "steps": steps, "scaling": "strong",
-            "attention_tflops_aggregate": tf, "gathered_scores_bit_identical_on_all_ranks": agree, "planted_class_recovered": ok}
+            "attention_tflops_aggregate": tf, "gathered_scores_bit_identical_on_all_ranks": agree, "planted_class_recovered": ok}, res
 
 
 def main():
@@ -441,14 +475,17 @@ def main():
     ap.add_argument("--force-path", type=int, default=0, help="0 auto, 1 fp32 kernels, 2 tcgen05 kernels")
     ap.add_argument("--chunk", type=int, default=0, help="windows per internal pass of arx_score (0 = library default)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    ap.add_argument("--min-timed-seconds", type=float, default=1.0, help="repeat the K-step block until this much timed work")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip sustained / other configs / cfg3 (headline numbers only)")
     ap.add_argument("--no-step-graph", action="store_true", help="launch every step eagerly instead of replaying one CUDA graph per step")
     ap.add_argument("--static-support", action="store_true",
                     help="diagnostic: set the support set once before timing instead of in every step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's logits / is_true as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -478,7 +515,9 @@ def main():
     if args.config == "cfg3":
         torch.cuda.set_stream(torch.cuda.Stream(device=dev))
         sampler = ClockSampler(local).start() if rank == 0 else None
-        r = cfg3_sharded(torch, dist, dev, world, rank, max(3, args.steps))
+        r, res = cfg3_sharded(torch, dist, dev, world, rank, args.steps)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, res)
         if rank == 0:
             line = {"metric": r["metric"], "value": r["value"], "unit": UNIT, "n_gpus": world, "steps": r["steps"], "warmup": 2,
                     "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f16",
@@ -612,11 +651,11 @@ def main():
             step_eager()
 
     def finish():
+        """Joins the last step; -> its per-rank (logits, is_true), as the caller of the step receives them."""
         if use_graph:
-            if world > 1:
-                gats[(step_no[0] - 1) & 1].gather()     # the last step's scores (every earlier gather rode inside the next graph)
-        else:
-            drain()
+            # the last step's scores (every earlier gather rode inside the next graph; no collective at N=1)
+            return gats[(step_no[0] - 1) & 1].gather()
+        return drain()
 
     for _ in range(args.warmup):
         flush.fill_(1)
@@ -634,28 +673,23 @@ def main():
             ev[k][0].record()
             step()
             if k == K - 1:
-                finish()                                # eager mode: the last collective is joined inside the last timed interval
+                last = finish()                         # eager mode: the last collective is joined inside the last timed interval
             ev[k][1].record()
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
-        return sum(a.elapsed_time(b) for a, b in ev)
+        return sum(a.elapsed_time(b) for a, b in ev), last
 
     sampler = ClockSampler(local)
     if rank == 0:            # one sampler per job: the ranks share few host cores
         sampler.start()
     l0 = model.launch_count()
-    first = timed_block(args.steps)
-    # every rank must run the same number of blocks: decide it from the slowest rank's first block
-    t = torch.tensor([first], dtype=torch.float64, device=dev)
-    if world > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    repeats = 1 if args.no_extras and args.min_timed_seconds <= 0 else max(1, min(400, int(math.ceil(args.min_timed_seconds * 1e3 / max(float(t[0]), 1e-3)))))
-    blocks = [first] + [timed_block(args.steps) for _ in range(repeats - 1)]
-    total_ms = sum(blocks)
-    n_steps_total = args.steps * repeats
+    total_ms, last = timed_block(args.steps)
+    n_steps_total = args.steps
     launches = (model.launch_count() - l0) + (launches_per_graph * n_steps_total if use_graph else 0)
     clocks = sampler.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
 
     # ---- stage timers: the same steps launched eagerly with CUDA events between the stages (arx_profile_*)
     model.profile(True)
@@ -779,7 +813,7 @@ def main():
     cfg3 = None
     if not args.no_extras:
         try:
-            cfg3 = cfg3_sharded(torch, dist, dev, world, rank, 5)
+            cfg3, _ = cfg3_sharded(torch, dist, dev, world, rank, 5)
         except Exception as e:
             cfg3 = {"error": repr(e)[:300]}
             if world > 1:
@@ -839,11 +873,10 @@ def main():
                            "launch": ("one CUDA graph per step (set_support + score; with N>1 the all-gather of the previous step's scores rides on a forked "
                                       "branch of the same graph, the last one is joined inside the last timed step)" if use_graph
                                       else "eager launches; the collective of batch k is joined after batch k+1 is scored"),
-                           "timing": f"CUDA events per step on the launching stream, summed over {repeats} blocks of exactly {args.steps} steps "
-                                     "(each block bracketed by barrier + synchronize); max over ranks; stage timers from a further pass of the same "
+                           "timing": f"CUDA events per step on the launching stream, summed over exactly {args.steps} steps "
+                                     "(bracketed by barrier + synchronize); max over ranks; stage timers from a further pass of the same "
                                      "steps launched eagerly with events between stages"},
-                "repeats": repeats, "timed_steps_total": n_steps_total, "timed_ms_total": total_ms,
-                "block_ms": {"first": blocks[0], "min": min(blocks), "max": max(blocks), "median": sorted(blocks)[len(blocks) // 2]},
+                "timed_steps_total": n_steps_total, "timed_ms_total": total_ms,
                 "clocks": clocks,
                 "e2e": {"value": e2e_val, "unit": UNIT, "h2d_bytes_per_step": world * B * T * J3 * 4,
                         "d2h_bytes_per_step": world * B * (WAY + 1) * 4, "steps": e2e_steps,
@@ -857,7 +890,7 @@ def main():
                 "gpu_launches": int(launches), "roofline": roofline, "roofline_per_kernel": per_kernel, "sustained": sustained,
                 "cfg3": cfg3, "other_configs": extras, "cpu_baseline": cpu, "parity_check_max_rel_err": err}
         print(json.dumps(line), flush=True)
-    teardown(torch, dist, world, [g for g in graph_steps if g is not None])
+    teardown(torch, dist, world, [g for g in graph_steps if g is not None], [model])
 
 
 if __name__ == "__main__":
