@@ -224,7 +224,9 @@ ARX_API int arx_profile_read(arx_handle *h, double *ms, int64_t *chunks, int32_t
  *         the frame MLP, 2048 head projection on the caller's stream, 4096 T=16 pair tuples on the tiled any-N kernels.
  *         8192 frame MLP as three launches (pose image, fc1, fc2) instead of the fused kernel, 16384 no L2 prefetch ahead of the
  *         head kernel's operand ring, 32768 the persistent front-end kernels take every SM even while a support chain is in flight.
- *         Bits 4 and 4096 select which support operands are built: set them BEFORE the support set.
+ *         Bits 4 and 4096 choose the kernels of the T=16 pairs when the support set is built (they decide which support
+ *         operands are built): set them BEFORE the support set.  Scoring keeps the kernels the current support operands
+ *         were built for; only the front end of the tiled kernels follows bit 4 at once.
  *  key 1: arm a timeline trace of CTA 0 of the attention kernel (value 1) of the fused frame-MLP kernel (value 2) or of the head kernel (value 3); 0 frees it.
  *  key 2: programmatic dependent launch for the score kernel chain.
  *  key 3: softmax-group scheduling of the attention kernel: < 0 the groups take turns on the MUFU phase

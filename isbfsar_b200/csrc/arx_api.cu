@@ -82,6 +82,7 @@ void free_support(arx_handle *h) {
     h->tr[i].ks = h->tr[i].vs = nullptr;
     h->tr[i].ks_img = h->tr[i].vs_img = h->tr[i].vs_img_bf = h->tr[i].uc_img = nullptr;
     h->tr[i].kc_tiles = h->tr[i].vct_tiles = h->tr[i].uc_tiles = nullptr;
+    h->tr[i].route = ARX_ROUTE_NONE;
   }
   cudaFree(h->ss_feat);
   cudaFree(h->ss_poses);
@@ -90,53 +91,71 @@ void free_support(arx_handle *h) {
   h->way = h->way_cap = 0;
 }
 
-// per-window workspace of the fp32 path
-struct Fp32Ws {
-  float *H1, *FE, *G, *Kq, *Vq, *Z, *partial, *y, *h1, *h2;
+#define ARX_EP_UNSUPPORTED (-100)   /* internal: episode mode asked for a shape the batched kernels do not cover */
+
+// per-window workspace of the T=16 pair pipeline
+struct PairWs {
   __half *kq_img, *x_img, *h_img, *f_img, *y_img, *h1_img;
-  float *uab;
-  float *P, *U;              // frame-stream form: per-frame position-independent projections / head columns
+  float *uab, *G, *partial, *P, *U;     // P, U: frame-stream form: per-frame position-independent projections / head columns
   size_t bytes;
 };
-Fp32Ws carve_fp32(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, void *base,
-                  bool tc = false, bool tuples32 = true, bool tcl = false, bool tc_head = false, bool stream = false) {
+PairWs carve_pair(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, bool frames_stream, void *base) {
   Carver c(base);
-  Fp32Ws w{};
-  const int nb = tc ? 4 : (tr.N + 63) / 64;
-  w.kq_img = tc ? c.take<__half>(n * 128 * 128) : nullptr;
+  PairWs w{};
   const int64_t rows_pad = (n * h->T + 127) / 128 * 128, n_pad = (n + 127) / 128 * 128;
-  w.x_img = (tcl && from_frames) ? c.take<__half>(rows_pad * 128) : nullptr;
-  w.h_img = (tcl && from_frames) ? c.take<__half>(rows_pad * 192) : nullptr;
-  w.f_img = tcl ? c.take<__half>(rows_pad * 320) : nullptr;      // 4 feature sub-tiles + the one-hot sub-tile
-  w.y_img = (tcl && tc_head && disc) ? c.take<__half>(n_pad * (int64_t)h->tl_d1.nk * 64) : nullptr;
-  w.h1_img = (tcl && tc_head && disc) ? c.take<__half>(n_pad * 256) : nullptr;
-  w.uab = (tcl && tc_head && disc) ? c.take<float>(rows_pad * 32) : nullptr;
-  w.H1 = (from_frames && !tcl) ? c.take<float>(n * h->T * h->H) : nullptr;
-  w.FE = (from_frames && !tcl) ? c.take<float>(n * h->T * h->F) : nullptr;
-  w.G = c.take<float>((tc ? rows_pad : n * h->T) * 2 * tr.c * h->D);     // chunked layout holds whole 128-row tiles
-  w.Kq = tuples32 ? c.take<float>(n * tr.N * h->D) : nullptr;
-  w.Vq = tuples32 ? c.take<float>(n * tr.N * h->D) : nullptr;
-  w.Z = tuples32 ? c.take<float>(n * way * tr.N * 2) : nullptr;
-  w.partial = c.take<float>(n * way * nb);
-  const bool disc32 = disc && !(tcl && tc_head);
-  w.y = disc32 ? c.take<float>(n * tr.N * h->T) : nullptr;
-  w.h1 = disc32 ? c.take<float>(n * 256) : nullptr;
-  w.h2 = disc32 ? c.take<float>(n * 64) : nullptr;
-  w.P = stream ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
-  w.U = stream ? c.take<float>((n + h->T) * 32) : nullptr;
+  w.kq_img = c.take<__half>(n * 128 * 128);
+  w.x_img = from_frames ? c.take<__half>(rows_pad * 128) : nullptr;
+  w.h_img = from_frames ? c.take<__half>(rows_pad * 192) : nullptr;
+  w.f_img = c.take<__half>(rows_pad * 320);      // 4 feature sub-tiles + the one-hot sub-tile
+  w.y_img = disc ? c.take<__half>(n_pad * (int64_t)h->tl_d1.nk * 64) : nullptr;
+  w.h1_img = disc ? c.take<__half>(n_pad * 256) : nullptr;
+  w.uab = disc ? c.take<float>(rows_pad * 32) : nullptr;
+  w.G = c.take<float>(rows_pad * 2 * tr.c * h->D);     // chunked layout holds whole 128-row tiles
+  w.partial = c.take<float>(n * way * 4);
+  w.P = frames_stream ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
+  w.U = frames_stream ? c.take<float>((n + h->T) * 32) : nullptr;
   w.bytes = c.off + 256;
   return w;
 }
 
-int64_t pick_chunk(arx_handle *h, const ArxTransformer &tr, int way, bool from_frames, bool disc, int64_t n_total, bool tc,
-                   bool tuples32, bool tcl, bool tc_head) {
-  Fp32Ws one = carve_fp32(h, tr, 128, way, from_frames, disc, nullptr, tc, tuples32, tcl, tc_head);
-  one.bytes = one.bytes / 128 + 1;
-  int64_t cap = h->cfg.max_chunk > 0 ? h->cfg.max_chunk : 4096;
-  const size_t budget = (size_t)3 << 30;
-  int64_t fit = (int64_t)(budget / one.bytes);
-  if (fit < 1) fit = 1;
-  return std::max<int64_t>(1, std::min<int64_t>(std::min(cap, fit), n_total));
+// per-window workspace of the fp32 CUDA-core kernels
+struct Fp32Ws {
+  float *H1, *FE, *G, *Kq, *Vq, *Z, *partial, *y, *h1, *h2;
+  size_t bytes;
+};
+Fp32Ws carve_generic(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, void *base) {
+  Carver c(base);
+  Fp32Ws w{};
+  w.H1 = from_frames ? c.take<float>(n * h->T * h->H) : nullptr;
+  w.FE = from_frames ? c.take<float>(n * h->T * h->F) : nullptr;
+  w.G = c.take<float>(n * h->T * 2 * tr.c * h->D);
+  w.Kq = c.take<float>(n * tr.N * h->D);
+  w.Vq = c.take<float>(n * tr.N * h->D);
+  w.Z = c.take<float>(n * way * tr.N * 2);
+  w.partial = c.take<float>(n * way * ((tr.N + 63) / 64));
+  w.y = disc ? c.take<float>(n * tr.N * h->T) : nullptr;
+  w.h1 = disc ? c.take<float>(n * 256) : nullptr;
+  w.h2 = disc ? c.take<float>(n * 64) : nullptr;
+  w.bytes = c.off + 256;
+  return w;
+}
+
+// Windows per pass (at most max_chunk, default 4096, and 3 GB of the layout carve(n, base)), the workspace for them and,
+// without the caller's chosen buffer, the argmax scratch after it.  one_pass (episode mode): more passes are unsupported.
+template <class Ws, class Carve>
+int plan_chunks(arx_handle *h, int64_t n_windows, bool one_pass, const int32_t *chosen_dev, Carve &&carve, int64_t *chunk, Ws *w,
+                int32_t **chosen_ws) {
+  const size_t per = carve(128, nullptr).bytes / 128 + 1;
+  const int64_t cap = h->cfg.max_chunk > 0 ? h->cfg.max_chunk : 4096;
+  const int64_t fit = (int64_t)(((size_t)3 << 30) / per);
+  *chunk = std::max<int64_t>(1, std::min(std::min(cap, fit), n_windows));
+  if (one_pass && *chunk < n_windows) return ARX_EP_UNSUPPORTED;
+  const size_t bytes = carve(*chunk, nullptr).bytes;
+  const int rc = arx_ws_reserve(h, bytes + (chosen_dev ? 0 : (size_t)*chunk * sizeof(int32_t) + 256));
+  if (rc) return rc;
+  *w = carve(*chunk, h->ws);
+  *chosen_ws = chosen_dev ? nullptr : reinterpret_cast<int32_t *>(static_cast<char *>(h->ws) + bytes);
+  return ARX_OK;
 }
 
 // frames (n_seq*T, 3J) -> features (n_seq*T, F)             (model.py:164-180)
@@ -144,6 +163,32 @@ int embed_frames(arx_handle *h, const float *X, int64_t rows, float *H1, float *
   int rc = arx_fp32_linear(h, X, h->J3, h->fc1_w, h->J3, h->fc1_b, H1, h->H, rows, h->H, h->J3, ARX_ACT_RELU, nullptr, 1, st);
   if (rc) return rc;
   return arx_fp32_linear(h, H1, h->H, h->fc2_w, h->H, h->fc2_b, FE, h->F, rows, h->F, h->H, ARX_ACT_RELU, nullptr, 1, st);
+}
+
+// the same on tensor cores, three launches: frames -> fp16 image x_img -> fc1 -> h_img -> fc2 -> feature image f_img
+// (f_nk sub-tiles; f_onehot: the one-hot sub-tile of the positional table, or -1)
+int embed_frames_tc(arx_handle *h, const float *X, int64_t rows, __half *x_img, __half *h_img, __half *f_img, int f_nk, int f_onehot,
+                    cudaStream_t st) {
+  int rc;
+  if ((rc = arx_tc_rows_to_img(h, X, h->J3, h->J3, rows, x_img, h->tl_fc1.nk, -1, st))) return rc;
+  if ((rc = arx_tc_linear_img(h, h->tl_fc1, x_img, rows, ARX_ACT_RELU, h_img, h->tl_fc2.nk, -1, st))) return rc;
+  return arx_tc_linear_img(h, h->tl_fc2, h_img, rows, ARX_ACT_RELU, f_img, f_nk, f_onehot, st);
+}
+
+// discriminator MLP on the CUDA cores: head input y (n, N*T) -> d1 -> d2 -> d3 + sigmoid   (model.py:183-204)
+int disc_tail_fp32(arx_handle *h, const ArxTransformer &tr, const float *y, float *h1, float *h2, int64_t n, float *is_true, cudaStream_t st) {
+  const int K1 = tr.N * h->T;
+  int rc;
+  if ((rc = arx_fp32_linear(h, y, K1, h->d1_w, K1, h->d1_b, h1, 256, n, 256, K1, ARX_ACT_RELU, nullptr, 1, st))) return rc;
+  if ((rc = arx_fp32_linear(h, h1, 256, h->d2_w, 256, h->d2_b, h2, 64, n, 64, 256, ARX_ACT_RELU, nullptr, 1, st))) return rc;
+  return arx_fp32_linear(h, h2, 64, h->d3_w, 64, h->d3_b, is_true, 1, n, 1, 64, ARX_ACT_SIGMOID, nullptr, 1, st);
+}
+
+// the same on tensor cores from the head input image y_img: d1 -> h1_img, then d2 + d3 + sigmoid in one launch
+int disc_tail_tc(arx_handle *h, const __half *y_img, __half *h1_img, int64_t n, float *is_true, cudaStream_t st) {
+  const int rc = arx_tc_linear_img(h, h->tl_d1, y_img, n, ARX_ACT_RELU, h1_img, h->tl_d2.nk, -1, st);
+  if (rc) return rc;
+  return arx_tc_linear_sigmoid_dot(h, h->tl_d2, h1_img, n, h->d3_w, h->d3_b, is_true, st);
 }
 
 // features -> per-frame projections with the positional encoding folded into a per-position bias
@@ -279,8 +324,6 @@ int arx_load_weights(arx_handle *h, const arx_weights *w, void *stream) {
 #define UP(dst, src, n) if ((rc = upload(h, dst, src, (n), od, st)) != ARX_OK) return rc
   UP(h->fc1_w, w->fc1_w, (size_t)h->H * h->J3); UP(h->fc1_b, w->fc1_b, h->H);
   UP(h->fc2_w, w->fc2_w, (size_t)h->F * h->H); UP(h->fc2_b, w->fc2_b, h->F);
-  const int maxlen = (int)(h->T * 1.5);
-  (void)maxlen;
   for (int i = 0; i < h->cfg.n_transformers; ++i) {
     ArxTransformer &tr = h->tr[i];
     const int D = h->D, F = h->F, c = tr.c;
@@ -511,16 +554,16 @@ static int support_scratch_reserve(arx_handle *h, int way, SupportScratch *out) 
 
 // Which kernels score transformer `tr`:  the T=16 pair pipeline (arx_tc3.cu and friends: fused tuple images, head by
 // linearity, graph replay), the tiled any-N tcgen05 kernels (arx_tcn.cu: T=32, triples, other T, LayerNorm affines
-// outside the static exp2 bound), or the fp32 CUDA-core kernels (forced, debug outputs, D != 128).
-static bool route_gen3(const arx_handle *h, const ArxTransformer &tr) {
-  return h->cfg.force_path != 1 && arx_tc_supported(h, tr) && h->T == 16 && tr.c == 2 && h->tc_linears && (h->tc_variant & (4096 | 4)) == 0;
-}
-// LayerNorm affines outside the static bound: the ROWMAX variant of the tiled kernels is overflow-safe, but the fp16
-// operands of QK^T are no longer accurate enough there (measured on B200: gamma = 3 gives 5e-3 relative logit error
-// against the stated 1e-3; the error grows with gamma^2 like the bound does).  Parity first: such weights score on the
-// fp32 kernels unless the caller forces the tensor-core path (force_path = 2), and the handle says so once on stderr.
-static bool route_tiled(const arx_handle *h, const ArxTransformer &tr) {
-  return h->cfg.force_path != 1 && !route_gen3(h, tr) && arx_tcn_supported(h, tr) && (!arx_tcn_needs_rowmax(tr) || h->cfg.force_path == 2);
+// outside the static exp2 bound), or the fp32 CUDA-core kernels (forced, D != 128; debug outputs take them at score time).
+static ArxRoute support_route(const arx_handle *h, const ArxTransformer &tr) {
+  if (h->cfg.force_path == 1) return ARX_ROUTE_FP32;
+  if (arx_tc_supported(h, tr) && h->T == 16 && tr.c == 2 && h->tc_linears && (h->tc_variant & (4096 | 4)) == 0) return ARX_ROUTE_PAIR;
+  // LayerNorm affines outside the static bound: the ROWMAX variant of the tiled kernels is overflow-safe, but the fp16
+  // operands of QK^T are no longer accurate enough there (measured on B200: gamma = 3 gives 5e-3 relative logit error
+  // against the stated 1e-3; the error grows with gamma^2 like the bound does).  Parity first: such weights score on the
+  // fp32 kernels unless the caller forces the tensor-core path (force_path = 2), and the handle says so once on stderr.
+  if (arx_tcn_supported(h, tr) && (!arx_tcn_needs_rowmax(tr) || h->cfg.force_path == 2)) return ARX_ROUTE_TILED;
+  return ARX_ROUTE_FP32;
 }
 static void warn_fp32_fallback(arx_handle *h, int ti) {
   const ArxTransformer &tr = h->tr[ti];
@@ -529,6 +572,26 @@ static void warn_fp32_fallback(arx_handle *h, int ti) {
   fprintf(stderr, "libarx: transformers[%d].norm_k has a LayerNorm affine outside the fp16 tensor-core bound (|S| <= %.0f > %.0f): scoring on the "
                   "fp32 CUDA-core kernels (about 30x slower) to stay within the 1e-3 tolerance; force_path=2 selects the tensor-core "
                   "row-max variant at reduced accuracy\n", ti, (double)tr.softmax_bound, 100.0 / ARX_SOFTMAX_LOG2E);
+}
+
+// Decides transformer i's route and builds the support operands it reads: the tuple tensors ks/vs from the per-frame
+// projections G (or, with G == nullptr, ks/vs are already in place: arx_import_support), the operand images and the
+// head's Uc of the pair pipeline, the class tiles of the tiled kernels.
+static int support_operands(arx_handle *h, int i, const float *G, int way, cudaStream_t st) {
+  ArxTransformer &tr = h->tr[i];
+  tr.route = support_route(h, tr);
+  const bool imgs = tr.route == ARX_ROUTE_PAIR;
+  int rc = ARX_OK;
+  if (G && h->D == 128) rc = arx_tc_support_build(h, tr, G, way, imgs, st);      // tuples + LayerNorm + operand images, one launch
+  else if (G) rc = arx_fp32_build_tuples(h, tr, G, way, tr.ks, tr.vs, st);
+  else if (imgs) rc = arx_tc_prep_support(h, tr, way, st);
+  if (rc) return rc;
+  if (imgs && i == 0 && h->cfg.has_discriminator && (rc = arx_tc2_support_uc(h, tr, way, st))) return rc;
+  if (tr.route == ARX_ROUTE_TILED) {
+    if ((rc = arx_tcn_prep_support(h, tr, way, i == 0 && h->cfg.has_discriminator && tr.c == 2 && h->T <= 32, st))) return rc;
+    h->tiles_gen[i] = h->support_seq + 1;
+  }
+  return ARX_OK;
 }
 
 // projection + tuple/LayerNorm/image build of the support set from frame features given as an fp16 image
@@ -544,17 +607,7 @@ static int support_from_features(arx_handle *h, const __half *f_img, const float
     } else {
       if ((rc = project_frames(h, tr, feats32, rows, G, st))) return rc;
     }
-    const bool imgs = route_gen3(h, tr);
-    if (h->D == 128) {
-      if ((rc = arx_tc_support_build(h, tr, G, way, imgs, st))) return rc;      // tuples + LayerNorm + operand images, one launch
-      if (imgs && i == 0 && h->tc_linears && h->cfg.has_discriminator && h->T == 16 && tr.c == 2 && (rc = arx_tc2_support_uc(h, tr, way, st))) return rc;
-      if (route_tiled(h, tr)) {
-        if ((rc = arx_tcn_prep_support(h, tr, way, i == 0 && h->cfg.has_discriminator && tr.c == 2 && h->T <= 32, st))) return rc;
-        h->tiles_gen[i] = h->support_seq + 1;
-      }
-    } else {
-      if ((rc = arx_fp32_build_tuples(h, tr, G, way, tr.ks, tr.vs, st))) return rc;
-    }
+    if ((rc = support_operands(h, i, G, way, st))) return rc;
   }
   h->way = way;
   return ARX_OK;
@@ -603,10 +656,8 @@ int arx_set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, vo
   if (h->tc_linears) {
     // same tensor-core pipeline as the query frames; the fp32 'support_features' are derived lazily on request
     h->ss_feat_valid = false;
-    if ((rc = arx_tc_rows_to_img(h, h->ss_poses, h->J3, h->J3, rows, sc.x_img, h->tl_fc1.nk, -1, ss))) return rc;
-    if ((rc = arx_tc_linear_img(h, h->tl_fc1, sc.x_img, rows, ARX_ACT_RELU, sc.h_img, h->tl_fc2.nk, -1, ss))) return rc;
-    if ((rc = arx_tc_linear_img(h, h->tl_fc2, sc.h_img, rows, ARX_ACT_RELU, sc.f_img, h->tr[0].tl_proj.nk,
-                                h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
+    if ((rc = embed_frames_tc(h, h->ss_poses, rows, sc.x_img, sc.h_img, sc.f_img, h->tr[0].tl_proj.nk,
+                              h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
       return rc;
     rc = support_from_features(h, sc.f_img, nullptr, way, sc.G, ss);
   } else {
@@ -688,13 +739,7 @@ int arx_import_support(arx_handle *h, const void *blob_dev, int32_t way, void *s
     p += n;
     ARX_CUDA(h, cudaMemcpyAsync(tr.vs, p, n * sizeof(float), cudaMemcpyDeviceToDevice, ss));
     p += n;
-    if (route_gen3(h, tr)) {
-      if ((rc = arx_tc_prep_support(h, tr, way, ss))) return rc;
-      if (i == 0 && h->tc_linears && h->cfg.has_discriminator && h->T == 16 && tr.c == 2 && (rc = arx_tc2_support_uc(h, tr, way, ss))) return rc;
-    } else if (route_tiled(h, tr)) {
-      if ((rc = arx_tcn_prep_support(h, tr, way, i == 0 && h->cfg.has_discriminator && tr.c == 2 && h->T <= 32, ss))) return rc;
-      h->tiles_gen[i] = h->support_seq + 1;
-    }
+    if ((rc = support_operands(h, i, nullptr, way, ss))) return rc;
   }
   h->way = way;
   return support_join_record(h);
@@ -714,6 +759,16 @@ static int prof_mark(arx_handle *h, int idx, cudaStream_t st) {
   }
   ARX_CUDA(h, cudaEventRecord(h->prof_events[h->prof_used - (ARX_N_STAGES + 1) + idx], st));
   return ARX_OK;
+}
+
+// front end on the CUDA cores, windows from b0: frames (query_dev, embedded here) or features (qfeats_dev) -> per-frame
+// projections G
+static int front_end_fp32(arx_handle *h, const ArxTransformer &tr, const float *query_dev, const float *qfeats_dev, int64_t b0, int64_t rows,
+                          float *H1, float *FE, float *G, cudaStream_t st) {
+  int rc;
+  if (query_dev && (rc = embed_frames(h, query_dev + b0 * h->T * h->J3, rows, H1, FE, st))) return rc;
+  if ((rc = prof_mark(h, 1, st))) return rc;
+  return project_frames(h, tr, query_dev ? FE : qfeats_dev + b0 * h->T * h->F, rows, G, st);
 }
 
 extern "C++" {
@@ -742,32 +797,36 @@ static ArxScoreGraph *score_graph_lookup(arx_handle *h, const ArxScoreGraphKey &
   return &h->graphs.back();
 }
 
-// Run one segment of the score chain: eagerly the first time a key is seen (one-time initialisation -- symbol
-// uploads, function attributes, allocations -- must not happen under capture), captured into a graph the second
-// time, replayed from then on.
-template <class F> static int score_segment(arx_handle *h, ArxScoreGraph *g, int seg, cudaStream_t st, F &&body) {
-  if (!g || g->seen < 1) return body();
-  if (!g->exec[seg]) {
+// Replay *exec on st, capturing body() on st into it first when it is empty.  The launches body() counts during the
+// capture are recorded in *launches instead, and every replay adds them to the handle's launch count.
+template <class F> static int graph_replay(arx_handle *h, cudaStream_t st, const char *what, cudaGraphExec_t *exec, int64_t *launches, F &&body) {
+  if (!*exec) {
     const int64_t l0 = h->launches;
     ARX_CUDA(h, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
     const int rc = body();
     cudaGraph_t graph = nullptr;
     const cudaError_t e = cudaStreamEndCapture(st, &graph);
     if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-    if (e != cudaSuccess || !graph) return arx_fail(h, ARX_ERR_CUDA, "score: stream capture failed: %s", cudaGetErrorString(e));
-    const cudaError_t e2 = cudaGraphInstantiate(&g->exec[seg], graph, 0);
+    if (e != cudaSuccess || !graph) return arx_fail(h, ARX_ERR_CUDA, "%s: stream capture failed: %s", what, cudaGetErrorString(e));
+    const cudaError_t e2 = cudaGraphInstantiate(exec, graph, 0);
     cudaGraphDestroy(graph);
-    if (e2 != cudaSuccess) { g->exec[seg] = nullptr; return arx_fail(h, ARX_ERR_CUDA, "score: graph instantiation failed: %s", cudaGetErrorString(e2)); }
-    g->launches[seg] = h->launches - l0;
+    if (e2 != cudaSuccess) { *exec = nullptr; return arx_fail(h, ARX_ERR_CUDA, "%s: graph instantiation failed: %s", what, cudaGetErrorString(e2)); }
+    *launches = h->launches - l0;
     h->launches = l0;
   }
-  ARX_CUDA(h, cudaGraphLaunch(g->exec[seg], st));
-  h->launches += g->launches[seg];
+  ARX_CUDA(h, cudaGraphLaunch(*exec, st));
+  h->launches += *launches;
   return ARX_OK;
 }
-}  // extern "C++"
 
-#define ARX_EP_UNSUPPORTED (-100)   /* internal: episode mode asked for a shape the batched kernels do not cover */
+// Run one segment of the score chain: eagerly the first time a key is seen (one-time initialisation -- symbol
+// uploads, function attributes, allocations -- must not happen under capture), captured into a graph the second
+// time, replayed from then on.
+template <class F> static int score_segment(arx_handle *h, ArxScoreGraph *g, int seg, cudaStream_t st, F &&body) {
+  if (!g || g->seen < 1) return body();
+  return graph_replay(h, st, "score", &g->exec[seg], &g->launches[seg], body);
+}
+}  // extern "C++"
 
 // ---- scoring on the tiled any-N tcgen05 kernels (arx_tcn.cu) -----------------------------------------------------
 struct TcnWs {
@@ -819,21 +878,11 @@ static int tcn_backend(arx_handle *h, const ArxTransformer &tr, const TcnWs &w, 
   if ((rc = prof_mark(h, 3, st))) return rc;
   if ((rc = arx_tcn_attention(h, tr, w.kq, w.G, ldg, n, way, w.partial, logits, ch, w.vq, st))) return rc;
   if ((rc = prof_mark(h, 4, st))) return rc;
-  if (is_true) {
-    if (tcl && ((int64_t)tr.N * h->T) % 64)       // fc1's K is padded to whole 64-column sub-tiles: the pad columns must be zero, not stale
-      ARX_CUDA(h, cudaMemsetAsync(w.y_img, 0, (size_t)((n + 127) / 128 * 128) * h->tl_d1.nk * 64 * sizeof(__half), st));
-    if ((rc = arx_tcn_head(h, tr, w.kq, w.G, ldg, n, ch, w.uab, w.y, w.y_img, tcl ? h->tl_d1.nk : 0, w.vq_head, st))) return rc;
-    if (tcl) {
-      if ((rc = arx_tc_linear_img(h, h->tl_d1, w.y_img, n, ARX_ACT_RELU, w.h1_img, h->tl_d2.nk, -1, st))) return rc;
-      if ((rc = arx_tc_linear_sigmoid_dot(h, h->tl_d2, w.h1_img, n, h->d3_w, h->d3_b, is_true, st))) return rc;
-    } else {
-      const int K1 = tr.N * h->T;
-      if ((rc = arx_fp32_linear(h, w.y, K1, h->d1_w, K1, h->d1_b, w.h1, 256, n, 256, K1, ARX_ACT_RELU, nullptr, 1, st))) return rc;
-      if ((rc = arx_fp32_linear(h, w.h1, 256, h->d2_w, 256, h->d2_b, w.h2, 64, n, 64, 256, ARX_ACT_RELU, nullptr, 1, st))) return rc;
-      if ((rc = arx_fp32_linear(h, w.h2, 64, h->d3_w, 64, h->d3_b, is_true, 1, n, 1, 64, ARX_ACT_SIGMOID, nullptr, 1, st))) return rc;
-    }
-  }
-  return ARX_OK;
+  if (!is_true) return ARX_OK;
+  if (tcl && ((int64_t)tr.N * h->T) % 64)       // fc1's K is padded to whole 64-column sub-tiles: the pad columns must be zero, not stale
+    ARX_CUDA(h, cudaMemsetAsync(w.y_img, 0, (size_t)((n + 127) / 128 * 128) * h->tl_d1.nk * 64 * sizeof(__half), st));
+  if ((rc = arx_tcn_head(h, tr, w.kq, w.G, ldg, n, ch, w.uab, w.y, w.y_img, tcl ? h->tl_d1.nk : 0, w.vq_head, st))) return rc;
+  return tcl ? disc_tail_tc(h, w.y_img, w.h1_img, n, is_true, st) : disc_tail_fp32(h, tr, w.y, w.h1, w.h2, n, is_true, st);
 }
 
 static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
@@ -843,30 +892,25 @@ static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float 
   const int way = h->way;
   if (!tr.kc_tiles) return arx_fail(h, ARX_ERR_STATE, "score: support operands of the tiled kernels are missing (set the support set again)");
   if (disc && !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "score: the open-set head of the tiled kernels needs pair tuples and T <= 32");
-  // windows per pass: workspace budget (the query tiles are 32 KB per 128 tuples per window)
-  const size_t per = carve_tcn(h, tr, 128, way, from_frames, disc, tcl, nullptr, frames_stream).bytes / 128 + 1;
-  int64_t chunk = h->cfg.max_chunk > 0 ? h->cfg.max_chunk : 4096;
-  chunk = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(chunk, (int64_t)(((size_t)3 << 30) / per)), n_windows));
-  const size_t need = carve_tcn(h, tr, chunk, way, from_frames, disc, tcl, nullptr, frames_stream).bytes + (chosen_dev ? 0 : (size_t)chunk * sizeof(int32_t) + 256);
-  int rc = arx_ws_reserve(h, need);
+  int64_t chunk;
+  TcnWs w;
+  int32_t *chosen_ws;
+  int rc = plan_chunks(h, n_windows, false, chosen_dev, [&](int64_t n, void *base) {
+    return carve_tcn(h, tr, n, way, from_frames, disc, tcl, base, frames_stream);
+  }, &chunk, &w, &chosen_ws);
   if (rc) return rc;
-  TcnWs w = carve_tcn(h, tr, chunk, way, from_frames, disc, tcl, h->ws, frames_stream);
-  int32_t *chosen_ws = chosen_dev ? nullptr : reinterpret_cast<int32_t *>(static_cast<char *>(h->ws) + need - (size_t)chunk * sizeof(int32_t) - 256);
   const int ldg = 2 * tr.c * h->D;
-  h->last_path = 3;
+  const int f_nk = tr.tl_proj.nk, f_onehot = tr.table_in_gemm ? f_nk - 1 : -1;     // feature image: + one-hot sub-tile
+  h->last_path = ARX_ROUTE_TILED;
   for (int64_t b0 = 0; b0 < n_windows; b0 += chunk) {
     const int64_t n = std::min(chunk, n_windows - b0), rows = n * h->T;
     if ((rc = prof_mark(h, 0, st))) return rc;
-    const float *FE = nullptr;
     if (frames_stream) {
       // frame stream: embed and project every frame once (position-independent), then form the windows' projections
       const int64_t rows_f = n + h->T - 1;
       if (tcl) {
-        const int f_nk = tr.tl_proj.nk;
         const ArxTcLinear &L = tr.table_in_gemm ? tr.tl_proj_nt : tr.tl_proj;
-        if ((rc = arx_tc_rows_to_img(h, query_dev + b0 * h->J3, h->J3, h->J3, rows_f, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc1, w.x_img, rows_f, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc2, w.h_img, rows_f, ARX_ACT_RELU, w.f_img, f_nk, -1, st))) return rc;
+        if ((rc = embed_frames_tc(h, query_dev + b0 * h->J3, rows_f, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
         if ((rc = prof_mark(h, 1, st))) return rc;
         if ((rc = arx_tc_linear_f32(h, L, w.f_img, f_nk, rows_f, w.P, ldg, nullptr, 1, st))) return rc;
       } else {
@@ -876,22 +920,12 @@ static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float 
       }
       if ((rc = arx_form_windows_launch(h, tr, w.P, nullptr, w.G, nullptr, n, false, st))) return rc;
     } else if (tcl) {
-      const int f_nk = tr.tl_proj.nk, f_onehot = tr.table_in_gemm ? f_nk - 1 : -1;
       if (from_frames) {
-        if ((rc = arx_tc_rows_to_img(h, query_dev + b0 * h->T * h->J3, h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, st))) return rc;
+        if ((rc = embed_frames_tc(h, query_dev + b0 * h->T * h->J3, rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
       } else if ((rc = arx_tc_rows_to_img(h, qfeats_dev + b0 * h->T * h->F, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
       if ((rc = prof_mark(h, 1, st))) return rc;
       if ((rc = arx_tc_linear_f32(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, ldg, tr.table_in_gemm ? nullptr : tr.bp, h->T, st))) return rc;
-    } else {
-      if (from_frames) {
-        if ((rc = embed_frames(h, query_dev + b0 * h->T * h->J3, rows, w.H1, w.FE, st))) return rc;
-        FE = w.FE;
-      } else FE = qfeats_dev + b0 * h->T * h->F;
-      if ((rc = prof_mark(h, 1, st))) return rc;
-      if ((rc = project_frames(h, tr, FE, rows, w.G, st))) return rc;
-    }
+    } else if ((rc = front_end_fp32(h, tr, query_dev, qfeats_dev, b0, rows, w.H1, w.FE, w.G, st))) return rc;
     if ((rc = prof_mark(h, 2, st))) return rc;
     int32_t *ch = chosen_dev ? chosen_dev + b0 : chosen_ws;
     if ((rc = tcn_backend(h, tr, w, n, way, tcl, logits_dev + b0 * way, is_true_dev ? is_true_dev + b0 : nullptr, ch, st))) return rc;
@@ -914,15 +948,14 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
   if (disc && (ti != 0 || !tr.uc_img)) return arx_fail(h, ARX_ERR_STATE, "score: open-set head operands missing (set the support set again)");
   const bool big_batch = n_windows * h->T >= 128ll * 2 * h->sm_count;             // persistent GEMMs pay off from ~2 tiles per SM
   const bool p_embed = big_batch && (h->tc_variant & 1024) == 0 && arx_tcp_supported(h->tl_fc1) && arx_tcp_supported(h->tl_fc2);
-  const int64_t chunk = pick_chunk(h, tr, way, from_frames, disc, n_windows, true, false, true, disc);
-  if (ep_way > 0 && chunk < n_windows) return ARX_EP_UNSUPPORTED;
-  Fp32Ws sz = carve_fp32(h, tr, chunk, way, from_frames, disc, nullptr, true, false, true, disc, frames_stream);
-  const size_t extra = chosen_dev ? 0 : (size_t)chunk * sizeof(int32_t) + 256;
-  int rc = arx_ws_reserve(h, sz.bytes + extra);
+  int64_t chunk;
+  PairWs w;
+  int32_t *chosen_ws;
+  int rc = plan_chunks(h, n_windows, ep_way > 0, chosen_dev, [&](int64_t n, void *base) {
+    return carve_pair(h, tr, n, way, from_frames, disc, frames_stream, base);
+  }, &chunk, &w, &chosen_ws);
   if (rc) return rc;
-  Fp32Ws w = carve_fp32(h, tr, chunk, way, from_frames, disc, h->ws, true, false, true, disc, frames_stream);
-  int32_t *chosen_ws = chosen_dev ? nullptr : reinterpret_cast<int32_t *>(static_cast<char *>(h->ws) + sz.bytes);
-  h->last_path = 2;
+  h->last_path = ARX_ROUTE_PAIR;
   bool aux_pending = false;
   const int reserve = (h->support_inflight && big_batch && (h->tc_variant & 32768) == 0) ? h->sm_reserve_n : 0;      // debug bit 32768: no reserved SMs
   ArxScoreGraph *sg = nullptr;
@@ -950,9 +983,7 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
       if (frames_stream) {
         // every frame is embedded and projected ONCE (position-independent); the windows are formed on the device
         const int64_t rows_f = n + h->T - 1;
-        if ((rc = arx_tc_rows_to_img(h, query_dev + b0 * h->J3, h->J3, h->J3, rows_f, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc1, w.x_img, rows_f, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_fc2, w.h_img, rows_f, ARX_ACT_RELU, w.f_img, f_nk, -1, st))) return rc;
+        if ((rc = embed_frames_tc(h, query_dev + b0 * h->J3, rows_f, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
         if ((rc = prof_mark(h, 1, st))) return rc;
         if ((rc = arx_tc_linear_f32(h, tr.tl_proj_nt, w.f_img, f_nk, rows_f, w.P, g_ld, nullptr, 1, st))) return rc;
         if (disc && (rc = arx_tc_linear_f32_small(h, tr.tl_uab, w.f_img, f_nk, rows_f, w.U, 32, nullptr, h->T, st))) return rc;
@@ -967,14 +998,11 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
                                       : static_cast<const void *>(query_dev + b0 * h->T * h->J3);
         if (p_embed && (h->tc_variant & 8192) == 0 && arx_mlp_fused_supported(h, xq)) {
           if ((rc = arx_mlp_fused(h, xq, h->query_f16, rows, w.f_img, f_nk, f_onehot, st))) return rc;      // one launch: poses -> feature image
-        } else if ((rc = arx_tc_rows_to_img(h, static_cast<const float *>(xq), h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-        else if (p_embed) {
+        } else if (p_embed) {
+          if ((rc = arx_tc_rows_to_img(h, static_cast<const float *>(xq), h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
           if ((rc = arx_tcp_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
           if ((rc = arx_tcp_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, st))) return rc;
-        } else {
-          if ((rc = arx_tc_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
-          if ((rc = arx_tc_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, st))) return rc;
-        }
+        } else if ((rc = embed_frames_tc(h, static_cast<const float *>(xq), rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
       } else if ((rc = arx_tc_rows_to_img(h, qfeats_dev + b0 * h->T * h->F, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
       if ((rc = prof_mark(h, 1, st))) return rc;
       if ((rc = arx_tcp_linear_chunked(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, st))) return rc;
@@ -1011,8 +1039,7 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
       if (disc) {
         if (aux_pending) { ARX_CUDA(h, cudaStreamWaitEvent(st, h->ev_aux_done, 0)); aux_pending = false; }
         if ((rc = arx_tc2_head_launch(h, tr, w.kq_img, w.uab, n, ch, w.y_img, h->tl_d1.nk, ep_way, st))) return rc;
-        if ((rc = arx_tc_linear_img(h, h->tl_d1, w.y_img, n, ARX_ACT_RELU, w.h1_img, h->tl_d2.nk, -1, st))) return rc;
-        if ((rc = arx_tc_linear_sigmoid_dot(h, h->tl_d2, w.h1_img, n, h->d3_w, h->d3_b, is_true_dev + b0, st))) return rc;
+        if ((rc = disc_tail_tc(h, w.y_img, w.h1_img, n, is_true_dev + b0, st))) return rc;
       }
       return ARX_OK;
     });
@@ -1029,25 +1056,19 @@ static int score_fp32(arx_handle *h, int ti, const float *query_dev, const float
   const ArxTransformer &tr = h->tr[ti];
   const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr;
   const int way = h->way;
-  const int64_t chunk = pick_chunk(h, tr, way, from_frames, disc, n_windows, false, true, false, false);
-  Fp32Ws sz = carve_fp32(h, tr, chunk, way, from_frames, disc, nullptr);
-  const size_t extra = chosen_dev ? 0 : (size_t)chunk * sizeof(int32_t) + 256;
-  int rc = arx_ws_reserve(h, sz.bytes + extra);
+  int64_t chunk;
+  Fp32Ws w;
+  int32_t *chosen_ws;
+  int rc = plan_chunks(h, n_windows, false, chosen_dev, [&](int64_t n, void *base) {
+    return carve_generic(h, tr, n, way, from_frames, disc, base);
+  }, &chunk, &w, &chosen_ws);
   if (rc) return rc;
-  Fp32Ws w = carve_fp32(h, tr, chunk, way, from_frames, disc, h->ws);
-  int32_t *chosen_ws = chosen_dev ? nullptr : reinterpret_cast<int32_t *>(static_cast<char *>(h->ws) + sz.bytes);
-  h->last_path = 1;
+  h->last_path = ARX_ROUTE_FP32;
   const int64_t NN = (int64_t)tr.N * tr.N, ND = (int64_t)tr.N * h->D;
   for (int64_t b0 = 0; b0 < n_windows; b0 += chunk) {
     const int64_t n = std::min(chunk, n_windows - b0), rows = n * h->T;
     if ((rc = prof_mark(h, 0, st))) return rc;
-    const float *FE;
-    if (from_frames) {
-      if ((rc = embed_frames(h, query_dev + b0 * h->T * h->J3, rows, w.H1, w.FE, st))) return rc;
-      FE = w.FE;
-    } else FE = qfeats_dev + b0 * h->T * h->F;
-    if ((rc = prof_mark(h, 1, st))) return rc;
-    if ((rc = project_frames(h, tr, FE, rows, w.G, st))) return rc;
+    if ((rc = front_end_fp32(h, tr, query_dev, qfeats_dev, b0, rows, w.H1, w.FE, w.G, st))) return rc;
     if ((rc = prof_mark(h, 2, st))) return rc;
     if ((rc = arx_fp32_build_tuples(h, tr, w.G, n, w.Kq, w.Vq, st))) return rc;
     if ((rc = support_wait(h, st))) return rc;
@@ -1057,12 +1078,7 @@ static int score_fp32(arx_handle *h, int ti, const float *query_dev, const float
                                  probs ? probs + b0 * way * NN : nullptr, protos ? protos + b0 * way * ND : nullptr, st)))
       return rc;
     if ((rc = prof_mark(h, 4, st))) return rc;
-    if (disc) {
-      const int K1 = tr.N * h->T;
-      if ((rc = arx_fp32_linear(h, w.y, K1, h->d1_w, K1, h->d1_b, w.h1, 256, n, 256, K1, ARX_ACT_RELU, nullptr, 1, st))) return rc;
-      if ((rc = arx_fp32_linear(h, w.h1, 256, h->d2_w, 256, h->d2_b, w.h2, 64, n, 64, 256, ARX_ACT_RELU, nullptr, 1, st))) return rc;
-      if ((rc = arx_fp32_linear(h, w.h2, 64, h->d3_w, 64, h->d3_b, is_true_dev + b0, 1, n, 1, 64, ARX_ACT_SIGMOID, nullptr, 1, st))) return rc;
-    }
+    if (disc && (rc = disc_tail_fp32(h, tr, w.y, w.h1, w.h2, n, is_true_dev + b0, st))) return rc;
     if ((rc = prof_mark(h, 5, st))) return rc;
   }
   return ARX_OK;
@@ -1081,12 +1097,13 @@ static int score_impl(arx_handle *h, int ti, const float *query_dev, const float
     return arx_fail(h, ARX_ERR_INVALID, "score: the discriminator is sized for pair tuples of transformers[0] (model.py:283-285)");
   if (ep_way > 0 && (int64_t)ep_way * n_windows != h->way) return arx_fail(h, ARX_ERR_STATE, "score: episode pool does not match the batch");
   const bool debug_out = probs || protos;
-  if (ep_way > 0 && (debug_out || !route_gen3(h, tr) || !tr.ks_img || !query_dev)) return ARX_EP_UNSUPPORTED;
+  const ArxRoute route = debug_out ? ARX_ROUTE_FP32 : tr.route;      // only the fp32 kernels write the debug outputs
+  if (ep_way > 0 && (route != ARX_ROUTE_PAIR || !query_dev)) return ARX_EP_UNSUPPORTED;
   int rc = workspace_wait(h, st);
   if (rc) return rc;
-  if (!debug_out && route_gen3(h, tr) && tr.ks_img)
+  if (route == ARX_ROUTE_PAIR)
     rc = score_gen3(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, ep_way, frames_stream);
-  else if (!debug_out && route_tiled(h, tr))
+  else if (route == ARX_ROUTE_TILED)
     rc = score_tcn(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, frames_stream);
   else if (frames_stream)
     rc = ARX_EP_UNSUPPORTED;            // the caller materialises the windows for the fp32 kernels
@@ -1179,8 +1196,8 @@ int arx_debug_attention(arx_handle *h, const float *query_dev, int64_t n_windows
 // results are bit-identical for inputs that are representable in fp16); only the T=16 pair pipeline and the tiled kernels
 // with tensor-core linear layers read halves
 static bool f16_input_ok(const arx_handle *h) {
-  const ArxTransformer &tr = h->tr[0];
-  return h->tc_linears && (h->tc_variant & 4) == 0 && ((route_gen3(h, tr) && tr.ks_img) || route_tiled(h, tr));
+  const ArxRoute route = h->tr[0].route;
+  return h->tc_linears && (h->tc_variant & 4) == 0 && (route == ARX_ROUTE_PAIR || route == ARX_ROUTE_TILED);
 }
 
 static int score_host_impl(arx_handle *h, const void *query_host_v, bool f16, int64_t n_windows, float *logits_host, float *is_true_host,
@@ -1332,7 +1349,7 @@ int arx_score_host_wait(arx_handle *h, int64_t ticket) {
 static void stream_free(arx_handle *h) {
   ArxStream &s = h->stream;
   if (s.exec) cudaGraphExecDestroy(s.exec);
-  cudaFree(s.ring); cudaFree(s.slot); cudaFree(s.x_dev); cudaFree(s.out_dev); cudaFree(s.logits); cudaFree(s.is_true); cudaFree(s.chosen);
+  cudaFree(s.ring); cudaFree(s.slot); cudaFree(s.x_dev); cudaFree(s.out_dev); cudaFree(s.logits);
   cudaFree(s.ws); cudaFree(s.iota); cudaFree(s.y_all);
   if (s.st2) { cudaStreamDestroy(s.st2); cudaEventDestroy(s.ev_fork); cudaEventDestroy(s.ev_join); }
   if (s.pin_in) cudaFreeHost(s.pin_in);
@@ -1359,7 +1376,7 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
   if (h->way < 1) return arx_fail(h, ARX_ERR_STATE, "stream_push: support set not set");
   ArxTransformer &tr = h->tr[0];
   const int way = h->way, NO = 2 * tr.c * h->D;
-  const bool disc = h->cfg.has_discriminator != 0, tcl = h->tc_linears;
+  const bool disc = h->cfg.has_discriminator != 0;
   if (h->cfg.force_path == 1 || !arx_tcn_supported(h, tr) || arx_tcn_needs_rowmax(tr) || tr.c != 2 || (disc && h->T > 32) || h->J3 > 256 || h->H > 256 ||
       h->F > 256)
     return arx_fail(h, ARX_ERR_INVALID, "stream_push: the resident streaming path covers pair tuples on the tiled tcgen05 kernels only");
@@ -1370,8 +1387,6 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
     ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&s.ring), (size_t)h->T * NO * sizeof(float)));
     ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&s.slot), sizeof(int)));
     ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&s.x_dev), (size_t)h->J3 * sizeof(float)));
-    ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&s.is_true), sizeof(float)));
-    ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&s.chosen), sizeof(int32_t)));
     ARX_CUDA(h, cudaMallocHost(reinterpret_cast<void **>(&s.pin_in), (size_t)h->J3 * sizeof(float)));
     ARX_CUDA(h, cudaMemsetAsync(s.ring, 0, (size_t)h->T * NO * sizeof(float), s.st));
     ARX_CUDA(h, cudaMemsetAsync(s.slot, 0, sizeof(int), s.st));
@@ -1450,29 +1465,12 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
   if (s.seen < 1 || prof || !graphs_enabled(h)) {
     if ((rc = body())) return rc;                       // first sighting: eager (allocations, one-time initialisation)
     s.seen++;
-  } else {
-    if (!s.exec) {
-      const int64_t l0 = h->launches;
-      ARX_CUDA(h, cudaStreamBeginCapture(s.st, cudaStreamCaptureModeThreadLocal));
-      rc = body();
-      cudaGraph_t graph = nullptr;
-      const cudaError_t e = cudaStreamEndCapture(s.st, &graph);
-      if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-      if (e != cudaSuccess || !graph) return arx_fail(h, ARX_ERR_CUDA, "stream_push: capture failed: %s", cudaGetErrorString(e));
-      const cudaError_t e2 = cudaGraphInstantiate(&s.exec, graph, 0);
-      cudaGraphDestroy(graph);
-      if (e2 != cudaSuccess) { s.exec = nullptr; return arx_fail(h, ARX_ERR_CUDA, "stream_push: graph instantiation failed: %s", cudaGetErrorString(e2)); }
-      s.seen = (int)(h->launches - l0);                  // launches per frame (>= 1)
-      h->launches = l0;
-    }
-    ARX_CUDA(h, cudaGraphLaunch(s.exec, s.st));
-    h->launches += s.seen;
-  }
+  } else if ((rc = graph_replay(h, s.st, "stream_push", &s.exec, &s.launches, body))) return rc;
   ARX_CUDA(h, cudaStreamSynchronize(s.st));
   memcpy(result_host, s.pin_out, (size_t)(way + 1) * sizeof(float));
   s.count++;
   if (valid) *valid = s.count >= h->T ? 1 : 0;            // ar.py:43-44: nothing to report before seq_len frames were seen
-  h->last_path = 3;
+  h->last_path = ARX_ROUTE_TILED;
   return ARX_OK;
 }
 

@@ -17,6 +17,15 @@ struct ArxTcLinear {
   int N = 0, K = 0, BN = 0, n_tiles = 0, nk = 0;
 };
 
+// Which kernels score a transformer; the values are those arx_last_path reports.  Decided when the support operands are
+// built (arx_api.cu: support_route), because each route needs operands of its own.
+enum ArxRoute {
+  ARX_ROUTE_NONE = 0,    // no support operands yet
+  ARX_ROUTE_FP32 = 1,    // fp32 CUDA-core kernels (arx_fp32.cu)
+  ARX_ROUTE_PAIR = 2,    // T=16 pair pipeline (arx_tc3.cu and friends)
+  ARX_ROUTE_TILED = 3,   // tiled any-N tcgen05 kernels (arx_tcn.cu)
+};
+
 struct ArxTransformer {
   int c = 0;            // tuple cardinality
   int N = 0;            // C(T,c)
@@ -30,6 +39,7 @@ struct ArxTransformer {
   float *ln_g = nullptr, *ln_b = nullptr;
   float ln_host[256] = {};  // host copy [gamma(128) | beta(128)] when D == 128: kernel-parameter operands of k_tuple_img
   int32_t *tuples = nullptr; // (N,c) int32, built on device
+  ArxRoute route = ARX_ROUTE_NONE;   // the route the support operands below were built for
   // support operands, fp32 generic path: (W,N,D) each
   float *ks = nullptr, *vs = nullptr;
   // support operands, tcgen05 path: fp16 UMMA smem images, see arx_tc.cu
@@ -73,8 +83,8 @@ struct ArxScoreGraph {
 struct ArxStream {
   float *ring = nullptr;            // (T, 2cD) position-independent projections of the last T frames
   int *slot = nullptr;              // device: ring slot the next frame goes to
-  float *x_dev = nullptr, *out_dev = nullptr, *logits = nullptr, *is_true = nullptr;
-  int32_t *chosen = nullptr, *iota = nullptr;
+  float *x_dev = nullptr, *out_dev = nullptr, *logits = nullptr;
+  int32_t *iota = nullptr;
   float *y_all = nullptr;
   cudaStream_t st2 = nullptr;       // the head of all classes runs beside the main attention launch
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
@@ -83,6 +93,7 @@ struct ArxStream {
   size_t ws_bytes = 0;
   cudaStream_t st = nullptr;
   cudaGraphExec_t exec = nullptr;
+  int64_t launches = 0;             // kernel launches one replay of exec stands for
   uint64_t sgen = 0, wgen = 0;      // support / weights generation the graph (and the tiled operands) were built for
   int way = 0, seen = 0;
   int64_t count = 0;                // frames pushed since the last reset
@@ -126,9 +137,7 @@ struct arx_handle {
   // workspace (grown on demand)
   void *ws = nullptr;
   size_t ws_bytes = 0;
-  // pinned staging for arx_score_host
-  void *pin_in[2] = {nullptr, nullptr};
-  void *pin_out[2] = {nullptr, nullptr};
+  // device staging for arx_score_host
   void *dev_in[2] = {nullptr, nullptr};
   void *dev_out[2] = {nullptr, nullptr};
   size_t stage_windows = 0;
