@@ -55,7 +55,8 @@ typedef struct arx_config {
   int32_t cardinality[ARX_MAX_TRANSFORMERS]; /* temp_set entries, 2 or 3                 */
   int32_t has_discriminator; /* 1 for model="DISC" (model.py:282-285)                    */
   int32_t max_chunk;      /* windows processed per internal pass (0 = default)           */
-  int32_t force_path;     /* 0 = auto, 1 = fp32 CUDA-core kernels, 2 = tcgen05 kernels   */
+  int32_t force_path;     /* 0 = auto, 1 = fp32 CUDA-core kernels, 2 = tcgen05 kernels   *
+                           * (also for LayerNorm affines past the accuracy bound, DESIGN 4) */
 } arx_config;
 
 /* Weights in the reference state_dict layouts (SURVEY.md 8b); host or device fp32. */

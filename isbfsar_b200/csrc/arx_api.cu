@@ -552,26 +552,36 @@ static int support_scratch_reserve(arx_handle *h, int way, SupportScratch *out) 
   return ARX_OK;
 }
 
+static float accuracy_bound(const ArxTransformer &tr) {
+  return tr.N < ARX_TC_FEW_TUPLES ? ARX_TC_ACCURACY_BOUND_FEW_TUPLES : ARX_TC_ACCURACY_BOUND;
+}
+// The tensor-core routes may score transformer `tr`: its LayerNorm affine is inside the accuracy bound, or the caller
+// forced them (force_path = 2) and accepts the reduced accuracy.
+static bool tc_admitted(const arx_handle *h, const ArxTransformer &tr) {
+  return h->cfg.force_path == 2 || tr.softmax_bound < accuracy_bound(tr);
+}
+
 // Which kernels score transformer `tr`:  the T=16 pair pipeline (arx_tc3.cu and friends: fused tuple images, head by
-// linearity, graph replay), the tiled any-N tcgen05 kernels (arx_tcn.cu: T=32, triples, other T, LayerNorm affines
-// outside the static exp2 bound), or the fp32 CUDA-core kernels (forced, D != 128; debug outputs take them at score time).
+// linearity, graph replay), the tiled any-N tcgen05 kernels (arx_tcn.cu: T=32, triples, other T, and under force_path = 2
+// LayerNorm affines past the overflow bound), or the fp32 CUDA-core kernels (forced, D != 128, LayerNorm affines past
+// the accuracy bound; debug outputs take them at score time).
 static ArxRoute support_route(const arx_handle *h, const ArxTransformer &tr) {
-  if (h->cfg.force_path == 1) return ARX_ROUTE_FP32;
+  // Past the accuracy bound the fp16 QK^T and bf16 P.V operands lose the 1e-3 tolerance well before exp2 can overflow
+  // (DESIGN 4: the error grows with the bound).  Parity first: such weights score on the fp32 kernels unless the caller
+  // forces the tensor-core routes, and the handle says so once on stderr.
+  if (h->cfg.force_path == 1 || !tc_admitted(h, tr)) return ARX_ROUTE_FP32;
   if (arx_tc_supported(h, tr) && h->T == 16 && tr.c == 2 && h->tc_linears && (h->tc_variant & (4096 | 4)) == 0) return ARX_ROUTE_PAIR;
-  // LayerNorm affines outside the static bound: the ROWMAX variant of the tiled kernels is overflow-safe, but the fp16
-  // operands of QK^T are no longer accurate enough there (measured on B200: gamma = 3 gives 5e-3 relative logit error
-  // against the stated 1e-3; the error grows with gamma^2 like the bound does).  Parity first: such weights score on the
-  // fp32 kernels unless the caller forces the tensor-core path (force_path = 2), and the handle says so once on stderr.
-  if (arx_tcn_supported(h, tr) && (!arx_tcn_needs_rowmax(tr) || h->cfg.force_path == 2)) return ARX_ROUTE_TILED;
+  if (arx_tcn_supported(h, tr)) return ARX_ROUTE_TILED;      // the ROWMAX variant past the overflow bound
   return ARX_ROUTE_FP32;
 }
 static void warn_fp32_fallback(arx_handle *h, int ti) {
   const ArxTransformer &tr = h->tr[ti];
-  if (h->cfg.force_path == 1 || (h->warned & (1u << ti)) || !arx_tcn_supported(h, tr) || !arx_tcn_needs_rowmax(tr)) return;
+  if (h->cfg.force_path == 1 || (h->warned & (1u << ti)) || !arx_tcn_supported(h, tr) || tc_admitted(h, tr)) return;
   h->warned |= 1u << ti;
-  fprintf(stderr, "libarx: transformers[%d].norm_k has a LayerNorm affine outside the fp16 tensor-core bound (|S| <= %.0f > %.0f): scoring on the "
-                  "fp32 CUDA-core kernels (about 30x slower) to stay within the 1e-3 tolerance; force_path=2 selects the tensor-core "
-                  "row-max variant at reduced accuracy\n", ti, (double)tr.softmax_bound, 100.0 / ARX_SOFTMAX_LOG2E);
+  fprintf(stderr, "libarx: transformers[%d].norm_k has a LayerNorm affine outside the fp16 tensor-core bound (|S| <= %.1f; accuracy "
+                  "bound %.1f, overflow bound %.1f): scoring on the fp32 CUDA-core kernels (about 30x slower) to stay within the "
+                  "1e-3 tolerance; force_path=2 selects the tensor-core kernels at reduced accuracy\n",
+          ti, (double)tr.softmax_bound, (double)accuracy_bound(tr), 100.0 / ARX_SOFTMAX_LOG2E);
 }
 
 // Decides transformer i's route and builds the support operands it reads: the tuple tensors ks/vs from the per-frame
@@ -1377,8 +1387,8 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
   ArxTransformer &tr = h->tr[0];
   const int way = h->way, NO = 2 * tr.c * h->D;
   const bool disc = h->cfg.has_discriminator != 0;
-  if (h->cfg.force_path == 1 || !arx_tcn_supported(h, tr) || arx_tcn_needs_rowmax(tr) || tr.c != 2 || (disc && h->T > 32) || h->J3 > 256 || h->H > 256 ||
-      h->F > 256)
+  if (h->cfg.force_path == 1 || !tc_admitted(h, tr) || !arx_tcn_supported(h, tr) || arx_tcn_needs_rowmax(tr) || tr.c != 2 || (disc && h->T > 32) ||
+      h->J3 > 256 || h->H > 256 || h->F > 256)
     return arx_fail(h, ARX_ERR_INVALID, "stream_push: the resident streaming path covers pair tuples on the tiled tcgen05 kernels only");
   ArxStream &s = h->stream;
   int rc;

@@ -9,6 +9,21 @@
 #include "../../include/arx.h"
 
 #define ARX_SOFTMAX_LOG2E 1.4426950408889634f
+// Two limits on the static softmax bound |S| <= (max|gamma| sqrt(D) + ||beta||_2)^2 / sqrt(D) of norm_k's LayerNorm
+// affine (ArxTransformer::softmax_bound):
+//   overflow: |S| log2(e) < 100 keeps exp2 without max-subtraction inside fp32 range.  It picks the row-max variant of
+//             the tiled kernels and bounds what the kernels without it may run on (arx_tc_supported, arx_tcn_needs_rowmax);
+//   accuracy: |S| below these keeps the fp16 QK^T and bf16 P.V operands within the 1e-3 relative tolerance.  It
+//             admits weights to the tensor-core routes by default (support_route, arx_stream_push).  Set from the B200
+//             sweep in profiles/r03_ln_bound_sweep.txt.  A logit averages the rounding error over the N query tuples, so
+//             at equal bound it falls like 1/sqrt(N), and the limit depends on N (DESIGN 4):
+//               N >= 120 (T=16 pairs and larger): the largest swept bound whose worst error is <= 0.6e-3 (19.1), headroom
+//                        for inputs the sweep did not draw;
+//               N < 120 (T=8 pairs): 2.5x the error at equal bound, 7e-4 already at gamma = 1 (11.3) and 1.1e-3 at 16.3;
+//                        this limit keeps gamma = 1 on the tensor cores and holds the tolerance itself, not 0.6e-3.
+#define ARX_TC_ACCURACY_BOUND 19.0f
+#define ARX_TC_ACCURACY_BOUND_FEW_TUPLES 12.0f
+#define ARX_TC_FEW_TUPLES 120
 
 // A linear layer prepared for the tcgen05 GEMM: fp16 weight image [n_tiles][nk][BN x 64] + zero-padded bias
 struct ArxTcLinear {

@@ -143,7 +143,7 @@ __global__ void k_finish_tc(const float *__restrict__ partial, float *__restrict
 }  // namespace
 
 bool arx_tc_supported(const arx_handle *h, const ArxTransformer &tr) {
-  // single-tile kernel: N <= 128; exp2 without max-subtraction needs the static LayerNorm bound to stay in fp32 range
+  // single-tile kernel: N <= 128; exp2 without max-subtraction needs the overflow bound on the LayerNorm affine
   return tr.N <= TILE && h->D == DD && tr.softmax_bound * ARX_SOFTMAX_LOG2E < 100.0f;
 }
 

@@ -52,7 +52,8 @@ __device__ __forceinline__ uint32_t ex2_bits(uint32_t x) {
 // exp2 of two pre-scaled scores on the FMA pipe instead of the MUFU (the co-limiting pipe): round-to-nearest split
 // x = n + f with the 1.5*2^23 magic constant, 2^f on [-0.5, 0.5] by a degree-3 polynomial (max relative error
 // 7.5e-5, far below the bf16 quantisation of P), exponent add by an integer shift-add.  |x| < 100 is guaranteed by
-// the LayerNorm bound checked at weight load (arx_tc_supported).
+// the overflow bound on the LayerNorm affine checked at weight load (arx_tc_supported), which also holds under
+// force_path = 2; by default the tighter accuracy bound (ARX_TC_ACCURACY_BOUND) keeps |x| far below it.
 __device__ __forceinline__ void exp2_poly2(uint32_t &a, uint32_t &b) {
   const uint64_t MAGIC = pack2(12582912.0f, 12582912.0f);
   const uint64_t x = pack2u(a, b);

@@ -779,7 +779,8 @@ __global__ void k_finish_n(const float *__restrict__ partial, float *__restrict_
 bool arx_tcn_supported(const arx_handle *h, const ArxTransformer &tr) {
   return h->D == DD && h->T <= 255 && tr.c >= 2 && tr.c <= 3;
 }
-// exp2 without a shift is only safe inside the static LayerNorm bound (SURVEY 7.2-1); outside it the ROWMAX variant runs
+// exp2 without a shift is only safe inside the overflow bound on the LayerNorm affine (SURVEY 7.2-1); past it the ROWMAX
+// variant runs.  Only force_path = 2 gets there: by default weights past the tighter accuracy bound score on the fp32 kernels.
 bool arx_tcn_needs_rowmax(const ArxTransformer &tr) { return !(tr.softmax_bound * ARX_SOFTMAX_LOG2E < 100.0f); }
 
 int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st) {
