@@ -133,13 +133,18 @@ ARX_API int arx_score_frames(arx_handle *h, const float *frames_dev, int64_t n_f
 
 /* TRXOS.forward in the training / evaluation call shape (modules/ar/utils/train.py:110-120,
  * modules/ar/utils/test/compute_fsos.py:89-98): every batch row is its own EPISODE -- query i is scored against
- * ITS OWN `way` support classes (model.py:59-148 never mixes batch rows).  All episodes go through the batched
- * kernels at once (the support operands of the n_episodes*way classes form one pool; window i attends classes
- * [i*way, (i+1)*way) of it).
+ * ITS OWN `way` support classes (model.py:59-148 never mixes batch rows).  On both tensor-core routes (the T=16 pair
+ * pipeline and the tiled kernels: T=32, other T, triples, debug bit 4096, force_path = 2 past the overflow bound)
+ * episodes go through the batched kernels a pass at a time: the support operands of the pass's episodes*way classes
+ * form one pool, and window i attends classes [i*way, (i+1)*way) of it.  A pass holds 256 episodes on the pair
+ * pipeline; on the tiled kernels as many as keep the pool within 1 GiB (at least one, at most 256).  The fp32 route
+ * (force_path = 1, LayerNorm affines past the accuracy bound, D != 128) scores one episode at a time.
+ * The pool holds the support operands of transformers[0] only, the transformer that scores episodes (model.py:320).
  *   support_dev (n_episodes, way, T, 3J) poses, or (n_episodes, way, T, F) frame features when is_features != 0
  *   (the ss_features argument); query_dev (n_episodes, T, 3J); outputs as arx_score.
- * REPLACES the handle's current support set (by the pool of the last pass): call arx_set_support_* again before
- * the next arx_score. */
+ * REPLACES the handle's current support set (by the pool of the last pass, transformers[0] only): call
+ * arx_set_support_* again before the next arx_score; until then arx_score_features(ti >= 1) and arx_export_support
+ * return ARX_ERR_STATE. */
 ARX_API int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_features, int32_t way, const float *query_dev,
                        int64_t n_episodes, float *logits_dev, float *is_true_dev, int32_t *chosen_dev, void *stream);
 

@@ -141,7 +141,8 @@ Fp32Ws carve_generic(arx_handle *h, const ArxTransformer &tr, int64_t n, int way
 }
 
 // Windows per pass (at most max_chunk, default 4096, and 3 GB of the layout carve(n, base)), the workspace for them and,
-// without the caller's chosen buffer, the argmax scratch after it.  one_pass (episode mode): more passes are unsupported.
+// without the caller's chosen buffer, the argmax scratch after it.  one_pass (episode mode of the T=16 pair pipeline, whose
+// kernels take no pool class offset): more passes are unsupported.
 template <class Ws, class Carve>
 int plan_chunks(arx_handle *h, int64_t n_windows, bool one_pass, const int32_t *chosen_dev, Carve &&carve, int64_t *chunk, Ws *w,
                 int32_t **chosen_ws) {
@@ -507,13 +508,14 @@ static int workspace_wait(arx_handle *h, cudaStream_t st) {
   return ARX_OK;
 }
 
-static int support_alloc(arx_handle *h, int way, cudaStream_t st) {
-  if (way <= h->way_cap) return ARX_OK;
+// support tensors of `way` classes for transformers [0, n_tr) (n_tr < n_transformers: the episode pool of arx_score_episodes)
+static int support_alloc(arx_handle *h, int way, int n_tr, cudaStream_t st) {
+  if (way <= h->way_cap && h->tr[n_tr - 1].ks) return ARX_OK;
   ARX_CUDA(h, cudaStreamSynchronize(st));
   ARX_CUDA(h, cudaDeviceSynchronize());
   free_support(h);
   int rc;
-  for (int i = 0; i < h->cfg.n_transformers; ++i) {
+  for (int i = 0; i < n_tr; ++i) {
     if ((rc = dev_alloc(h, &h->tr[i].ks, (size_t)way * h->tr[i].N * h->D))) return rc;
     if ((rc = dev_alloc(h, &h->tr[i].vs, (size_t)way * h->tr[i].N * h->D))) return rc;
   }
@@ -584,6 +586,9 @@ static void warn_fp32_fallback(arx_handle *h, int ti) {
           ti, (double)tr.softmax_bound, (double)accuracy_bound(tr), 100.0 / ARX_SOFTMAX_LOG2E);
 }
 
+// The tiled route builds the class tiles of the open-set head (Uc) for transformer i
+static bool tiled_head(const arx_handle *h, int i) { return i == 0 && h->cfg.has_discriminator && h->tr[i].c == 2 && h->T <= 32; }
+
 // Decides transformer i's route and builds the support operands it reads: the tuple tensors ks/vs from the per-frame
 // projections G (or, with G == nullptr, ks/vs are already in place: arx_import_support), the operand images and the
 // head's Uc of the pair pipeline, the class tiles of the tiled kernels.
@@ -598,17 +603,18 @@ static int support_operands(arx_handle *h, int i, const float *G, int way, cudaS
   if (rc) return rc;
   if (imgs && i == 0 && h->cfg.has_discriminator && (rc = arx_tc2_support_uc(h, tr, way, st))) return rc;
   if (tr.route == ARX_ROUTE_TILED) {
-    if ((rc = arx_tcn_prep_support(h, tr, way, i == 0 && h->cfg.has_discriminator && tr.c == 2 && h->T <= 32, st))) return rc;
+    if ((rc = arx_tcn_prep_support(h, tr, way, tiled_head(h, i), st))) return rc;
     h->tiles_gen[i] = h->support_seq + 1;
   }
   return ARX_OK;
 }
 
 // projection + tuple/LayerNorm/image build of the support set from frame features given as an fp16 image
-// (tensor-core path) or as fp32 rows (general path)
-static int support_from_features(arx_handle *h, const __half *f_img, const float *feats32, int way, float *G, cudaStream_t st) {
+// (tensor-core path) or as fp32 rows (general path), for transformers [0, n_tr); the others are left without operands
+static int support_from_features(arx_handle *h, const __half *f_img, const float *feats32, int way, int n_tr, float *G, cudaStream_t st) {
   int rc;
-  for (int i = 0; i < h->cfg.n_transformers; ++i) {
+  for (int i = n_tr; i < h->cfg.n_transformers; ++i) h->tr[i].route = ARX_ROUTE_NONE;
+  for (int i = 0; i < n_tr; ++i) {
     ArxTransformer &tr = h->tr[i];
     const int64_t rows = (int64_t)way * h->T;
     if (f_img) {
@@ -623,12 +629,9 @@ static int support_from_features(arx_handle *h, const __half *f_img, const float
   return ARX_OK;
 }
 
-int arx_set_support_features(arx_handle *h, const float *feats_dev, int32_t way, void *stream) {
-  if (!h || !feats_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
-  if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "set_support: weights not loaded");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+static int set_support_features(arx_handle *h, const float *feats_dev, int32_t way, int n_tr, cudaStream_t st) {
   int rc;
-  if ((rc = support_alloc(h, way, st))) return rc;
+  if ((rc = support_alloc(h, way, n_tr, st))) return rc;
   SupportScratch sc;
   if ((rc = support_scratch_reserve(h, way, &sc))) return rc;
   if ((rc = support_wait(h, st))) return rc;                       // a previous chain may still be writing ss_feat
@@ -641,20 +644,23 @@ int arx_set_support_features(arx_handle *h, const float *feats_dev, int32_t way,
     if ((rc = arx_tc_rows_to_img(h, h->ss_feat, h->F, h->F, (int64_t)way * h->T, sc.f_img, h->tr[0].tl_proj.nk,
                                  h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
       return rc;
-    rc = support_from_features(h, sc.f_img, nullptr, way, sc.G, ss);
+    rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
   } else {
-    rc = support_from_features(h, nullptr, h->ss_feat, way, sc.G, ss);
+    rc = support_from_features(h, nullptr, h->ss_feat, way, n_tr, sc.G, ss);
   }
   if (rc) return rc;
   return support_join_record(h);
 }
 
-int arx_set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, void *stream) {
-  if (!h || !poses_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
+int arx_set_support_features(arx_handle *h, const float *feats_dev, int32_t way, void *stream) {
+  if (!h || !feats_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
   if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "set_support: weights not loaded");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return set_support_features(h, feats_dev, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
+}
+
+static int set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, int n_tr, cudaStream_t st) {
   int rc;
-  if ((rc = support_alloc(h, way, st))) return rc;
+  if ((rc = support_alloc(h, way, n_tr, st))) return rc;
   SupportScratch sc;
   if ((rc = support_scratch_reserve(h, way, &sc))) return rc;
   const int64_t rows = (int64_t)way * h->T;
@@ -669,16 +675,22 @@ int arx_set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, vo
     if ((rc = embed_frames_tc(h, h->ss_poses, rows, sc.x_img, sc.h_img, sc.f_img, h->tr[0].tl_proj.nk,
                               h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
       return rc;
-    rc = support_from_features(h, sc.f_img, nullptr, way, sc.G, ss);
+    rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
   } else {
     // general path: arx_embed stages through the shared workspace, so it stays on the caller's stream
     if ((rc = arx_embed(h, h->ss_poses, rows, h->ss_feat, st))) return rc;
     h->ss_feat_valid = true;
     if ((rc = support_fork(h, st, &ss))) return rc;
-    rc = support_from_features(h, nullptr, h->ss_feat, way, sc.G, ss);
+    rc = support_from_features(h, nullptr, h->ss_feat, way, n_tr, sc.G, ss);
   }
   if (rc) return rc;
   return support_join_record(h);
+}
+
+int arx_set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, void *stream) {
+  if (!h || !poses_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
+  if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "set_support: weights not loaded");
+  return set_support_poses(h, poses_dev, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
 }
 
 static int support_features_materialise(arx_handle *h, cudaStream_t st) {
@@ -716,6 +728,10 @@ int arx_export_support(arx_handle *h, void *blob_dev, void *stream) {
   if (!h || !blob_dev) return arx_fail(h, ARX_ERR_INVALID, "export_support: bad argument");
   if (h->way < 1) return arx_fail(h, ARX_ERR_STATE, "export_support: no support set");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  for (int i = 0; i < h->cfg.n_transformers; ++i)
+    if (h->tr[i].route == ARX_ROUTE_NONE)
+      return arx_fail(h, ARX_ERR_STATE, "export_support: transformers[%d] has no support operands (arx_score_episodes keeps those of "
+                                        "transformers[0] only): set the support set again", i);
   int rc = support_wait(h, st);                       // the chain that produces ks/vs runs on the side stream
   if (rc) return rc;
   float *p = static_cast<float *>(blob_dev);
@@ -733,7 +749,7 @@ int arx_import_support(arx_handle *h, const void *blob_dev, int32_t way, void *s
   if (!h || !blob_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "import_support: bad argument");
   if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "import_support: weights not loaded");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int rc = support_alloc(h, way, st);
+  int rc = support_alloc(h, way, h->cfg.n_transformers, st);
   if (rc) return rc;
   // like set_support: the copies and the operand-image builds run on the side stream (after everything queued on
   // `st`, i.e. after the collective that filled the blob), overlapped with the query-side kernels of the next score
@@ -879,27 +895,30 @@ static TcnWs carve_tcn(arx_handle *h, const ArxTransformer &tr, int64_t n, int w
 }
 
 // query tiles -> cross-attention -> logits / argmax -> open-set head, from the row-major per-frame projections w.G
+// ep_way > 0: episode mode, window w of this pass attends pool classes [cls_base + w*way, cls_base + (w+1)*way)
 static int tcn_backend(arx_handle *h, const ArxTransformer &tr, const TcnWs &w, int64_t n, int way, bool tcl, float *logits, float *is_true,
-                       int32_t *ch, cudaStream_t st) {
+                       int32_t *ch, int ep_way, int64_t cls_base, cudaStream_t st) {
   const int ldg = 2 * tr.c * h->D;
   int rc;
   if ((rc = support_wait(h, st))) return rc;          // tup_packed and the class tiles come from the support chain
   if ((rc = arx_tcn_prep_query(h, tr, w.G, ldg, n, w.kq, st))) return rc;
   if ((rc = prof_mark(h, 3, st))) return rc;
-  if ((rc = arx_tcn_attention(h, tr, w.kq, w.G, ldg, n, way, w.partial, logits, ch, w.vq, st))) return rc;
+  if ((rc = arx_tcn_attention(h, tr, w.kq, w.G, ldg, n, way, w.partial, logits, ch, w.vq, ep_way > 0, cls_base, st))) return rc;
   if ((rc = prof_mark(h, 4, st))) return rc;
   if (!is_true) return ARX_OK;
   if (tcl && ((int64_t)tr.N * h->T) % 64)       // fc1's K is padded to whole 64-column sub-tiles: the pad columns must be zero, not stale
     ARX_CUDA(h, cudaMemsetAsync(w.y_img, 0, (size_t)((n + 127) / 128 * 128) * h->tl_d1.nk * 64 * sizeof(__half), st));
-  if ((rc = arx_tcn_head(h, tr, w.kq, w.G, ldg, n, ch, w.uab, w.y, w.y_img, tcl ? h->tl_d1.nk : 0, w.vq_head, st))) return rc;
+  if ((rc = arx_tcn_head(h, tr, w.kq, w.G, ldg, n, ch, w.uab, w.y, w.y_img, tcl ? h->tl_d1.nk : 0, w.vq_head, ep_way, cls_base, st))) return rc;
   return tcl ? disc_tail_tc(h, w.y_img, w.h1_img, n, is_true, st) : disc_tail_fp32(h, tr, w.y, w.h1, w.h2, n, is_true, st);
 }
 
+// ep_way > 0: episode mode -- window b attends classes [b*ep_way, (b+1)*ep_way) of the support pool; the windows may
+// still be split into several passes (the kernels take the pass's first pool class)
 static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
-                     float *is_true_dev, int32_t *chosen_dev, cudaStream_t st, bool frames_stream = false) {
+                     float *is_true_dev, int32_t *chosen_dev, cudaStream_t st, int ep_way, bool frames_stream = false) {
   const ArxTransformer &tr = h->tr[ti];
   const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr, tcl = h->tc_linears && (h->tc_variant & 4) == 0;
-  const int way = h->way;
+  const int way = ep_way > 0 ? ep_way : h->way;
   if (!tr.kc_tiles) return arx_fail(h, ARX_ERR_STATE, "score: support operands of the tiled kernels are missing (set the support set again)");
   if (disc && !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "score: the open-set head of the tiled kernels needs pair tuples and T <= 32");
   int64_t chunk;
@@ -938,7 +957,8 @@ static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float 
     } else if ((rc = front_end_fp32(h, tr, query_dev, qfeats_dev, b0, rows, w.H1, w.FE, w.G, st))) return rc;
     if ((rc = prof_mark(h, 2, st))) return rc;
     int32_t *ch = chosen_dev ? chosen_dev + b0 : chosen_ws;
-    if ((rc = tcn_backend(h, tr, w, n, way, tcl, logits_dev + b0 * way, is_true_dev ? is_true_dev + b0 : nullptr, ch, st))) return rc;
+    if ((rc = tcn_backend(h, tr, w, n, way, tcl, logits_dev + b0 * way, is_true_dev ? is_true_dev + b0 : nullptr, ch, ep_way, b0 * way, st)))
+      return rc;
     if ((rc = prof_mark(h, 5, st))) return rc;
   }
   return ARX_OK;
@@ -1106,15 +1126,18 @@ static int score_impl(arx_handle *h, int ti, const float *query_dev, const float
   if (disc && (!h->cfg.has_discriminator || ti != 0 || tr.c != 2))
     return arx_fail(h, ARX_ERR_INVALID, "score: the discriminator is sized for pair tuples of transformers[0] (model.py:283-285)");
   if (ep_way > 0 && (int64_t)ep_way * n_windows != h->way) return arx_fail(h, ARX_ERR_STATE, "score: episode pool does not match the batch");
+  if (tr.route == ARX_ROUTE_NONE)
+    return arx_fail(h, ARX_ERR_STATE, "score: transformers[%d] has no support operands (arx_score_episodes keeps those of transformers[0] "
+                                      "only): set the support set again", ti);
   const bool debug_out = probs || protos;
   const ArxRoute route = debug_out ? ARX_ROUTE_FP32 : tr.route;      // only the fp32 kernels write the debug outputs
-  if (ep_way > 0 && (route != ARX_ROUTE_PAIR || !query_dev)) return ARX_EP_UNSUPPORTED;
+  if (ep_way > 0 && (route == ARX_ROUTE_FP32 || !query_dev)) return ARX_EP_UNSUPPORTED;
   int rc = workspace_wait(h, st);
   if (rc) return rc;
   if (route == ARX_ROUTE_PAIR)
     rc = score_gen3(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, ep_way, frames_stream);
   else if (route == ARX_ROUTE_TILED)
-    rc = score_tcn(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, frames_stream);
+    rc = score_tcn(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, ep_way, frames_stream);
   else if (frames_stream)
     rc = ARX_EP_UNSUPPORTED;            // the caller materialises the windows for the fp32 kernels
   else if (h->cfg.force_path == 2 && !debug_out)
@@ -1135,6 +1158,24 @@ int arx_score(arx_handle *h, const float *query_dev, int64_t n_windows, float *l
                     static_cast<cudaStream_t>(stream));
 }
 
+// Support pool of arx_score_episodes on the tiled route: a pass scores `piece` episodes against one pool of piece*way
+// support classes, and piece is chosen so that the pool takes at most this many bytes (at most 256 episodes, at least one).
+static const size_t ARX_EPISODE_POOL_BUDGET = (size_t)1 << 30;
+
+// Device bytes of one class of that pool (transformer 0 only): the fp32 tuple tensors ks / vs, the class tiles Kc and
+// Vc^T (and Uc for the open-set head), its rows of ss_feat and ss_poses, and its rows of the support scratch.  At T=32,
+// F=256, 30 joints: pairs with the head (temp_set [2, 3], scratch sized for triples) 1 084 674 B, 49 episodes of 20-way
+// per pass; triples (N=4960, temp_set [3]) 7 818 498 B, 6 episodes of 20-way per pass.
+static size_t tiled_pool_class_bytes(arx_handle *h) {
+  const ArxTransformer &tr = h->tr[0];
+  const size_t tile = 128 * 128 * sizeof(__half), ns = tr.Npad / 128;
+  size_t b = 2 * (size_t)tr.N * h->D * sizeof(float);
+  b += (tiled_head(h, 0) ? 3 : 2) * ns * tile;
+  b += (size_t)h->T * (h->F + h->J3) * sizeof(float);
+  b += support_scratch(h, 128, nullptr).bytes / 128;
+  return b;
+}
+
 int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_features, int32_t way, const float *query_dev, int64_t n_episodes,
                        float *logits_dev, float *is_true_dev, int32_t *chosen_dev, void *stream) {
   if (!h || !support_dev || !query_dev || !logits_dev || way < 1 || n_episodes < 0) return arx_fail(h, ARX_ERR_INVALID, "score_episodes: bad argument");
@@ -1142,25 +1183,37 @@ int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_featu
   if (!h->cfg.has_discriminator) is_true_dev = nullptr;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const size_t per_class = (size_t)h->T * (is_features ? h->F : h->J3);
-  const int64_t piece = 256;                 // episodes per pass: the pool holds piece*way classes of support operands
+  // support operands of transformers[0] only: episodes are scored by it alone (model.py:320)
+  auto set_support = [&](int64_t e0, int64_t n_classes) -> int {
+    const float *sup = support_dev + (size_t)e0 * way * per_class;
+    return is_features ? set_support_features(h, sup, (int32_t)n_classes, 1, st) : set_support_poses(h, sup, (int32_t)n_classes, 1, st);
+  };
+  auto one_at_a_time = [&](int64_t e0, int64_t e1) -> int {      // the same kernels as set_support + arx_score
+    for (int64_t e = e0; e < e1; ++e) {
+      int rc = set_support(e, way);
+      if (rc) return rc;
+      rc = score_impl(h, 0, query_dev + (size_t)e * h->T * h->J3, nullptr, 1, logits_dev + e * way, is_true_dev ? is_true_dev + e : nullptr,
+                      chosen_dev ? chosen_dev + e : nullptr, nullptr, nullptr, st);
+      if (rc) return rc;
+    }
+    return ARX_OK;
+  };
+  // The route depends on the configuration and the weights only: decided before any pool is built.  The fp32 kernels
+  // (force_path = 1, LayerNorm affines past the accuracy bound, D != 128) have no episode mode.
+  const ArxRoute route = support_route(h, h->tr[0]);
+  if (route == ARX_ROUTE_FP32) return one_at_a_time(0, n_episodes);
+  // The pair pipeline keeps 256 episodes per pass; the tiled route sizes its pool by ARX_EPISODE_POOL_BUDGET.
+  const int64_t piece = route == ARX_ROUTE_PAIR
+                            ? 256
+                            : std::max<int64_t>(1, std::min<int64_t>(256, (int64_t)(ARX_EPISODE_POOL_BUDGET / ((size_t)way * tiled_pool_class_bytes(h)))));
   for (int64_t e0 = 0; e0 < n_episodes; e0 += piece) {
     const int64_t m = std::min(piece, n_episodes - e0);
-    const float *sup = support_dev + (size_t)e0 * way * per_class;
-    int rc = is_features ? arx_set_support_features(h, sup, (int32_t)(m * way), stream) : arx_set_support_poses(h, sup, (int32_t)(m * way), stream);
+    int rc = set_support(e0, m * way);
     if (rc) return rc;
     rc = score_impl(h, 0, query_dev + (size_t)e0 * h->T * h->J3, nullptr, m, logits_dev + e0 * way, is_true_dev ? is_true_dev + e0 : nullptr,
                     chosen_dev ? chosen_dev + e0 : nullptr, nullptr, nullptr, st, way);
-    if (rc == ARX_EP_UNSUPPORTED) {
-      // shapes without the batched-episode kernels (other T / cardinality / fp32 path): one episode at a time, same kernels as arx_score
-      for (int64_t e = e0; e < e0 + m; ++e) {
-        const float *se = support_dev + (size_t)e * way * per_class;
-        rc = is_features ? arx_set_support_features(h, se, way, stream) : arx_set_support_poses(h, se, way, stream);
-        if (rc) return rc;
-        rc = score_impl(h, 0, query_dev + (size_t)e * h->T * h->J3, nullptr, 1, logits_dev + e * way, is_true_dev ? is_true_dev + e : nullptr,
-                        chosen_dev ? chosen_dev + e : nullptr, nullptr, nullptr, st);
-        if (rc) return rc;
-      }
-    } else if (rc) return rc;
+    if (rc == ARX_EP_UNSUPPORTED) rc = one_at_a_time(e0, e0 + m);      // pair pipeline: max_chunk below the pass
+    if (rc) return rc;
   }
   return ARX_OK;
 }
@@ -1461,7 +1514,7 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
       if ((rc = arx_tcn_head_all(h, tr, w.kq, w.G, ldg, way, s.iota, w.uab, s.y_all, w.vq_head, s.st2))) return rc;
       ARX_CUDA(h, cudaEventRecord(s.ev_join, s.st2));
     }
-    if ((rc = arx_tcn_attention_partial(h, tr, w.kq, w.G, ldg, 1, way, w.partial, w.vq, s.st))) return rc;
+    if ((rc = arx_tcn_attention_partial(h, tr, w.kq, w.G, ldg, 1, way, w.partial, w.vq, false, 0, s.st))) return rc;
     if ((rc = prof_mark(h, 4, s.st))) return rc;
     if (disc) ARX_CUDA(h, cudaStreamWaitEvent(s.st, s.ev_join, 0));
     if ((rc = arx_stream_tail_launch(h, tr, w.partial, s.y_all, w.h1, s.logits, s.out_dev, s.slot, way, s.st))) return rc;

@@ -327,14 +327,14 @@ bool arx_tcn_needs_rowmax(const ArxTransformer &tr);
 int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st);
 int arx_tcn_prep_query(arx_handle *h, const ArxTransformer &tr, const float *G, int ldg, int64_t n_win, __half *kq_tiles, cudaStream_t st);
 int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
-                      float *partial, float *logits, int32_t *chosen, __half *vq_ws, cudaStream_t st);
+                      float *partial, float *logits, int32_t *chosen, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st);
 int arx_tcn_head(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, const int32_t *chosen,
-                 float *uab, float *y, __half *y_img, int y_nk, __half *vq_ws, cudaStream_t st);
+                 float *uab, float *y, __half *y_img, int y_nk, __half *vq_ws, int ep_way, int64_t cls_base, cudaStream_t st);
 
 int arx_tcn_head_all(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int way, const int32_t *iota,
                      float *uab, float *y_all, __half *vq_ws, cudaStream_t st);
 int arx_tcn_attention_partial(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
-                              float *partial, __half *vq_ws, cudaStream_t st);
+                              float *partial, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st);
 
 // ---- streaming kernels (arx_stream.cu)
 int arx_stream_frame_launch(arx_handle *h, const ArxTransformer &tr, const float *x_dev, float *ring, int *slot_next, cudaStream_t st);

@@ -26,6 +26,8 @@
 // straight into the fp16 activation image of discriminator.fc1.
 // ROWMAX variant: subtracts a running row maximum before exp2 (online rescaling of Z across query tiles), for
 // LayerNorm affines outside the static bound under which exp2 needs no shift (SURVEY 7.2-1).
+// Episode mode (arx_score_episodes): every window has its own support classes, window w of a launch attends classes
+// [cls_base + w*way, cls_base + (w+1)*way) of one pool of class tiles; the query side and the head are per window as always.
 // Work unit = (window, class), round-robin over one persistent CTA per SM; 16 warps, warp-specialised; every
 // mbarrier wait carries a watchdog (a protocol bug traps instead of hanging the GPU).
 #include "arx_internal.cuh"
@@ -69,6 +71,11 @@ struct AttnNParams {
   int free_a;               // pass A: the softmax groups run free instead of taking turns on the MUFU phase
   int poly;                 // pass A: every other register pair takes the FMA-pipe exp2 polynomial
   int same_window;          // mode 1: every unit scores window 0 (against class chosen[u]); y row = u (streaming: the head of ALL classes at once)
+  // class tiles of unit u: cls_base + u % cls_mod (mode 0), cls_base + u*cls_stride + chosen[u] (mode 1).  Ordinary launches:
+  // cls_base = cls_stride = 0, cls_mod = way.  Episode mode (a pool of per-window support sets): window w of the launch attends
+  // pool classes [cls_base + w*way, cls_base + (w+1)*way), so cls_mod = n_win*way (no wrap) and cls_stride = way
+  // (`chosen` stays in [0, way): the argmax within the episode)
+  int cls_base, cls_mod, cls_stride;
 };
 
 // Watchdog wait: a protocol bug must not hang the GPU.  On a timeout (~1 s) the first thread to notice records
@@ -157,7 +164,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_attn_tcn(const AttnNParams p) {
         int k = 0, kr = 0;                     // kr: items of the Vc ring (selection operands and Vc^T tiles alike)
         for (int ui = 0; ui < my_units; ++ui) {
           const int u = blockIdx.x + ui * gridDim.x;
-          const size_t cls = head ? (size_t)p.chosen[u] : (size_t)(u % p.way);
+          const size_t cls = (size_t)p.cls_base + (head ? (size_t)u * p.cls_stride + p.chosen[u] : (size_t)(u % p.cls_mod));
           const size_t win = head ? (p.same_window ? 0 : (size_t)u) : (size_t)(u / p.way);
           const uint8_t *kc0 = reinterpret_cast<const uint8_t *>(p.kc_img) + cls * ns * IMG_BYTES;
           const uint8_t *vc0 = reinterpret_cast<const uint8_t *>(p.vct_img) + cls * ns * IMG_BYTES;
@@ -824,6 +831,7 @@ int arx_tcn_prep_query(arx_handle *h, const ArxTransformer &tr, const float *G, 
 }
 
 static int tcn_launch(arx_handle *h, const ArxTransformer &tr, AttnNParams &p, int n_units, cudaStream_t st) {
+  if (p.same_window && p.cls_stride) return arx_fail(h, ARX_ERR_INVALID, "tiled attention kernel: same_window and episode mode do not combine");
   const int grid = n_units < h->sm_count ? n_units : h->sm_count;
   // two regions: a head launch may run beside a main launch on another stream (streaming path)
   const size_t zhalf = (size_t)h->sm_count * 2 * 2 * 2 * tr.Npad, zbytes = 2 * zhalf * sizeof(float);
@@ -879,9 +887,10 @@ static int tcn_prep_vq(arx_handle *h, const ArxTransformer &tr, const float *tab
   return ARX_OK;
 }
 
-// squared-distance partials only (the streaming tail forms logits / argmax itself)
+// squared-distance partials only (the streaming tail forms logits / argmax itself).  episodes: window w attends the pool
+// classes [cls_base + w*way, cls_base + (w+1)*way) instead of classes [0, way)
 int arx_tcn_attention_partial(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
-                              float *partial, __half *vq_ws, cudaStream_t st) {
+                              float *partial, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st) {
   int rc = tcn_prep_vq(h, tr, G, ldg, tr.c * h->D, h->D, 128, n_win, vq_ws, st);
   if (rc) return rc;
   AttnNParams p{};
@@ -889,13 +898,14 @@ int arx_tcn_attention_partial(arx_handle *h, const ArxTransformer &tr, const __h
   p.partial = partial;
   p.n_win = (int)n_win; p.way = way; p.N = tr.N; p.T = h->T; p.c = tr.c; p.nq = p.ns = tr.Npad / 128;
   p.mode = 0;
+  p.cls_base = episodes ? (int)cls_base : 0; p.cls_mod = episodes ? (int)n_win * way : way;
   return tcn_launch(h, tr, p, (int)n_win * way, st);
 }
 
 // logits (n_win, way) and chosen (n_win) of transformer `tr` from the query tiles; G = row-major per-frame projections
 int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
-                      float *partial, float *logits, int32_t *chosen, __half *vq_ws, cudaStream_t st) {
-  int rc = arx_tcn_attention_partial(h, tr, kq_tiles, G, ldg, n_win, way, partial, vq_ws, st);
+                      float *partial, float *logits, int32_t *chosen, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st) {
+  int rc = arx_tcn_attention_partial(h, tr, kq_tiles, G, ldg, n_win, way, partial, vq_ws, episodes, cls_base, st);
   if (rc) return rc;
   k_finish_n<<<(unsigned)((n_win + 127) / 128), 128, 0, st>>>(partial, logits, chosen, n_win, way, tr.N);
   ARX_LAUNCH_CHECK(h);
@@ -920,9 +930,10 @@ int arx_tcn_head_all(arx_handle *h, const ArxTransformer &tr, const __half *kq_t
   return tcn_launch(h, tr, p, way, st);
 }
 
-// open-set head input y = dimensionality_reduction(diff of the winning class) (model.py:323-324,196), pair tuples
+// open-set head input y = dimensionality_reduction(diff of the winning class) (model.py:323-324,196), pair tuples.
+// ep_way > 0: episode mode, window w's winner chosen[w] is class cls_base + w*ep_way + chosen[w] of the pool
 int arx_tcn_head(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, const int32_t *chosen,
-                 float *uab, float *y, __half *y_img, int y_nk, __half *vq_ws, cudaStream_t st) {
+                 float *uab, float *y, __half *y_img, int y_nk, __half *vq_ws, int ep_way, int64_t cls_base, cudaStream_t st) {
   if (tr.c != 2 || h->T > 32 || !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "tcn_head: pair tuples with T <= 32 only");
   k_head_uab<<<(unsigned)std::min<int64_t>((n_win * h->T + 3) / 4, 4 * h->sm_count), 256, 0, st>>>(G, ldg, tr.c * h->D, h->dr_w, h->dr_b, uab, n_win * h->T,
                                                                                                        h->T);
@@ -935,5 +946,6 @@ int arx_tcn_head(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles
   p.y = y; p.y_img = y_img; p.y_nk = y_nk; p.L = h->T;
   p.n_win = (int)n_win; p.way = 1; p.N = tr.N; p.T = h->T; p.c = tr.c; p.nq = p.ns = tr.Npad / 128;
   p.mode = 1;
+  p.cls_base = ep_way > 0 ? (int)cls_base : 0; p.cls_stride = ep_way > 0 ? ep_way : 0;
   return tcn_launch(h, tr, p, (int)n_win, st);
 }

@@ -11,7 +11,9 @@ This module reproduces that arithmetic over any iterable of episode batches in t
 (`support_set`/`target_set` dicts keyed "sk", `support_classes`, `target_class`, `known`); the dataset I/O itself is out
 of scope (SURVEY.md section 2 row 8), so `synthetic_fsos_episodes` provides loader-shaped synthetic episodes.  The
 model argument is anything with the reference `forward(ss_data, ss_labels, query_data)` signature: the CUDA `TRXOS`
-of this package scores every batch in one batched-episode pass (`arx_score_episodes`).
+of this package scores every batch through `arx_score_episodes`, in batched-episode passes on both tensor-core routes
+(T=16 pairs: 256 episodes per pass; the tiled kernels, e.g. the T=32 cfg4 shape: as many episodes as keep the support
+pool within 1 GiB) and one episode at a time on the fp32 route.
 """
 from __future__ import annotations
 
