@@ -119,7 +119,10 @@ ARX_API int arx_import_support(arx_handle *h, const void *blob_dev, int32_t way,
  * support set, transformers[0] + discriminator:
  *   query_dev (B,T,3J) -> logits_dev (B,W) [= -distance], is_true_dev (B) in (0,1)
  *   [may be NULL / ignored without discriminator], chosen_dev (B) int32 argmax
- *   (first maximum on ties, model.py:323) [may be NULL]. */
+ *   (first maximum on ties, model.py:323) [may be NULL].
+ * The discriminator is sized for pair tuples (model.py:282-285): is_true needs temp_set[0] = 2.  On the tiled tcgen05
+ * kernels the open-set head covers every seq_len the handle accepts (2..64); the head's T columns are accumulator lanes
+ * of the attention kernel's head mode. */
 ARX_API int arx_score(arx_handle *h, const float *query_dev, int64_t n_windows,
               float *logits_dev, float *is_true_dev, int32_t *chosen_dev, void *stream);
 
@@ -187,7 +190,8 @@ ARX_API int arx_score_host_wait(arx_handle *h, int64_t ticket);
  * window's per-frame projections as ring + positional table, scores the window against the current support set
  * (transformers[0] + discriminator) and returns result_host[0..way) = softmax(logits) (ar.py:77), result_host[way] = is_true
  * (ar.py:78).  *valid = 0 until seq_len frames have been pushed since the last reset (ar.py:43-44).  One H2D (the frame),
- * one CUDA-graph launch and one D2H per call; synchronises the handle's internal stream.  Pair tuples only.
+ * one CUDA-graph launch and one D2H per call; synchronises the handle's internal stream.  Pair tuples only (with or
+ * without the discriminator, any seq_len up to 64), on the tiled tcgen05 kernels.
  * arx_stream_reset forgets the window (previous_frames = []). */
 ARX_API int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, int32_t *valid);
 ARX_API int arx_stream_reset(arx_handle *h);

@@ -587,7 +587,7 @@ static void warn_fp32_fallback(arx_handle *h, int ti) {
 }
 
 // The tiled route builds the class tiles of the open-set head (Uc) for transformer i
-static bool tiled_head(const arx_handle *h, int i) { return i == 0 && h->cfg.has_discriminator && h->tr[i].c == 2 && h->T <= 32; }
+static bool tiled_head(const arx_handle *h, int i) { return i == 0 && h->cfg.has_discriminator && arx_tcn_head_supported(h, h->tr[i]); }
 
 // Decides transformer i's route and builds the support operands it reads: the tuple tensors ks/vs from the per-frame
 // projections G (or, with G == nullptr, ks/vs are already in place: arx_import_support), the operand images and the
@@ -879,7 +879,7 @@ static TcnWs carve_tcn(arx_handle *h, const ArxTransformer &tr, int64_t n, int w
   w.vq_head = disc ? c.take<__half>((size_t)n * nsel * 8192) : nullptr;
   if (disc) {
     const int64_t K1 = (int64_t)tr.N * h->T;
-    w.uab = c.take<float>(rows * 64 + 256);
+    w.uab = c.take<float>(rows * 2 * arx_tcn_head_cols(h->T) + 256);
     if (tcl) {
       w.y_img = c.take<__half>(n_pad * (int64_t)h->tl_d1.nk * 64);
       w.h1_img = c.take<__half>(n_pad * 256);
@@ -920,7 +920,7 @@ static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float 
   const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr, tcl = h->tc_linears && (h->tc_variant & 4) == 0;
   const int way = ep_way > 0 ? ep_way : h->way;
   if (!tr.kc_tiles) return arx_fail(h, ARX_ERR_STATE, "score: support operands of the tiled kernels are missing (set the support set again)");
-  if (disc && !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "score: the open-set head of the tiled kernels needs pair tuples and T <= 32");
+  if (disc && !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "score: the open-set head of the tiled kernels needs pair tuples and T <= 64");
   int64_t chunk;
   TcnWs w;
   int32_t *chosen_ws;
@@ -1165,7 +1165,8 @@ static const size_t ARX_EPISODE_POOL_BUDGET = (size_t)1 << 30;
 // Device bytes of one class of that pool (transformer 0 only): the fp32 tuple tensors ks / vs, the class tiles Kc and
 // Vc^T (and Uc for the open-set head), its rows of ss_feat and ss_poses, and its rows of the support scratch.  At T=32,
 // F=256, 30 joints: pairs with the head (temp_set [2, 3], scratch sized for triples) 1 084 674 B, 49 episodes of 20-way
-// per pass; triples (N=4960, temp_set [3]) 7 818 498 B, 6 episodes of 20-way per pass.
+// per pass; triples (N=4960, temp_set [3]) 7 818 498 B, 6 episodes of 20-way per pass.  T=64 pairs with the head (N=2016,
+// temp_set [2]): 3 938 818 B, 13 episodes of 20-way per pass.
 static size_t tiled_pool_class_bytes(arx_handle *h) {
   const ArxTransformer &tr = h->tr[0];
   const size_t tile = 128 * 128 * sizeof(__half), ns = tr.Npad / 128;
@@ -1440,7 +1441,7 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
   ArxTransformer &tr = h->tr[0];
   const int way = h->way, NO = 2 * tr.c * h->D;
   const bool disc = h->cfg.has_discriminator != 0;
-  if (h->cfg.force_path == 1 || !tc_admitted(h, tr) || !arx_tcn_supported(h, tr) || arx_tcn_needs_rowmax(tr) || tr.c != 2 || (disc && h->T > 32) ||
+  if (h->cfg.force_path == 1 || !tc_admitted(h, tr) || !arx_tcn_supported(h, tr) || arx_tcn_needs_rowmax(tr) || tr.c != 2 ||
       h->J3 > 256 || h->H > 256 || h->F > 256)
     return arx_fail(h, ARX_ERR_INVALID, "stream_push: the resident streaming path covers pair tuples on the tiled tcgen05 kernels only");
   ArxStream &s = h->stream;

@@ -324,6 +324,10 @@ int arx_tuple_img(arx_handle *h, const ArxTransformer &tr, const float *gc, int 
 // ---- tiled any-N tcgen05 attention (arx_tcn.cu)
 bool arx_tcn_supported(const arx_handle *h, const ArxTransformer &tr);
 bool arx_tcn_needs_rowmax(const ArxTransformer &tr);
+// the open-set head on the tiled kernels: pair tuples, head columns L = T <= 64 (TMEM lanes of the MODE 1 accumulator)
+bool arx_tcn_head_supported(const arx_handle *h, const ArxTransformer &tr);
+// columns per frame part of the head table UAB (row stride 2x this): 32 for T <= 32, 64 above
+int arx_tcn_head_cols(int T);
 int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st);
 int arx_tcn_prep_query(arx_handle *h, const ArxTransformer &tr, const float *G, int ldg, int64_t n_win, __half *kq_tiles, cudaStream_t st);
 int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,

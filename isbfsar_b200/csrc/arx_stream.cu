@@ -118,6 +118,9 @@ __global__ void __launch_bounds__(256) k_stream_tiles(const float *__restrict__ 
 // logits / argmax of ONE window from the distance partials (model.py:131-135,323: first maximum wins), then discriminator
 // fc1 (model.py:198) on the winning class's head input: h1 = relu(W1 y + b1), 256 x (N*T).  One warp per output row, the
 // row read as independent 16-byte loads (15 per lane at T=16).  Block 0 also publishes the logits.
+// K = N*T = T^2 (T-1) / 2 is a multiple of 4 only for T = 0 (mod 4) or T = 1 (mod 8).  For other K the rows of W1 and y start
+// at different offsets from a 16-byte boundary: a scalar head brings the row of W1 to its boundary, the body reads it as
+// float4 and y as scalars, and a scalar tail ends the row.
 __global__ void __launch_bounds__(256) k_stream_fc1(const float *__restrict__ partial, const float *__restrict__ y_all, const float *__restrict__ w,
                                                     const float *__restrict__ b, float *__restrict__ h1, float *__restrict__ logits, int K, int way,
                                                     int N, int has_disc) {
@@ -130,16 +133,33 @@ __global__ void __launch_bounds__(256) k_stream_fc1(const float *__restrict__ pa
     if (lg > best) { best = lg; bi = c; }
   }
   if (!has_disc) return;
-  const float4 *y = reinterpret_cast<const float4 *>(y_all + (size_t)bi * K);
   const int lane = threadIdx.x & 31, row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= 256) return;
-  const float4 *wr = reinterpret_cast<const float4 *>(w + (size_t)row * K);
   float a0 = 0.f, a1 = 0.f;
+  if ((K & 3) == 0) {
+    const float4 *y = reinterpret_cast<const float4 *>(y_all + (size_t)bi * K);
+    const float4 *wr = reinterpret_cast<const float4 *>(w + (size_t)row * K);
 #pragma unroll 8
-  for (int k = lane; k < K / 4; k += 32) {
-    const float4 wv = __ldg(wr + k), yv = __ldg(y + k);
-    a0 = fmaf(wv.x, yv.x, fmaf(wv.y, yv.y, a0));
-    a1 = fmaf(wv.z, yv.z, fmaf(wv.w, yv.w, a1));
+    for (int k = lane; k < K / 4; k += 32) {
+      const float4 wv = __ldg(wr + k), yv = __ldg(y + k);
+      a0 = fmaf(wv.x, yv.x, fmaf(wv.y, yv.y, a0));
+      a1 = fmaf(wv.z, yv.z, fmaf(wv.w, yv.w, a1));
+    }
+  } else {
+    const float *y = y_all + (size_t)bi * K, *wr = w + (size_t)row * K;
+    const int hd = (int)((4u - (uint32_t)(((size_t)row * K) & 3u)) & 3u), nb = (K - hd) >> 2;   // w itself is 16-byte aligned
+    if (lane < hd) a0 = __ldg(wr + lane) * __ldg(y + lane);
+    const float4 *w4 = reinterpret_cast<const float4 *>(wr + hd);
+    const float *yb = y + hd;
+#pragma unroll 4
+    for (int k = lane; k < nb; k += 32) {
+      const float4 wv = __ldg(w4 + k);
+      const float *yk = yb + 4 * k;
+      a0 = fmaf(wv.x, __ldg(yk), fmaf(wv.y, __ldg(yk + 1), a0));
+      a1 = fmaf(wv.z, __ldg(yk + 2), fmaf(wv.w, __ldg(yk + 3), a1));
+    }
+    const int k = hd + 4 * nb + lane;
+    if (k < K) a1 = fmaf(__ldg(wr + k), __ldg(y + k), a1);
   }
   float a = a0 + a1;
 #pragma unroll
@@ -247,7 +267,6 @@ int arx_stream_tail_launch(arx_handle *h, const ArxTransformer &tr, const float 
                            int *slot_next, int way, cudaStream_t st) {
   const int disc = h->cfg.has_discriminator ? 1 : 0;
   const int K1 = tr.N * h->T;
-  if (disc && (K1 & 3)) return arx_fail(h, ARX_ERR_INVALID, "stream: N*T must be a multiple of 4");
   k_stream_fc1<<<disc ? 32 : 1, 256, 0, st>>>(partial, y_all, h->d1_w, h->d1_b, h1, logits, K1, way, tr.N, disc);
   ARX_LAUNCH_CHECK(h);
   k_stream_tail<<<1, 256, 0, st>>>(h1, h->d2_w, h->d2_b, h->d3_w, h->d3_b, logits, out, slot_next, way, h->T, disc);

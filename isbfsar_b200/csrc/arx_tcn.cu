@@ -635,7 +635,9 @@ __global__ void __launch_bounds__(256) k_prep_vct_tiles(const float *__restrict_
   }
 }
 
-// Head operand Uc tiles (bf16): rows l < L hold sum_d Wdr[l][d].Vc[s][d], rows >= L are zero.  grid (way, ns), 128 threads (one per s)
+// Head operand Uc tiles (bf16): rows l < L hold sum_d Wdr[l][d].Vc[s][d], rows >= L are zero.  grid (way, ns), 128 threads (one per s).
+// LMAX >= L: the rows one thread keeps in registers (32 for T <= 32, 64 for T <= 64; the 32-row instance is the one T <= 32 always ran)
+template <int LMAX>
 __global__ void __launch_bounds__(128) k_prep_uc_tiles(const float *__restrict__ vs, const float *__restrict__ dr_w, __half *__restrict__ img, int N,
                                                        int ns, int L) {
   extern __shared__ float w_s[];                 // [L][128]
@@ -644,15 +646,15 @@ __global__ void __launch_bounds__(128) k_prep_uc_tiles(const float *__restrict__
   const size_t cls = blockIdx.x;
   const int st = blockIdx.y, r = threadIdx.x, s = st * 128 + r;
   uint8_t *out = reinterpret_cast<uint8_t *>(img) + (cls * ns + st) * IMG_BYTES;
-  float acc[32];
+  float acc[LMAX];
 #pragma unroll
-  for (int l = 0; l < 32; ++l) acc[l] = 0.f;
+  for (int l = 0; l < LMAX; ++l) acc[l] = 0.f;
   if (s < N) {
     const float4 *v = reinterpret_cast<const float4 *>(vs + (cls * N + s) * DD);
     for (int d4 = 0; d4 < 32; ++d4) {
       const float4 x = v[d4];
 #pragma unroll
-      for (int l = 0; l < 32; ++l) {
+      for (int l = 0; l < LMAX; ++l) {
         if (l < L) {
           const float4 ww = *reinterpret_cast<const float4 *>(&w_s[l * 128 + d4 * 4]);
           acc[l] += x.x * ww.x + x.y * ww.y + x.z * ww.z + x.w * ww.w;
@@ -660,11 +662,11 @@ __global__ void __launch_bounds__(128) k_prep_uc_tiles(const float *__restrict__
       }
     }
   }
-  // column r of the tile for every row: rows l < 32 carry values, rows 32..127 zero
+  // column r of the tile for every row: rows l < L carry values, rows L..127 zero
   for (int l = 0; l < 128; ++l) {
     float val = 0.f;
 #pragma unroll
-    for (int m = 0; m < 32; ++m) if (m == l) val = acc[m];
+    for (int m = 0; m < LMAX; ++m) if (m == l) val = acc[m];
     *reinterpret_cast<__nv_bfloat16 *>(out + (r >> 6) * SUB_BYTES + sw128_offset(l, r & 63)) = __float2bfloat16_rn(l < L ? val : 0.f);
   }
 }
@@ -727,25 +729,28 @@ __global__ void __launch_bounds__(256) k_prep_sel_tiles(const uint32_t *__restri
   }
 }
 
-// Head table: UAB[row][p*32 + l] = sum_d Wdr[l][d] . Gv_p[row][d] (+ bdr[l] for p == 0); rows = n_win*T, pair tuples
-// Persistent over groups of four rows; Wdr is staged TRANSPOSED in shared memory once per CTA (the first version ran one CTA per row
-// with every thread walking its own weight row in global memory: 32 sectors per load, 1.9 ms for 65 536 rows -- 15 % of a T=32 score).
+// Head table: UAB[row][p*LP + l] = sum_d Wdr[l][d] . Gv_p[row][d] (+ bdr[l] for p == 0); rows = n_win*T, pair tuples, L <= LP
+// columns per frame part (LP = 32 for T <= 32, 64 for T <= 64: arx_tcn_head_cols), row stride 2*LP.
+// Persistent over groups of 256 / (2*LP) rows; Wdr is staged TRANSPOSED in shared memory once per CTA (the first version ran one CTA per
+// row with every thread walking its own weight row in global memory: 32 sectors per load, 1.9 ms for 65 536 rows -- 15 % of a T=32 score).
 // Same summation order as before (bias first, d ascending): bit-identical.
+template <int LP>
 __global__ void __launch_bounds__(256) k_head_uab(const float *__restrict__ G, int ldg, int voff, const float *__restrict__ dr_w,
                                                   const float *__restrict__ dr_b, float *__restrict__ uab, int64_t rows, int L) {
-  __shared__ float wT[DD][33];                      // wT[d][l], padded: the transposing store is conflict-free too
-  __shared__ __align__(16) float g_s[4][2 * DD];
+  constexpr int RG = 256 / (2 * LP);                // rows per group: one thread per (row, frame part, column)
+  __shared__ float wT[DD][LP + 1];                  // wT[d][l], padded: the transposing store is conflict-free too
+  __shared__ __align__(16) float g_s[RG][2 * DD];
   const int tid = threadIdx.x;
-  for (int e = tid; e < 32 * DD; e += 256) {
+  for (int e = tid; e < LP * DD; e += 256) {
     const int l = e / DD, dd = e - l * DD;
     wT[dd][l] = l < L ? dr_w[(size_t)l * DD + dd] : 0.f;
   }
-  const int slot = tid >> 6, pp = (tid >> 5) & 1, l = tid & 31;
+  const int slot = tid / (2 * LP), pp = (tid / LP) & 1, l = tid % LP;
   const float bias = (pp == 0 && l < L) ? dr_b[l] : 0.f;
-  for (int64_t r0 = (int64_t)blockIdx.x * 4; r0 < rows; r0 += (int64_t)gridDim.x * 4) {
+  for (int64_t r0 = (int64_t)blockIdx.x * RG; r0 < rows; r0 += (int64_t)gridDim.x * RG) {
     __syncthreads();                                // the previous group's rows have been consumed (first pass: wT is complete)
-    if (r0 + slot < rows)                           // 4 rows x 256 floats: one float4 per thread, coalesced
-      *reinterpret_cast<float4 *>(&g_s[slot][(tid & 63) * 4]) = *reinterpret_cast<const float4 *>(G + (r0 + slot) * ldg + voff + (tid & 63) * 4);
+    if (tid < RG * 64 && r0 + (tid >> 6) < rows)    // RG rows x 256 floats: one float4 per thread, coalesced
+      *reinterpret_cast<float4 *>(&g_s[tid >> 6][(tid & 63) * 4]) = *reinterpret_cast<const float4 *>(G + (r0 + (tid >> 6)) * ldg + voff + (tid & 63) * 4);
     __syncthreads();
     if (r0 + slot < rows) {
       float a = bias;
@@ -753,7 +758,7 @@ __global__ void __launch_bounds__(256) k_head_uab(const float *__restrict__ G, i
 #pragma unroll 8
         for (int dd = 0; dd < DD; ++dd) a = fmaf(wT[dd][l], g_s[slot][pp * DD + dd], a);
       }
-      uab[(r0 + slot) * 64 + pp * 32 + l] = a;
+      uab[(r0 + slot) * (2 * LP) + pp * LP + l] = a;
     }
   }
 }
@@ -786,6 +791,8 @@ __global__ void k_finish_n(const float *__restrict__ partial, float *__restrict_
 bool arx_tcn_supported(const arx_handle *h, const ArxTransformer &tr) {
   return h->D == DD && h->T <= 255 && tr.c >= 2 && tr.c <= 3;
 }
+bool arx_tcn_head_supported(const arx_handle *h, const ArxTransformer &tr) { return tr.c == 2 && h->T <= 64; }
+int arx_tcn_head_cols(int T) { return T <= 32 ? 32 : 64; }
 // exp2 without a shift is only safe inside the overflow bound on the LayerNorm affine (SURVEY 7.2-1); past it the ROWMAX
 // variant runs.  Only force_path = 2 gets there: by default weights past the tighter accuracy bound score on the fp32 kernels.
 bool arx_tcn_needs_rowmax(const ArxTransformer &tr) { return !(tr.softmax_bound * ARX_SOFTMAX_LOG2E < 100.0f); }
@@ -812,7 +819,8 @@ int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_h
   ARX_LAUNCH_CHECK(h);
   if (with_head) {
     if (!tr.uc_tiles) ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.uc_tiles), bytes));
-    k_prep_uc_tiles<<<dim3(way, ns), 128, h->T * 128 * sizeof(float), st>>>(tr.vs, h->dr_w, tr.uc_tiles, tr.N, ns, h->T);
+    auto kern = arx_tcn_head_cols(h->T) == 32 ? k_prep_uc_tiles<32> : k_prep_uc_tiles<64>;
+    kern<<<dim3(way, ns), 128, h->T * 128 * sizeof(float), st>>>(tr.vs, h->dr_w, tr.uc_tiles, tr.N, ns, h->T);
     ARX_LAUNCH_CHECK(h);
   }
   return ARX_OK;
@@ -887,6 +895,16 @@ static int tcn_prep_vq(arx_handle *h, const ArxTransformer &tr, const float *tab
   return ARX_OK;
 }
 
+// head table UAB of n_win windows (k_head_uab: rows = n_win*T, 2*LP columns) and selection operand A of the head from it
+static int tcn_head_table(arx_handle *h, const ArxTransformer &tr, const float *G, int ldg, int64_t n_win, float *uab, __half *vq_ws, cudaStream_t st) {
+  const int lp = arx_tcn_head_cols(h->T), rg = 256 / (2 * lp);
+  const int64_t rows = n_win * h->T;
+  auto kern = lp == 32 ? k_head_uab<32> : k_head_uab<64>;
+  kern<<<(unsigned)std::min<int64_t>((rows + rg - 1) / rg, 4 * h->sm_count), 256, 0, st>>>(G, ldg, tr.c * h->D, h->dr_w, h->dr_b, uab, rows, h->T);
+  ARX_LAUNCH_CHECK(h);
+  return tcn_prep_vq(h, tr, uab, 2 * lp, 0, lp, h->T, n_win, vq_ws, st);
+}
+
 // squared-distance partials only (the streaming tail forms logits / argmax itself).  episodes: window w attends the pool
 // classes [cls_base + w*way, cls_base + (w+1)*way) instead of classes [0, way)
 int arx_tcn_attention_partial(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
@@ -916,10 +934,8 @@ int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_
 // attention launch instead of after it; `iota` = device array 0..way-1
 int arx_tcn_head_all(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int way, const int32_t *iota,
                      float *uab, float *y_all, __half *vq_ws, cudaStream_t st) {
-  if (tr.c != 2 || h->T > 32 || !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "tcn_head: pair tuples with T <= 32 only");
-  k_head_uab<<<(unsigned)((h->T + 3) / 4), 256, 0, st>>>(G, ldg, tr.c * h->D, h->dr_w, h->dr_b, uab, h->T, h->T);
-  ARX_LAUNCH_CHECK(h);
-  int rc = tcn_prep_vq(h, tr, uab, 64, 0, 32, h->T, 1, vq_ws, st);
+  if (!arx_tcn_head_supported(h, tr) || !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "tcn_head: pair tuples with T <= 64 only");
+  int rc = tcn_head_table(h, tr, G, ldg, 1, uab, vq_ws, st);
   if (rc) return rc;
   AttnNParams p{};
   p.kq_img = kq_tiles; p.kc_img = tr.kc_tiles; p.vct_img = tr.uc_tiles; p.vq_img = vq_ws; p.sel_img = tr.sel_tiles; p.nsel = tcn_nsel(h, tr);
@@ -934,11 +950,8 @@ int arx_tcn_head_all(arx_handle *h, const ArxTransformer &tr, const __half *kq_t
 // ep_way > 0: episode mode, window w's winner chosen[w] is class cls_base + w*ep_way + chosen[w] of the pool
 int arx_tcn_head(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, const int32_t *chosen,
                  float *uab, float *y, __half *y_img, int y_nk, __half *vq_ws, int ep_way, int64_t cls_base, cudaStream_t st) {
-  if (tr.c != 2 || h->T > 32 || !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "tcn_head: pair tuples with T <= 32 only");
-  k_head_uab<<<(unsigned)std::min<int64_t>((n_win * h->T + 3) / 4, 4 * h->sm_count), 256, 0, st>>>(G, ldg, tr.c * h->D, h->dr_w, h->dr_b, uab, n_win * h->T,
-                                                                                                       h->T);
-  ARX_LAUNCH_CHECK(h);
-  int rc = tcn_prep_vq(h, tr, uab, 64, 0, 32, h->T, n_win, vq_ws, st);
+  if (!arx_tcn_head_supported(h, tr) || !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "tcn_head: pair tuples with T <= 64 only");
+  int rc = tcn_head_table(h, tr, G, ldg, n_win, uab, vq_ws, st);
   if (rc) return rc;
   AttnNParams p{};
   p.kq_img = kq_tiles; p.kc_img = tr.kc_tiles; p.vct_img = tr.uc_tiles; p.vq_img = vq_ws; p.sel_img = tr.sel_tiles; p.nsel = tcn_nsel(h, tr);
