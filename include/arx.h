@@ -128,9 +128,9 @@ ARX_API int arx_score(arx_handle *h, const float *query_dev, int64_t n_windows,
 
 /* Frame-stream form of arx_score: frames_dev (n_frames, 3J) is a sequence of camera frames and EVERY sliding window of
  * seq_len consecutive frames is scored (window w = frames w .. w+T-1, what n_frames successive ActionRecognizer.inference
- * calls see, ar.py:42-50): logits_dev (n_frames-T+1, W), is_true_dev (n_frames-T+1).  Each frame is embedded and projected
- * ONCE (the projection is position-independent; the positional table is added per window position when the windows are
- * formed on the device), and a caller uploads 3J floats per window instead of T*3J. */
+ * calls see, ar.py:42-50): logits_dev (n_frames-T+1, W), is_true_dev (n_frames-T+1).  On every route each frame is embedded
+ * and projected ONCE (the projection is position-independent; the positional table is added per window position when the
+ * windows are formed on the device), and a caller uploads 3J floats per window instead of T*3J. */
 ARX_API int arx_score_frames(arx_handle *h, const float *frames_dev, int64_t n_frames,
                      float *logits_dev, float *is_true_dev, int32_t *chosen_dev, void *stream);
 

@@ -91,7 +91,31 @@ void free_support(arx_handle *h) {
   h->way = h->way_cap = 0;
 }
 
-#define ARX_EP_UNSUPPORTED (-100)   /* internal: episode mode asked for a shape the batched kernels do not cover */
+// What a scoring pass reads: pose windows (n, T, 3J), a frame stream (n + T - 1 frames of 3J; window w = frames w .. w+T-1)
+// or feature windows (n, T, F).  Pose rows may be fp16 (arx_score_host*_f16); only routes with tc_front_end take them.
+struct Query {
+  enum Kind { WINDOWS, FRAMES, FEATURES };
+  const void *rows;
+  Kind kind;
+  bool f16;
+  bool poses() const { return kind != FEATURES; }
+  // input rows that n windows read
+  int64_t n_rows(const arx_handle *h, int64_t n) const { return kind == FRAMES ? n + h->T - 1 : n * h->T; }
+  // the rows of the chunk that starts at window b0
+  const void *at(const arx_handle *h, int64_t b0) const {
+    const int64_t off = (kind == FRAMES ? b0 : b0 * h->T) * (poses() ? h->J3 : h->F);
+    return static_cast<const char *>(rows) + off * (f16 ? sizeof(__half) : sizeof(float));
+  }
+  const float *f32(const arx_handle *h, int64_t b0) const { return static_cast<const float *>(at(h, b0)); }
+};
+
+// Where a pass writes: logits (n, way), is_true (n; null: no open-set head), chosen (n; null: argmax scratch in the
+// workspace) and the debug outputs only the fp32 kernels write (probs (n, way, N, N), protos (n, way, N, D); null: none)
+struct Outputs {
+  float *logits, *is_true;
+  int32_t *chosen;
+  float *probs = nullptr, *protos = nullptr;
+};
 
 // per-window workspace of the T=16 pair pipeline
 struct PairWs {
@@ -99,35 +123,38 @@ struct PairWs {
   float *uab, *G, *partial, *P, *U;     // P, U: frame-stream form: per-frame position-independent projections / head columns
   size_t bytes;
 };
-PairWs carve_pair(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, bool frames_stream, void *base) {
+PairWs carve_pair(arx_handle *h, const ArxTransformer &tr, const Query &q, int64_t n, int way, bool disc, void *base) {
   Carver c(base);
   PairWs w{};
+  const bool frames = q.kind == Query::FRAMES;
   const int64_t rows_pad = (n * h->T + 127) / 128 * 128, n_pad = (n + 127) / 128 * 128;
   w.kq_img = c.take<__half>(n * 128 * 128);
-  w.x_img = from_frames ? c.take<__half>(rows_pad * 128) : nullptr;
-  w.h_img = from_frames ? c.take<__half>(rows_pad * 192) : nullptr;
+  w.x_img = q.poses() ? c.take<__half>(rows_pad * 128) : nullptr;
+  w.h_img = q.poses() ? c.take<__half>(rows_pad * 192) : nullptr;
   w.f_img = c.take<__half>(rows_pad * 320);      // 4 feature sub-tiles + the one-hot sub-tile
   w.y_img = disc ? c.take<__half>(n_pad * (int64_t)h->tl_d1.nk * 64) : nullptr;
   w.h1_img = disc ? c.take<__half>(n_pad * 256) : nullptr;
   w.uab = disc ? c.take<float>(rows_pad * 32) : nullptr;
   w.G = c.take<float>(rows_pad * 2 * tr.c * h->D);     // chunked layout holds whole 128-row tiles
   w.partial = c.take<float>(n * way * 4);
-  w.P = frames_stream ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
-  w.U = frames_stream ? c.take<float>((n + h->T) * 32) : nullptr;
+  w.P = frames ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
+  w.U = frames ? c.take<float>((n + h->T) * 32) : nullptr;
   w.bytes = c.off + 256;
   return w;
 }
 
 // per-window workspace of the fp32 CUDA-core kernels
 struct Fp32Ws {
-  float *H1, *FE, *G, *Kq, *Vq, *Z, *partial, *y, *h1, *h2;
+  float *H1, *FE, *P, *G, *Kq, *Vq, *Z, *partial, *y, *h1, *h2;
   size_t bytes;
 };
-Fp32Ws carve_generic(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, void *base) {
+Fp32Ws carve_generic(arx_handle *h, const ArxTransformer &tr, const Query &q, int64_t n, int way, bool disc, void *base) {
   Carver c(base);
   Fp32Ws w{};
-  w.H1 = from_frames ? c.take<float>(n * h->T * h->H) : nullptr;
-  w.FE = from_frames ? c.take<float>(n * h->T * h->F) : nullptr;
+  const int64_t rows_in = q.n_rows(h, n);
+  w.H1 = q.poses() ? c.take<float>(rows_in * h->H) : nullptr;
+  w.FE = q.poses() ? c.take<float>(rows_in * h->F) : nullptr;
+  w.P = q.kind == Query::FRAMES ? c.take<float>(rows_in * 2 * tr.c * h->D) : nullptr;
   w.G = c.take<float>(n * h->T * 2 * tr.c * h->D);
   w.Kq = c.take<float>(n * tr.N * h->D);
   w.Vq = c.take<float>(n * tr.N * h->D);
@@ -140,21 +167,20 @@ Fp32Ws carve_generic(arx_handle *h, const ArxTransformer &tr, int64_t n, int way
   return w;
 }
 
-// Windows per pass (at most max_chunk, default 4096, and 3 GB of the layout carve(n, base)), the workspace for them and,
-// without the caller's chosen buffer, the argmax scratch after it.  one_pass (episode mode of the T=16 pair pipeline, whose
-// kernels take no pool class offset): more passes are unsupported.
-template <class Ws, class Carve>
-int plan_chunks(arx_handle *h, int64_t n_windows, bool one_pass, const int32_t *chosen_dev, Carve &&carve, int64_t *chunk, Ws *w,
-                int32_t **chosen_ws) {
+// Windows per pass: at most max_chunk (default 4096), and at most 3 GB of the layout carve(n, base)
+template <class Carve> int64_t pass_windows(const arx_handle *h, int64_t n_windows, Carve &&carve) {
   const size_t per = carve(128, nullptr).bytes / 128 + 1;
   const int64_t cap = h->cfg.max_chunk > 0 ? h->cfg.max_chunk : 4096;
   const int64_t fit = (int64_t)(((size_t)3 << 30) / per);
-  *chunk = std::max<int64_t>(1, std::min(std::min(cap, fit), n_windows));
-  if (one_pass && *chunk < n_windows) return ARX_EP_UNSUPPORTED;
-  const size_t bytes = carve(*chunk, nullptr).bytes;
-  const int rc = arx_ws_reserve(h, bytes + (chosen_dev ? 0 : (size_t)*chunk * sizeof(int32_t) + 256));
+  return std::max<int64_t>(1, std::min(std::min(cap, fit), n_windows));
+}
+
+// The workspace for passes of `chunk` windows and, without the caller's chosen buffer, the argmax scratch after it
+template <class Ws, class Carve> int pass_reserve(arx_handle *h, int64_t chunk, const int32_t *chosen_dev, Carve &&carve, Ws *w, int32_t **chosen_ws) {
+  const size_t bytes = carve(chunk, nullptr).bytes;
+  const int rc = arx_ws_reserve(h, bytes + (chosen_dev ? 0 : (size_t)chunk * sizeof(int32_t) + 256));
   if (rc) return rc;
-  *w = carve(*chunk, h->ws);
+  *w = carve(chunk, h->ws);
   *chosen_ws = chosen_dev ? nullptr : reinterpret_cast<int32_t *>(static_cast<char *>(h->ws) + bytes);
   return ARX_OK;
 }
@@ -166,12 +192,12 @@ int embed_frames(arx_handle *h, const float *X, int64_t rows, float *H1, float *
   return arx_fp32_linear(h, H1, h->H, h->fc2_w, h->H, h->fc2_b, FE, h->F, rows, h->F, h->H, ARX_ACT_RELU, nullptr, 1, st);
 }
 
-// the same on tensor cores, three launches: frames -> fp16 image x_img -> fc1 -> h_img -> fc2 -> feature image f_img
-// (f_nk sub-tiles; f_onehot: the one-hot sub-tile of the positional table, or -1)
-int embed_frames_tc(arx_handle *h, const float *X, int64_t rows, __half *x_img, __half *h_img, __half *f_img, int f_nk, int f_onehot,
+// the same on tensor cores, three launches: frames (fp32, or fp16 when `f16`) -> fp16 image x_img -> fc1 -> h_img -> fc2 ->
+// feature image f_img (f_nk sub-tiles; f_onehot: the one-hot sub-tile of the positional table, or -1)
+int embed_frames_tc(arx_handle *h, const void *X, bool f16, int64_t rows, __half *x_img, __half *h_img, __half *f_img, int f_nk, int f_onehot,
                     cudaStream_t st) {
   int rc;
-  if ((rc = arx_tc_rows_to_img(h, X, h->J3, h->J3, rows, x_img, h->tl_fc1.nk, -1, st))) return rc;
+  if ((rc = arx_tc_rows_to_img(h, X, f16, h->J3, h->J3, rows, x_img, h->tl_fc1.nk, -1, st))) return rc;
   if ((rc = arx_tc_linear_img(h, h->tl_fc1, x_img, rows, ARX_ACT_RELU, h_img, h->tl_fc2.nk, -1, st))) return rc;
   return arx_tc_linear_img(h, h->tl_fc2, h_img, rows, ARX_ACT_RELU, f_img, f_nk, f_onehot, st);
 }
@@ -641,7 +667,7 @@ static int set_support_features(arx_handle *h, const float *feats_dev, int32_t w
   cudaStream_t ss;
   if ((rc = support_fork(h, st, &ss))) return rc;                  // the caller's buffer is not touched past this point
   if (h->tc_linears) {
-    if ((rc = arx_tc_rows_to_img(h, h->ss_feat, h->F, h->F, (int64_t)way * h->T, sc.f_img, h->tr[0].tl_proj.nk,
+    if ((rc = arx_tc_rows_to_img(h, h->ss_feat, false, h->F, h->F, (int64_t)way * h->T, sc.f_img, h->tr[0].tl_proj.nk,
                                  h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
       return rc;
     rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
@@ -672,7 +698,7 @@ static int set_support_poses(arx_handle *h, const float *poses_dev, int32_t way,
   if (h->tc_linears) {
     // same tensor-core pipeline as the query frames; the fp32 'support_features' are derived lazily on request
     h->ss_feat_valid = false;
-    if ((rc = embed_frames_tc(h, h->ss_poses, rows, sc.x_img, sc.h_img, sc.f_img, h->tr[0].tl_proj.nk,
+    if ((rc = embed_frames_tc(h, h->ss_poses, false, rows, sc.x_img, sc.h_img, sc.f_img, h->tr[0].tl_proj.nk,
                               h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
       return rc;
     rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
@@ -787,14 +813,24 @@ static int prof_mark(arx_handle *h, int idx, cudaStream_t st) {
   return ARX_OK;
 }
 
-// front end on the CUDA cores, windows from b0: frames (query_dev, embedded here) or features (qfeats_dev) -> per-frame
-// projections G
-static int front_end_fp32(arx_handle *h, const ArxTransformer &tr, const float *query_dev, const float *qfeats_dev, int64_t b0, int64_t rows,
-                          float *H1, float *FE, float *G, cudaStream_t st) {
+// front end on the CUDA cores, the n windows from b0 -> row-major per-frame projections G.  Poses are embedded here (H1, FE).
+// A frame stream embeds and projects every frame once without the positional table (P), and the windows are formed from
+// that: k_linear adds the table after the accumulation, so either way G holds the same bits.
+static int front_end_fp32(arx_handle *h, const ArxTransformer &tr, const Query &q, int64_t b0, int64_t n, float *H1, float *FE, float *P,
+                          float *G, cudaStream_t st) {
+  const int64_t rows = q.n_rows(h, n);
+  const int ldg = 2 * tr.c * h->D;
   int rc;
-  if (query_dev && (rc = embed_frames(h, query_dev + b0 * h->T * h->J3, rows, H1, FE, st))) return rc;
+  if (q.poses() && (rc = embed_frames(h, q.f32(h, b0), rows, H1, FE, st))) return rc;
   if ((rc = prof_mark(h, 1, st))) return rc;
-  return project_frames(h, tr, query_dev ? FE : qfeats_dev + b0 * h->T * h->F, rows, G, st);
+  if (q.kind != Query::FRAMES) return project_frames(h, tr, q.poses() ? FE : q.f32(h, b0), rows, G, st);
+  if ((rc = arx_fp32_linear(h, FE, h->F, tr.wp, h->F, nullptr, P, ldg, rows, ldg, h->F, ARX_ACT_NONE, nullptr, 1, st))) return rc;
+  return arx_form_windows_launch(h, tr, P, nullptr, G, nullptr, n, false, st);
+}
+
+// The route runs its front end on the tensor-core linear layers: the one front end that reads fp16 pose rows
+static bool tc_front_end(const arx_handle *h, ArxRoute route) {
+  return (route == ARX_ROUTE_PAIR || route == ARX_ROUTE_TILED) && h->tc_linears && (h->tc_variant & 4) == 0;
 }
 
 extern "C++" {
@@ -860,17 +896,16 @@ struct TcnWs {
   float *H1, *FE, *G, *partial, *uab, *y, *h1, *h2, *P;
   size_t bytes;
 };
-static TcnWs carve_tcn(arx_handle *h, const ArxTransformer &tr, int64_t n, int way, bool from_frames, bool disc, bool tcl, void *base,
-                       bool stream = false) {
+static TcnWs carve_tcn(arx_handle *h, const ArxTransformer &tr, const Query &q, int64_t n, int way, bool disc, bool tcl, void *base) {
   Carver c(base);
   TcnWs w{};
   const int64_t rows = n * h->T, rows_pad = (rows + 127) / 128 * 128, n_pad = (n + 127) / 128 * 128;
   const int nq = tr.Npad / 128;
-  w.x_img = (tcl && from_frames) ? c.take<__half>(rows_pad * 128) : nullptr;
-  w.h_img = (tcl && from_frames) ? c.take<__half>(rows_pad * 192) : nullptr;
+  w.x_img = (tcl && q.poses()) ? c.take<__half>(rows_pad * 128) : nullptr;
+  w.h_img = (tcl && q.poses()) ? c.take<__half>(rows_pad * 192) : nullptr;
   w.f_img = tcl ? c.take<__half>(rows_pad * 320) : nullptr;
-  w.H1 = (!tcl && from_frames) ? c.take<float>(rows * h->H) : nullptr;
-  w.FE = (!tcl && from_frames) ? c.take<float>(rows * h->F) : nullptr;
+  w.H1 = (!tcl && q.poses()) ? c.take<float>(rows * h->H) : nullptr;
+  w.FE = (!tcl && q.poses()) ? c.take<float>(rows * h->F) : nullptr;
   w.G = c.take<float>(rows_pad * 2 * tr.c * h->D);
   w.kq = c.take<__half>((size_t)n * nq * 128 * 128);
   w.partial = c.take<float>(n * way * 4);
@@ -889,7 +924,7 @@ static TcnWs carve_tcn(arx_handle *h, const ArxTransformer &tr, int64_t n, int w
       w.h2 = c.take<float>(n * 64);
     }
   }
-  w.P = stream ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
+  w.P = q.kind == Query::FRAMES ? c.take<float>((n + h->T) * 2 * tr.c * h->D) : nullptr;
   w.bytes = c.off + 256;
   return w;
 }
@@ -914,50 +949,43 @@ static int tcn_backend(arx_handle *h, const ArxTransformer &tr, const TcnWs &w, 
 
 // ep_way > 0: episode mode -- window b attends classes [b*ep_way, (b+1)*ep_way) of the support pool; the windows may
 // still be split into several passes (the kernels take the pass's first pool class)
-static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
-                     float *is_true_dev, int32_t *chosen_dev, cudaStream_t st, int ep_way, bool frames_stream = false) {
+static int score_tcn(arx_handle *h, int ti, const Query &q, int64_t n_windows, const Outputs &out, cudaStream_t st, int ep_way) {
   const ArxTransformer &tr = h->tr[ti];
-  const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr, tcl = h->tc_linears && (h->tc_variant & 4) == 0;
+  const bool disc = out.is_true != nullptr, tcl = tc_front_end(h, ARX_ROUTE_TILED);
   const int way = ep_way > 0 ? ep_way : h->way;
   if (!tr.kc_tiles) return arx_fail(h, ARX_ERR_STATE, "score: support operands of the tiled kernels are missing (set the support set again)");
   if (disc && !tr.uc_tiles) return arx_fail(h, ARX_ERR_INVALID, "score: the open-set head of the tiled kernels needs pair tuples and T <= 64");
-  int64_t chunk;
+  auto carve = [&](int64_t n, void *base) { return carve_tcn(h, tr, q, n, way, disc, tcl, base); };
+  const int64_t chunk = pass_windows(h, n_windows, carve);
   TcnWs w;
   int32_t *chosen_ws;
-  int rc = plan_chunks(h, n_windows, false, chosen_dev, [&](int64_t n, void *base) {
-    return carve_tcn(h, tr, n, way, from_frames, disc, tcl, base, frames_stream);
-  }, &chunk, &w, &chosen_ws);
+  int rc = pass_reserve(h, chunk, out.chosen, carve, &w, &chosen_ws);
   if (rc) return rc;
   const int ldg = 2 * tr.c * h->D;
   const int f_nk = tr.tl_proj.nk, f_onehot = tr.table_in_gemm ? f_nk - 1 : -1;     // feature image: + one-hot sub-tile
   h->last_path = ARX_ROUTE_TILED;
   for (int64_t b0 = 0; b0 < n_windows; b0 += chunk) {
-    const int64_t n = std::min(chunk, n_windows - b0), rows = n * h->T;
+    const int64_t n = std::min(chunk, n_windows - b0), rows = q.n_rows(h, n);
     if ((rc = prof_mark(h, 0, st))) return rc;
-    if (frames_stream) {
+    if (!tcl) {
+      if ((rc = front_end_fp32(h, tr, q, b0, n, w.H1, w.FE, w.P, w.G, st))) return rc;
+    } else if (q.kind == Query::FRAMES) {
       // frame stream: embed and project every frame once (position-independent), then form the windows' projections
-      const int64_t rows_f = n + h->T - 1;
-      if (tcl) {
-        const ArxTcLinear &L = tr.table_in_gemm ? tr.tl_proj_nt : tr.tl_proj;
-        if ((rc = embed_frames_tc(h, query_dev + b0 * h->J3, rows_f, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
-        if ((rc = prof_mark(h, 1, st))) return rc;
-        if ((rc = arx_tc_linear_f32(h, L, w.f_img, f_nk, rows_f, w.P, ldg, nullptr, 1, st))) return rc;
-      } else {
-        if ((rc = embed_frames(h, query_dev + b0 * h->J3, rows_f, w.H1, w.FE, st))) return rc;
-        if ((rc = prof_mark(h, 1, st))) return rc;
-        if ((rc = arx_fp32_linear(h, w.FE, h->F, tr.wp, h->F, nullptr, w.P, ldg, rows_f, ldg, h->F, ARX_ACT_NONE, nullptr, 1, st))) return rc;
-      }
+      const ArxTcLinear &L = tr.table_in_gemm ? tr.tl_proj_nt : tr.tl_proj;
+      if ((rc = embed_frames_tc(h, q.at(h, b0), q.f16, rows, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
+      if ((rc = prof_mark(h, 1, st))) return rc;
+      if ((rc = arx_tc_linear_f32(h, L, w.f_img, f_nk, rows, w.P, ldg, nullptr, 1, st))) return rc;
       if ((rc = arx_form_windows_launch(h, tr, w.P, nullptr, w.G, nullptr, n, false, st))) return rc;
-    } else if (tcl) {
-      if (from_frames) {
-        if ((rc = embed_frames_tc(h, query_dev + b0 * h->T * h->J3, rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
-      } else if ((rc = arx_tc_rows_to_img(h, qfeats_dev + b0 * h->T * h->F, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
+    } else {
+      if (q.poses()) {
+        if ((rc = embed_frames_tc(h, q.at(h, b0), q.f16, rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
+      } else if ((rc = arx_tc_rows_to_img(h, q.at(h, b0), false, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
       if ((rc = prof_mark(h, 1, st))) return rc;
       if ((rc = arx_tc_linear_f32(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, ldg, tr.table_in_gemm ? nullptr : tr.bp, h->T, st))) return rc;
-    } else if ((rc = front_end_fp32(h, tr, query_dev, qfeats_dev, b0, rows, w.H1, w.FE, w.G, st))) return rc;
+    }
     if ((rc = prof_mark(h, 2, st))) return rc;
-    int32_t *ch = chosen_dev ? chosen_dev + b0 : chosen_ws;
-    if ((rc = tcn_backend(h, tr, w, n, way, tcl, logits_dev + b0 * way, is_true_dev ? is_true_dev + b0 : nullptr, ch, ep_way, b0 * way, st)))
+    int32_t *ch = out.chosen ? out.chosen + b0 : chosen_ws;
+    if ((rc = tcn_backend(h, tr, w, n, way, tcl, out.logits + b0 * way, disc ? out.is_true + b0 : nullptr, ch, ep_way, b0 * way, st)))
       return rc;
     if ((rc = prof_mark(h, 5, st))) return rc;
   }
@@ -969,75 +997,71 @@ static int score_tcn(arx_handle *h, int ti, const float *query_dev, const float 
 // tuple images (gather + LayerNorm + exp2 pre-scale) -> [join the support chain] -> cross-attention + distances ->
 // logits / argmax -> open-set head by linearity -> fc1 -> fc2 + fc3 + sigmoid.  Replayed as two CUDA graphs (before /
 // after the join) when the arguments recur.
-// frames_stream: query_dev is a FRAME stream (n_windows + T - 1 rows of 3J); window w = frames w .. w+T-1 (arx_score_frames)
-static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
-                      float *is_true_dev, int32_t *chosen_dev, cudaStream_t st, int ep_way, bool frames_stream = false) {
+static int score_gen3(arx_handle *h, int ti, const Query &q, int64_t n_windows, const Outputs &out, cudaStream_t st, int ep_way) {
   const ArxTransformer &tr = h->tr[ti];
-  const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr;
+  const bool disc = out.is_true != nullptr;
   const int way = ep_way > 0 ? ep_way : h->way;
   if (disc && (ti != 0 || !tr.uc_img)) return arx_fail(h, ARX_ERR_STATE, "score: open-set head operands missing (set the support set again)");
   const bool big_batch = n_windows * h->T >= 128ll * 2 * h->sm_count;             // persistent GEMMs pay off from ~2 tiles per SM
   const bool p_embed = big_batch && (h->tc_variant & 1024) == 0 && arx_tcp_supported(h->tl_fc1) && arx_tcp_supported(h->tl_fc2);
-  int64_t chunk;
+  auto carve = [&](int64_t n, void *base) { return carve_pair(h, tr, q, n, way, disc, base); };
+  const int64_t chunk = pass_windows(h, n_windows, carve);
+  // the episode-mode kernels take no pool class offset: arx_score_episodes sizes its passes to one chunk
+  if (ep_way > 0 && chunk < n_windows) return arx_fail(h, ARX_ERR_INVALID, "score: an episode pass of the pair pipeline exceeds one chunk");
   PairWs w;
   int32_t *chosen_ws;
-  int rc = plan_chunks(h, n_windows, ep_way > 0, chosen_dev, [&](int64_t n, void *base) {
-    return carve_pair(h, tr, n, way, from_frames, disc, frames_stream, base);
-  }, &chunk, &w, &chosen_ws);
+  int rc = pass_reserve(h, chunk, out.chosen, carve, &w, &chosen_ws);
   if (rc) return rc;
   h->last_path = ARX_ROUTE_PAIR;
   bool aux_pending = false;
+  // A support chain still running on the side stream (set_support right before this pass) is six small dependent kernels;
+  // the persistent front-end kernels own every SM with their shared memory, so the chain only advanced in the gaps between
+  // them and the join below waited ~25 us for it.  The front end leaves it a few SMs of its own.
   const int reserve = (h->support_inflight && big_batch && (h->tc_variant & 32768) == 0) ? h->sm_reserve_n : 0;      // debug bit 32768: no reserved SMs
+  const int sms = h->sm_count - reserve;
   ArxScoreGraph *sg = nullptr;
   bool capturable = st != nullptr && st != cudaStreamLegacy && st != cudaStreamPerThread && graphs_enabled(h);     // the default streams cannot be captured
   if (capturable && capture_id(st) != 0) capturable = false;      // a caller that is capturing this stream itself gets plain launches
-  if (capturable && disc && from_frames && !frames_stream && chunk >= n_windows && !h->prof_on && !h->trace_buf) {
+  if (capturable && disc && q.kind == Query::WINDOWS && chunk >= n_windows && !h->prof_on && !h->trace_buf) {
     ArxScoreGraphKey key;
-    key.q = query_dev; key.lo = logits_dev; key.it = is_true_dev; key.ch = chosen_dev; key.ws = h->ws; key.n = n_windows; key.way = way;
-    key.variant = h->tc_variant | (h->pdl ? (1 << 20) : 0) | (ep_way > 0 ? (1 << 21) : 0) | (h->query_f16 ? (1 << 22) : 0) | (reserve ? (1 << 23) : 0);
+    key.q = q.rows; key.lo = out.logits; key.it = out.is_true; key.ch = out.chosen; key.ws = h->ws; key.n = n_windows; key.way = way;
+    key.variant = h->tc_variant | (h->pdl ? (1 << 20) : 0) | (ep_way > 0 ? (1 << 21) : 0) | (q.f16 ? (1 << 22) : 0) | (reserve ? (1 << 23) : 0);
     key.poly = h->attn_poly; key.stagger = h->attn_stagger; key.sgen = h->support_gen; key.wgen = h->weights_gen;
     sg = score_graph_lookup(h, key);
   }
   const int f_nk = tr.tl_proj.nk, f_onehot = tr.table_in_gemm ? f_nk - 1 : -1;     // feature image: + one-hot sub-tile
   const int g_ld = 2 * tr.c * h->D, g_voff = tr.c * h->D;
   for (int64_t b0 = 0; b0 < n_windows; b0 += chunk) {
-    const int64_t n = std::min(chunk, n_windows - b0), rows = n * h->T;
+    const int64_t n = std::min(chunk, n_windows - b0), rows = q.n_rows(h, n);
     if ((rc = prof_mark(h, 0, st))) return rc;
-    // A support chain still running on the side stream (set_support right before this pass) is six small dependent kernels;
-    // the persistent front-end kernels own every SM with their shared memory, so the chain only advanced in the gaps between
-    // them and the join below waited ~25 us for it.  Leave it a few SMs of its own for the length of the front end.
-    h->sm_reserve = reserve;
     rc = score_segment(h, sg, 0, st, [&]() -> int {
       int rc = ARX_OK;
       const float alpha = ARX_SOFTMAX_LOG2E / sqrtf((float)h->D);
-      if (frames_stream) {
+      const void *xq = q.at(h, b0);
+      if (q.kind == Query::FRAMES) {
         // every frame is embedded and projected ONCE (position-independent); the windows are formed on the device
-        const int64_t rows_f = n + h->T - 1;
-        if ((rc = embed_frames_tc(h, query_dev + b0 * h->J3, rows_f, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
+        if ((rc = embed_frames_tc(h, xq, q.f16, rows, w.x_img, w.h_img, w.f_img, f_nk, -1, st))) return rc;
         if ((rc = prof_mark(h, 1, st))) return rc;
-        if ((rc = arx_tc_linear_f32(h, tr.tl_proj_nt, w.f_img, f_nk, rows_f, w.P, g_ld, nullptr, 1, st))) return rc;
-        if (disc && (rc = arx_tc_linear_f32_small(h, tr.tl_uab, w.f_img, f_nk, rows_f, w.U, 32, nullptr, h->T, st))) return rc;
+        if ((rc = arx_tc_linear_f32(h, tr.tl_proj_nt, w.f_img, f_nk, rows, w.P, g_ld, nullptr, 1, st))) return rc;
+        if (disc && (rc = arx_tc_linear_f32_small(h, tr.tl_uab, w.f_img, f_nk, rows, w.U, 32, nullptr, h->T, st))) return rc;
         if ((rc = arx_form_windows_launch(h, tr, w.P, disc ? w.U : nullptr, w.G, w.uab, n, true, st))) return rc;
         if ((rc = prof_mark(h, 2, st))) return rc;
-        if ((rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, st))) return rc;
+        if ((rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, sms, st))) return rc;
         return ARX_OK;
       }
-      if (from_frames) {
-        // (an fp16 pass -- arx_score_host*_f16 -- carries its rows at half the stride)
-        const void *xq = h->query_f16 ? static_cast<const void *>(reinterpret_cast<const __half *>(query_dev) + b0 * h->T * h->J3)
-                                      : static_cast<const void *>(query_dev + b0 * h->T * h->J3);
-        if (p_embed && (h->tc_variant & 8192) == 0 && arx_mlp_fused_supported(h, xq)) {
-          if ((rc = arx_mlp_fused(h, xq, h->query_f16, rows, w.f_img, f_nk, f_onehot, st))) return rc;      // one launch: poses -> feature image
-        } else if (p_embed) {
-          if ((rc = arx_tc_rows_to_img(h, static_cast<const float *>(xq), h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-          if ((rc = arx_tcp_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, st))) return rc;
-          if ((rc = arx_tcp_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, st))) return rc;
-        } else if ((rc = embed_frames_tc(h, static_cast<const float *>(xq), rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
-      } else if ((rc = arx_tc_rows_to_img(h, qfeats_dev + b0 * h->T * h->F, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
+      if (!q.poses()) {
+        if ((rc = arx_tc_rows_to_img(h, xq, q.f16, h->F, h->F, rows, w.f_img, f_nk, f_onehot, st))) return rc;
+      } else if (p_embed && (h->tc_variant & 8192) == 0 && arx_mlp_fused_supported(h, xq)) {
+        if ((rc = arx_mlp_fused(h, xq, q.f16, rows, w.f_img, f_nk, f_onehot, sms, st))) return rc;      // one launch: poses -> feature image
+      } else if (p_embed) {
+        if ((rc = arx_tc_rows_to_img(h, xq, q.f16, h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
+        if ((rc = arx_tcp_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, sms, st))) return rc;
+        if ((rc = arx_tcp_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, sms, st))) return rc;
+      } else if ((rc = embed_frames_tc(h, xq, q.f16, rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
       if ((rc = prof_mark(h, 1, st))) return rc;
-      if ((rc = arx_tcp_linear_chunked(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, st))) return rc;
+      if ((rc = arx_tcp_linear_chunked(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, sms, st))) return rc;
       if ((rc = prof_mark(h, 2, st))) return rc;
-      if ((h->tc_variant & 64) == 0 && (rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, st))) return rc;   // bit 6: timing only
+      if ((h->tc_variant & 64) == 0 && (rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, sms, st))) return rc;   // bit 6: timing only
       if (disc) {
         // only the head pass reads these 32 columns: run them on a second stream, beside the tuple build + attention
         const bool aux = (h->tc_variant & 2048) == 0 && !h->prof_on && !sg;      // (a graph segment must end joined)
@@ -1057,19 +1081,18 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
       }
       return ARX_OK;
     });
-    h->sm_reserve = 0;
     if (rc) return rc;
     if ((rc = support_wait(h, st))) return rc;                   // join the support chain (side stream) before its operands are read
     if ((rc = prof_mark(h, 3, st))) return rc;
-    int32_t *ch = chosen_dev ? chosen_dev + b0 : chosen_ws;
+    int32_t *ch = out.chosen ? out.chosen + b0 : chosen_ws;
     rc = score_segment(h, sg, 1, st, [&]() -> int {
       int rc = ARX_OK;
-      if ((rc = arx_tc_attention(h, tr, w.kq_img, w.G, n, way, w.partial, logits_dev + b0 * way, ch, g_ld, g_voff, true, ep_way > 0, st))) return rc;
+      if ((rc = arx_tc_attention(h, tr, w.kq_img, w.G, n, way, w.partial, out.logits + b0 * way, ch, g_ld, g_voff, true, ep_way > 0, st))) return rc;
       if ((rc = prof_mark(h, 4, st))) return rc;
       if (disc) {
         if (aux_pending) { ARX_CUDA(h, cudaStreamWaitEvent(st, h->ev_aux_done, 0)); aux_pending = false; }
         if ((rc = arx_tc2_head_launch(h, tr, w.kq_img, w.uab, n, ch, w.y_img, h->tl_d1.nk, ep_way, st))) return rc;
-        if ((rc = disc_tail_tc(h, w.y_img, w.h1_img, n, is_true_dev + b0, st))) return rc;
+        if ((rc = disc_tail_tc(h, w.y_img, w.h1_img, n, out.is_true + b0, st))) return rc;
       }
       return ARX_OK;
     });
@@ -1081,70 +1104,62 @@ static int score_gen3(arx_handle *h, int ti, const float *query_dev, const float
 }
 
 // ---- fp32 CUDA-core kernels: any shape, debug outputs (softmax scores, prototypes), forced path ---------------------
-static int score_fp32(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
-                      float *is_true_dev, int32_t *chosen_dev, float *probs, float *protos, cudaStream_t st) {
+static int score_fp32(arx_handle *h, int ti, const Query &q, int64_t n_windows, const Outputs &out, cudaStream_t st) {
   const ArxTransformer &tr = h->tr[ti];
-  const bool from_frames = query_dev != nullptr, disc = is_true_dev != nullptr;
+  const bool disc = out.is_true != nullptr;
   const int way = h->way;
-  int64_t chunk;
+  auto carve = [&](int64_t n, void *base) { return carve_generic(h, tr, q, n, way, disc, base); };
+  const int64_t chunk = pass_windows(h, n_windows, carve);
   Fp32Ws w;
   int32_t *chosen_ws;
-  int rc = plan_chunks(h, n_windows, false, chosen_dev, [&](int64_t n, void *base) {
-    return carve_generic(h, tr, n, way, from_frames, disc, base);
-  }, &chunk, &w, &chosen_ws);
+  int rc = pass_reserve(h, chunk, out.chosen, carve, &w, &chosen_ws);
   if (rc) return rc;
   h->last_path = ARX_ROUTE_FP32;
   const int64_t NN = (int64_t)tr.N * tr.N, ND = (int64_t)tr.N * h->D;
   for (int64_t b0 = 0; b0 < n_windows; b0 += chunk) {
-    const int64_t n = std::min(chunk, n_windows - b0), rows = n * h->T;
+    const int64_t n = std::min(chunk, n_windows - b0);
     if ((rc = prof_mark(h, 0, st))) return rc;
-    if ((rc = front_end_fp32(h, tr, query_dev, qfeats_dev, b0, rows, w.H1, w.FE, w.G, st))) return rc;
+    if ((rc = front_end_fp32(h, tr, q, b0, n, w.H1, w.FE, w.P, w.G, st))) return rc;
     if ((rc = prof_mark(h, 2, st))) return rc;
     if ((rc = arx_fp32_build_tuples(h, tr, w.G, n, w.Kq, w.Vq, st))) return rc;
     if ((rc = support_wait(h, st))) return rc;
     if ((rc = prof_mark(h, 3, st))) return rc;
-    int32_t *ch = chosen_dev ? chosen_dev + b0 : chosen_ws;
-    if ((rc = arx_fp32_attention(h, tr, w.Kq, w.Vq, n, way, w.Z, w.partial, logits_dev + b0 * way, ch, disc ? w.y : nullptr,
-                                 probs ? probs + b0 * way * NN : nullptr, protos ? protos + b0 * way * ND : nullptr, st)))
+    int32_t *ch = out.chosen ? out.chosen + b0 : chosen_ws;
+    if ((rc = arx_fp32_attention(h, tr, w.Kq, w.Vq, n, way, w.Z, w.partial, out.logits + b0 * way, ch, disc ? w.y : nullptr,
+                                 out.probs ? out.probs + b0 * way * NN : nullptr, out.protos ? out.protos + b0 * way * ND : nullptr, st)))
       return rc;
     if ((rc = prof_mark(h, 4, st))) return rc;
-    if (disc && (rc = disc_tail_fp32(h, tr, w.y, w.h1, w.h2, n, is_true_dev + b0, st))) return rc;
+    if (disc && (rc = disc_tail_fp32(h, tr, w.y, w.h1, w.h2, n, out.is_true + b0, st))) return rc;
     if ((rc = prof_mark(h, 5, st))) return rc;
   }
   return ARX_OK;
 }
 
 // ep_way > 0: episode mode -- window b is scored against classes [b*ep_way, (b+1)*ep_way) of the support pool
-static int score_impl(arx_handle *h, int ti, const float *query_dev, const float *qfeats_dev, int64_t n_windows, float *logits_dev,
-                      float *is_true_dev, int32_t *chosen_dev, float *probs, float *protos, cudaStream_t st, int ep_way = 0,
-                      bool frames_stream = false) {
+static int score_impl(arx_handle *h, int ti, const Query &q, int64_t n_windows, const Outputs &out, cudaStream_t st, int ep_way = 0) {
   if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "score: weights not loaded");
   if (h->way < 1) return arx_fail(h, ARX_ERR_STATE, "score: support set not set");
   if (n_windows == 0) return ARX_OK;
   const ArxTransformer &tr = h->tr[ti];
-  const bool disc = is_true_dev != nullptr;
-  if (disc && (!h->cfg.has_discriminator || ti != 0 || tr.c != 2))
+  if (out.is_true && (!h->cfg.has_discriminator || ti != 0 || tr.c != 2))
     return arx_fail(h, ARX_ERR_INVALID, "score: the discriminator is sized for pair tuples of transformers[0] (model.py:283-285)");
   if (ep_way > 0 && (int64_t)ep_way * n_windows != h->way) return arx_fail(h, ARX_ERR_STATE, "score: episode pool does not match the batch");
   if (tr.route == ARX_ROUTE_NONE)
     return arx_fail(h, ARX_ERR_STATE, "score: transformers[%d] has no support operands (arx_score_episodes keeps those of transformers[0] "
                                       "only): set the support set again", ti);
-  const bool debug_out = probs || protos;
+  const bool debug_out = out.probs || out.protos;
   const ArxRoute route = debug_out ? ARX_ROUTE_FP32 : tr.route;      // only the fp32 kernels write the debug outputs
-  if (ep_way > 0 && (route == ARX_ROUTE_FP32 || !query_dev)) return ARX_EP_UNSUPPORTED;
   int rc = workspace_wait(h, st);
   if (rc) return rc;
   if (route == ARX_ROUTE_PAIR)
-    rc = score_gen3(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, ep_way, frames_stream);
+    rc = score_gen3(h, ti, q, n_windows, out, st, ep_way);
   else if (route == ARX_ROUTE_TILED)
-    rc = score_tcn(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, st, ep_way, frames_stream);
-  else if (frames_stream)
-    rc = ARX_EP_UNSUPPORTED;            // the caller materialises the windows for the fp32 kernels
+    rc = score_tcn(h, ti, q, n_windows, out, st, ep_way);
   else if (h->cfg.force_path == 2 && !debug_out)
     rc = arx_fail(h, ARX_ERR_INVALID, "score: force_path=2 but no tcgen05 path covers this shape (N=%d, D=%d)", tr.N, h->D);
   else {
     if (!debug_out) warn_fp32_fallback(h, ti);
-    rc = score_fp32(h, ti, query_dev, qfeats_dev, n_windows, logits_dev, is_true_dev, chosen_dev, probs, protos, st);
+    rc = score_fp32(h, ti, q, n_windows, out, st);
   }
   if (rc) return rc;
   return score_done_record(h, st);
@@ -1154,7 +1169,7 @@ int arx_score(arx_handle *h, const float *query_dev, int64_t n_windows, float *l
               void *stream) {
   if (!h || !query_dev || !logits_dev || n_windows < 0) return arx_fail(h, ARX_ERR_INVALID, "score: bad argument");
   if (!h->cfg.has_discriminator) is_true_dev = nullptr;
-  return score_impl(h, 0, query_dev, nullptr, n_windows, logits_dev, is_true_dev, chosen_dev, nullptr, nullptr,
+  return score_impl(h, 0, {query_dev, Query::WINDOWS, false}, n_windows, {logits_dev, is_true_dev, chosen_dev},
                     static_cast<cudaStream_t>(stream));
 }
 
@@ -1189,14 +1204,19 @@ int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_featu
     const float *sup = support_dev + (size_t)e0 * way * per_class;
     return is_features ? set_support_features(h, sup, (int32_t)n_classes, 1, st) : set_support_poses(h, sup, (int32_t)n_classes, 1, st);
   };
-  auto one_at_a_time = [&](int64_t e0, int64_t e1) -> int {      // the same kernels as set_support + arx_score
-    for (int64_t e = e0; e < e1; ++e) {
-      int rc = set_support(e, way);
-      if (rc) return rc;
-      rc = score_impl(h, 0, query_dev + (size_t)e * h->T * h->J3, nullptr, 1, logits_dev + e * way, is_true_dev ? is_true_dev + e : nullptr,
-                      chosen_dev ? chosen_dev + e : nullptr, nullptr, nullptr, st);
-      if (rc) return rc;
-    }
+  const Query q{query_dev, Query::WINDOWS, false};
+  // episodes [e0, e0 + m) against a pool of m*way support classes (ep_way = way), or one at a time against a support set of
+  // their own (ep_way = 0: the same kernels as set_support + arx_score)
+  auto score = [&](int64_t e0, int64_t m, int ep_way) -> int {
+    const int rc = set_support(e0, m * way);
+    if (rc) return rc;
+    return score_impl(h, 0, {q.at(h, e0), Query::WINDOWS, false}, m,
+                      {logits_dev + e0 * way, is_true_dev ? is_true_dev + e0 : nullptr, chosen_dev ? chosen_dev + e0 : nullptr},
+                      st, ep_way);
+  };
+  auto one_at_a_time = [&](int64_t e0, int64_t e1) -> int {
+    for (int64_t e = e0; e < e1; ++e)
+      if (const int rc = score(e, 1, 0)) return rc;
     return ARX_OK;
   };
   // The route depends on the configuration and the weights only: decided before any pool is built.  The fp32 kernels
@@ -1207,14 +1227,14 @@ int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_featu
   const int64_t piece = route == ARX_ROUTE_PAIR
                             ? 256
                             : std::max<int64_t>(1, std::min<int64_t>(256, (int64_t)(ARX_EPISODE_POOL_BUDGET / ((size_t)way * tiled_pool_class_bytes(h)))));
+  const bool disc = is_true_dev != nullptr;
   for (int64_t e0 = 0; e0 < n_episodes; e0 += piece) {
     const int64_t m = std::min(piece, n_episodes - e0);
-    int rc = set_support(e0, m * way);
-    if (rc) return rc;
-    rc = score_impl(h, 0, query_dev + (size_t)e0 * h->T * h->J3, nullptr, m, logits_dev + e0 * way, is_true_dev ? is_true_dev + e0 : nullptr,
-                    chosen_dev ? chosen_dev + e0 : nullptr, nullptr, nullptr, st, way);
-    if (rc == ARX_EP_UNSUPPORTED) rc = one_at_a_time(e0, e0 + m);      // pair pipeline: max_chunk below the pass
-    if (rc) return rc;
+    // the episode-mode kernels of the pair pipeline take no pool class offset: a pass must fit one chunk
+    const bool one_chunk = route != ARX_ROUTE_PAIR || pass_windows(h, m, [&](int64_t n, void *base) {
+      return carve_pair(h, h->tr[0], q, n, way, disc, base);
+    }) >= m;
+    if (const int rc = one_chunk ? score(e0, m, way) : one_at_a_time(e0, e0 + m)) return rc;
   }
   return ARX_OK;
 }
@@ -1223,24 +1243,16 @@ int arx_score_frames(arx_handle *h, const float *frames_dev, int64_t n_frames, f
                      void *stream) {
   if (!h || !frames_dev || !logits_dev || n_frames < 0) return arx_fail(h, ARX_ERR_INVALID, "score_frames: bad argument");
   if (!h->cfg.has_discriminator) is_true_dev = nullptr;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t n_windows = n_frames - h->T + 1;
   if (n_windows <= 0) return ARX_OK;                      // fewer than seq_len frames: nothing to report (ar.py:43-44)
-  int rc = score_impl(h, 0, frames_dev, nullptr, n_windows, logits_dev, is_true_dev, chosen_dev, nullptr, nullptr, st, 0, true);
-  if (rc != ARX_EP_UNSUPPORTED) return rc;
-  // shapes on the fp32 kernels: materialise the windows, then the ordinary path
-  float *win = nullptr;
-  ARX_CUDA(h, cudaMallocAsync(reinterpret_cast<void **>(&win), (size_t)n_windows * h->T * h->J3 * sizeof(float), st));
-  if ((rc = arx_make_windows_launch(h, frames_dev, win, n_windows, st)) == ARX_OK)
-    rc = score_impl(h, 0, win, nullptr, n_windows, logits_dev, is_true_dev, chosen_dev, nullptr, nullptr, st);
-  cudaFreeAsync(win, st);
-  return rc;
+  return score_impl(h, 0, {frames_dev, Query::FRAMES, false}, n_windows, {logits_dev, is_true_dev, chosen_dev},
+                    static_cast<cudaStream_t>(stream));
 }
 
 int arx_score_features(arx_handle *h, int32_t ti, const float *qfeats_dev, int64_t n_windows, float *logits_dev, void *stream) {
   if (!h || !qfeats_dev || !logits_dev || n_windows < 0 || ti < 0 || ti >= h->cfg.n_transformers)
     return arx_fail(h, ARX_ERR_INVALID, "score_features: bad argument");
-  return score_impl(h, ti, nullptr, qfeats_dev, n_windows, logits_dev, nullptr, nullptr, nullptr, nullptr,
+  return score_impl(h, ti, {qfeats_dev, Query::FEATURES, false}, n_windows, {logits_dev, nullptr, nullptr},
                     static_cast<cudaStream_t>(stream));
 }
 
@@ -1250,26 +1262,20 @@ int arx_debug_attention(arx_handle *h, const float *query_dev, int64_t n_windows
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float *logits = nullptr;
   ARX_CUDA(h, cudaMalloc(&logits, (size_t)std::max<int64_t>(1, n_windows) * h->way * sizeof(float)));
-  int rc = score_impl(h, 0, query_dev, nullptr, n_windows, logits, nullptr, nullptr, probs_dev, prototypes_dev, st);
+  int rc = score_impl(h, 0, {query_dev, Query::WINDOWS, false}, n_windows, {logits, nullptr, nullptr, probs_dev, prototypes_dev}, st);
   cudaStreamSynchronize(st);
   cudaFree(logits);
   return rc;
 }
 
 // fp16 host rows go straight into the fp16 operand image of the first GEMM (the fp32 path rounds to fp16 there anyway, so
-// results are bit-identical for inputs that are representable in fp16); only the T=16 pair pipeline and the tiled kernels
-// with tensor-core linear layers read halves
-static bool f16_input_ok(const arx_handle *h) {
-  const ArxRoute route = h->tr[0].route;
-  return h->tc_linears && (h->tc_variant & 4) == 0 && (route == ARX_ROUTE_PAIR || route == ARX_ROUTE_TILED);
-}
-
+// results are bit-identical for inputs that are representable in fp16)
 static int score_host_impl(arx_handle *h, const void *query_host_v, bool f16, int64_t n_windows, float *logits_host, float *is_true_host,
                            int32_t *chosen_host) {
   if (!h || !query_host_v || !logits_host || n_windows < 0) return arx_fail(h, ARX_ERR_INVALID, "score_host: bad argument");
   if (h->way < 1) return arx_fail(h, ARX_ERR_STATE, "score_host: support set not set");
   if (n_windows == 0) return ARX_OK;
-  if (f16 && !f16_input_ok(h)) return arx_fail(h, ARX_ERR_INVALID, "score_host_f16: fp16 rows need the tensor-core linear layers (this shape scores on the fp32 kernels)");
+  if (f16 && !tc_front_end(h, h->tr[0].route)) return arx_fail(h, ARX_ERR_INVALID, "score_host_f16: fp16 rows need the tensor-core linear layers (this shape scores on the fp32 kernels)");
   const char *query_host = static_cast<const char *>(query_host_v);
   const bool disc = h->cfg.has_discriminator && is_true_host;
   const int way = h->way;
@@ -1308,9 +1314,7 @@ static int score_host_impl(arx_handle *h, const void *query_host_v, bool f16, in
     int32_t *dch = reinterpret_cast<int32_t *>(dist + stage);
     ARX_CUDA(h, cudaMemcpyAsync(din, query_host + b0 * in_per, n * in_per, cudaMemcpyHostToDevice, st));
     if (i > 0) ARX_CUDA(h, cudaStreamWaitEvent(st, h->stage_ev[s ^ 1], 0));   // previous chunk done with the workspace
-    h->query_f16 = f16;
-    int rc = score_impl(h, 0, din, nullptr, n, dlog, disc ? dist : nullptr, dch, nullptr, nullptr, st);
-    h->query_f16 = false;
+    const int rc = score_impl(h, 0, {din, Query::WINDOWS, f16}, n, {dlog, disc ? dist : nullptr, dch}, st);
     if (rc) return rc;
     ARX_CUDA(h, cudaEventRecord(h->stage_ev[s], st));
     ARX_CUDA(h, cudaMemcpyAsync(logits_host + b0 * way, dlog, (size_t)n * way * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1334,7 +1338,7 @@ static int score_host_submit_impl(arx_handle *h, const void *query_host, bool f1
                                   int32_t *chosen_host, int64_t *ticket) {
   if (!h || !query_host || !logits_host || !ticket || n_windows <= 0) return arx_fail(h, ARX_ERR_INVALID, "score_host_submit: bad argument");
   if (h->way < 1) return arx_fail(h, ARX_ERR_STATE, "score_host_submit: support set not set");
-  if (f16 && !f16_input_ok(h)) return arx_fail(h, ARX_ERR_INVALID, "score_host_submit_f16: fp16 rows need the tensor-core linear layers");
+  if (f16 && !tc_front_end(h, h->tr[0].route)) return arx_fail(h, ARX_ERR_INVALID, "score_host_submit_f16: fp16 rows need the tensor-core linear layers");
   const bool disc = h->cfg.has_discriminator && is_true_host;
   const int way = h->way;
   const size_t in_per = (size_t)h->T * h->J3 * sizeof(float);          // staging is sized for fp32 rows (fp16 requests use half of it)
@@ -1376,9 +1380,7 @@ static int score_host_submit_impl(arx_handle *h, const void *query_host, bool f1
   // scoring: after its inputs arrived and after the results previously held in this slot went back to the host
   ARX_CUDA(h, cudaStreamWaitEvent(h->hs_comp, h->hs_ev_h2d[s], 0));
   if (slot_used) ARX_CUDA(h, cudaStreamWaitEvent(h->hs_comp, h->hs_ev_done[s], 0));
-  h->query_f16 = f16;
-  int rc = score_impl(h, 0, din, nullptr, n_windows, dlog, disc ? dist : nullptr, dch, nullptr, nullptr, h->hs_comp);
-  h->query_f16 = false;
+  const int rc = score_impl(h, 0, {din, Query::WINDOWS, f16}, n_windows, {dlog, disc ? dist : nullptr, dch}, h->hs_comp);
   if (rc) return rc;
   ARX_CUDA(h, cudaEventRecord(h->hs_ev_comp[s], h->hs_comp));
   ARX_CUDA(h, cudaStreamWaitEvent(h->hs_d2h, h->hs_ev_comp[s], 0));
@@ -1481,7 +1483,7 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
         ARX_CUDA(h, cudaEventCreateWithFlags(&s.ev_join, cudaEventDisableTiming));
       }
     }
-    const size_t need = carve_tcn(h, tr, 1, way, false, disc, false, nullptr).bytes;      // fp32 head buffers (one window: matvec kernels)
+    const size_t need = carve_tcn(h, tr, {nullptr, Query::FEATURES, false}, 1, way, disc, false, nullptr).bytes;      // fp32 head buffers (one window: matvec kernels)
     if (need > s.ws_bytes) {
       cudaFree(s.ws);
       s.ws = nullptr;
@@ -1496,7 +1498,7 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
     }
     s.way = way; s.sgen = h->support_seq; s.wgen = h->weights_gen;
   }
-  TcnWs w = carve_tcn(h, tr, 1, way, false, disc, false, s.ws);
+  TcnWs w = carve_tcn(h, tr, {nullptr, Query::FEATURES, false}, 1, way, disc, false, s.ws);
   auto body = [&]() -> int {
     int rc;
     if ((rc = prof_mark(h, 0, s.st))) return rc;          // stage timers: 0 H2D + frame MLP/projection, 1 window + query tiles, 2 -, 3 attention, 4 head + D2H
@@ -1569,7 +1571,7 @@ int arx_heads_forward(arx_handle *h, const float *feats_dev, int64_t n_frames, f
   __half *img = static_cast<__half *>(h->ws);
   for (int64_t f0 = 0; f0 < n_frames; f0 += chunk) {
     const int64_t rows = std::min(chunk, n_frames - f0) * 64;
-    if ((rc = arx_tc_rows_to_img(h, feats_dev + f0 * 64 * K, K, K, rows, img, nk, -1, st))) return rc;
+    if ((rc = arx_tc_rows_to_img(h, feats_dev + f0 * 64 * K, false, K, K, rows, img, nk, -1, st))) return rc;
     if ((rc = arx_tc_linear_f32(h, h->tl_heads, img, nk, rows, logits_dev + f0 * 64 * N, N, nullptr, 1, st, true))) return rc;
   }
   return score_done_record(h, st);

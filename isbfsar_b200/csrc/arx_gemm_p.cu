@@ -307,7 +307,7 @@ __global__ void __launch_bounds__(256, 2) k_tuple_img(const __grid_constant__ Tu
   if (tid == 0) bulk_wait_all();
 }
 
-template <int BN, int OUT, int NSTG> int launch_p(arx_handle *h, GemmPParams &p, cudaStream_t st) {
+template <int BN, int OUT, int NSTG> int launch_p(arx_handle *h, GemmPParams &p, int sms, cudaStream_t st) {
   const uint32_t fixed = p.nk * BN * 128 + 4 * NSTG * 4096 + BN * 4 + 256 + 1024;
   const uint32_t cap = 232448;
   int nsta = (int)((cap - fixed) / A_SUB);
@@ -317,7 +317,7 @@ template <int BN, int OUT, int NSTG> int launch_p(arx_handle *h, GemmPParams &p,
   const uint32_t smem = fixed + nsta * A_SUB;
   auto kern = k_gemm_p<BN, OUT, NSTG>;
   { const int rc_ = arx_func_smem(h, kern, (int)smem); if (rc_) return rc_; }
-  int grid = ((h->sm_count - h->sm_reserve) / p.n_tiles) * p.n_tiles;
+  int grid = (sms / p.n_tiles) * p.n_tiles;
   if (grid > p.m_tiles * p.n_tiles) grid = p.m_tiles * p.n_tiles;
   kern<<<grid, P_THREADS, smem, st>>>(p);
   ARX_LAUNCH_CHECK(h);
@@ -328,29 +328,29 @@ template <int BN, int OUT, int NSTG> int launch_p(arx_handle *h, GemmPParams &p,
 
 bool arx_tcp_supported(const ArxTcLinear &L) { return (L.BN == 256 || L.BN == 192) && (size_t)L.nk * L.BN * 128 + 2 * A_SUB + 4 * 4096 + 4096 <= 232448; }
 
-// act(A.W^T + b) -> fp16 activation image with c_nk K-sub-tiles per row tile (persistent kernel)
+// act(A.W^T + b) -> fp16 activation image with c_nk K-sub-tiles per row tile (persistent kernel on `sms` SMs)
 int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                       cudaStream_t st) {
+                       int sms, cudaStream_t st) {
   GemmPParams p{};
   p.a_img = a_img; p.w_img = L.w_img; p.bias = L.bias; p.nk = L.nk; p.a_nk = L.nk; p.m_tiles = (int)((M + 127) / 128); p.n_tiles = L.n_tiles;
   p.act = act; p.c_img = c_img; p.c_nk = c_nk; p.onehot_sub = onehot_sub;
-  if (L.BN == 192) return launch_p<192, POUT_IMG16, 4>(h, p, st);
-  if (L.BN == 256) return launch_p<256, POUT_IMG16, 4>(h, p, st);
+  if (L.BN == 192) return launch_p<192, POUT_IMG16, 4>(h, p, sms, st);
+  if (L.BN == 256) return launch_p<256, POUT_IMG16, 4>(h, p, sms, st);
   return arx_fail(h, ARX_ERR_INVALID, "tcp_linear_img: unsupported BN %d", L.BN);
 }
 
 // A.W^T -> chunked fp32 projections Gc (see the file header); the buffer holds ceil(M/128)*128 rows
-int arx_tcp_linear_chunked(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *gc, cudaStream_t st) {
+int arx_tcp_linear_chunked(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *gc, int sms, cudaStream_t st) {
   GemmPParams p{};
   p.a_img = a_img; p.w_img = L.w_img; p.bias = nullptr; p.nk = L.nk; p.a_nk = a_nk; p.m_tiles = (int)((M + 127) / 128); p.n_tiles = L.n_tiles;
   p.act = ARX_ACT_NONE; p.gc = gc; p.onehot_sub = -1;
-  if (L.BN == 256) return launch_p<256, POUT_F32C, 1>(h, p, st);
+  if (L.BN == 256) return launch_p<256, POUT_F32C, 1>(h, p, sms, st);
   return arx_fail(h, ARX_ERR_INVALID, "tcp_linear_chunked: unsupported BN %d", L.BN);
 }
 
 // Kq operand images of n_win query windows from the chunked per-frame K projections (T=16 pair tuples, slot order)
 int arx_tuple_img(arx_handle *h, const ArxTransformer &tr, const float *gc, int n_chunks, int64_t n_win, __half *kq_img, float alpha,
-                  cudaStream_t st) {
+                  int sms, cudaStream_t st) {
   if (!(h->dev_init & ARX_INIT_PSLOTS)) {         // __constant__ symbols are per device: once per handle, not per process
     int32_t slots[256];
     arx_tc2_slot_table(slots);
@@ -359,7 +359,7 @@ int arx_tuple_img(arx_handle *h, const ArxTransformer &tr, const float *gc, int 
   }
   const uint32_t smem = 65536 + 16 * TI_STRIDE * 4 + 1024 + 128;
   { const int rc_ = arx_func_smem(h, k_tuple_img, (int)smem); if (rc_) return rc_; }
-  const int64_t grid = n_win < 2 * (h->sm_count - h->sm_reserve) ? n_win : 2 * (h->sm_count - h->sm_reserve);
+  const int64_t grid = n_win < 2 * sms ? n_win : 2 * sms;
   TupleParams p{};
   for (int d = 0; d < 128; ++d) { p.gs[d] = tr.ln_host[d] * alpha; p.gs[128 + d] = tr.ln_host[128 + d] * alpha; }
   p.gc = gc; p.kq_img = kq_img; p.n_chunks = n_chunks; p.n_win = (int)n_win;

@@ -286,14 +286,15 @@ int arx_tc_linear_prepare(arx_handle *h, ArxTcLinear &L, const float *W, int ldw
   return ARX_OK;
 }
 
-int arx_tc_rows_to_img(arx_handle *h, const float *X, int lda, int K, int64_t M, __half *img, int nk, int onehot_sub, cudaStream_t st) {
+int arx_tc_rows_to_img(arx_handle *h, const void *X, bool f16, int lda, int K, int64_t M, __half *img, int nk, int onehot_sub, cudaStream_t st) {
   const int64_t total = ((M + 127) / 128) * 128 * nk * 8;
-  if (h->query_f16) {          // the caller's rows are fp16 (arx_score_host*_f16): same image, no rounding step
-    k_rows_to_img<__half><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(reinterpret_cast<const __half *>(X), lda, K, M, img, nk, onehot_sub);
+  if (f16) {          // fp16 rows (arx_score_host*_f16): same image, no rounding step
+    k_rows_to_img<__half><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(static_cast<const __half *>(X), lda, K, M, img, nk, onehot_sub);
     ARX_LAUNCH_CHECK(h);
     return ARX_OK;
   }
-  ARX_CUDA(h, arx_launch_pdl(k_rows_to_img<float>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, h->pdl, X, lda, K, M, img, nk, onehot_sub));
+  ARX_CUDA(h, arx_launch_pdl(k_rows_to_img<float>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, h->pdl,
+                             static_cast<const float *>(X), lda, K, M, img, nk, onehot_sub));
   h->launches++;
   return ARX_OK;
 }

@@ -174,7 +174,6 @@ struct arx_handle {
   double prof_ms[ARX_N_STAGES] = {0, 0, 0, 0, 0};
   int64_t prof_chunks = 0;
   int last_path = 0;
-  bool query_f16 = false;       // set around a scoring pass whose query rows are fp16 (arx_score_host*_f16): first-stage image kernel reads halves
   std::vector<ArxScoreGraph> graphs;     // small LRU cache (arx_score with recurring arguments)
   uint64_t graph_tick = 0, support_gen = 0, weights_gen = 0;
   uint64_t support_seq = 0;              // increments whenever a new support set is set / imported
@@ -191,8 +190,7 @@ struct arx_handle {
   float mlp_bias_host[192 + 256] = {};   // host copies of the (zero padded) fc1 / fc2 biases: kernel-parameter operands of k_mlp_p
   bool mlp_bias_host_ok = false;
   bool support_inflight = false;    // a support chain was forked onto the side stream and no scoring pass has joined it yet
-  int sm_reserve_n = 4;             // how many (environment variable ARX_SM_RESERVE overrides)
-  int sm_reserve = 0;               // SMs the persistent front-end kernels leave free (for that chain) during the current pass
+  int sm_reserve_n = 4;             // SMs the persistent front-end kernels leave free for that chain (environment variable ARX_SM_RESERVE overrides)
   int tcn_free_a = 1;               // tiled attention, pass A: softmax groups free-running (debug key 7)
   int tcn_poly = 1;                 // tiled attention, pass A: half of the exponentials on the FMA pipe (debug key 6)
   int *tcn_diag = nullptr;          // watchdog record of the tiled attention kernel
@@ -269,7 +267,8 @@ int arx_tc_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_i
 
 // ---- tcgen05 GEMM (arx_gemm_tc.cu) ------------------------------------------------
 int arx_tc_linear_prepare(arx_handle *h, ArxTcLinear &L, const float *W, int ldw, const float *bias, int N, int K, int BN, cudaStream_t st);
-int arx_tc_rows_to_img(arx_handle *h, const float *X, int lda, int K, int64_t M, __half *img, int nk, int onehot_sub, cudaStream_t st);
+// rows X (M, K; fp32, or fp16 when `f16`) -> fp16 operand image
+int arx_tc_rows_to_img(arx_handle *h, const void *X, bool f16, int lda, int K, int64_t M, __half *img, int nk, int onehot_sub, cudaStream_t st);
 int arx_tc_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
                       cudaStream_t st);
 int arx_tc_linear_f32(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *C, int ldc, const float *table, int T,
@@ -312,14 +311,15 @@ int arx_tc3_attention_launch(arx_handle *h, const ArxTransformer &tr, const __ha
                              float *partial, int g_ld, int g_voff, bool g_chunked, bool episodes, cudaStream_t st);
 // ---- persistent GEMM + tuple images (arx_gemm_p.cu)
 bool arx_tcp_supported(const ArxTcLinear &L);
+// The persistent kernels below run on at most `sms` SMs (fewer than sm_count leave room to a support chain in flight).
 // fused frame MLP (arx_mlp_p.cu)
 bool arx_mlp_fused_supported(const arx_handle *h, const void *x);
-int arx_mlp_fused(arx_handle *h, const void *x, bool f16, int64_t rows, __half *f_img, int c_nk, int onehot_sub, cudaStream_t st);
+int arx_mlp_fused(arx_handle *h, const void *x, bool f16, int64_t rows, __half *f_img, int c_nk, int onehot_sub, int sms, cudaStream_t st);
 int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                       cudaStream_t st);
-int arx_tcp_linear_chunked(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *gc, cudaStream_t st);
+                       int sms, cudaStream_t st);
+int arx_tcp_linear_chunked(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *gc, int sms, cudaStream_t st);
 int arx_tuple_img(arx_handle *h, const ArxTransformer &tr, const float *gc, int n_chunks, int64_t n_win, __half *kq_img, float alpha,
-                  cudaStream_t st);
+                  int sms, cudaStream_t st);
 
 // ---- tiled any-N tcgen05 attention (arx_tcn.cu)
 bool arx_tcn_supported(const arx_handle *h, const ArxTransformer &tr);
@@ -348,7 +348,6 @@ int arx_stream_tail_launch(arx_handle *h, const ArxTransformer &tr, const float 
 
 int arx_form_windows_launch(arx_handle *h, const ArxTransformer &tr, const float *P, const float *U, float *G, float *uab, int64_t n_win, bool chunked,
                             cudaStream_t st);
-int arx_make_windows_launch(arx_handle *h, const float *frames, float *win, int64_t n_win, cudaStream_t st);
 
 // ---- tuple table (arx_tuples.cu) -------------------------------------------------
 int arx_build_tuple_table(arx_handle *h, int T, int c, int N, int32_t *out_dev, cudaStream_t st);

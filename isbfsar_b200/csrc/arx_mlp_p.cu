@@ -278,15 +278,16 @@ bool arx_mlp_fused_supported(const arx_handle *h, const void *x) {
          (reinterpret_cast<uintptr_t>(x) & 7u) == 0;
 }
 
-// f_img[m_tiles][c_nk] = relu(fc2(relu(fc1(x)))) (+ the one-hot sub-tile at index onehot_sub, -1 = none); x (rows, J3) fp32, or fp16 when `f16`
-int arx_mlp_fused(arx_handle *h, const void *x, bool f16, int64_t rows, __half *f_img, int c_nk, int onehot_sub, cudaStream_t st) {
+// f_img[m_tiles][c_nk] = relu(fc2(relu(fc1(x)))) (+ the one-hot sub-tile at index onehot_sub, -1 = none); x (rows, J3) fp32, or fp16 when `f16`;
+// persistent on at most `sms` SMs
+int arx_mlp_fused(arx_handle *h, const void *x, bool f16, int64_t rows, __half *f_img, int c_nk, int onehot_sub, int sms, cudaStream_t st) {
   MlpParams p{};
   p.x = x; p.w1_img = h->tl_fc1.w_img; p.w2_img = h->tl_fc2.w_img; p.f_img = f_img; p.rows = rows;
   p.trace = h->trace_sel == 2 ? h->trace_buf : nullptr;
   p.m_tiles = (int)((rows + 127) / 128); p.c_nk = c_nk; p.onehot_sub = onehot_sub; p.k16_1 = (h->J3 + 15) / 16;
   memcpy(p.b1, h->mlp_bias_host, sizeof(p.b1));
   memcpy(p.b2, h->mlp_bias_host + BN1, sizeof(p.b2));
-  const int grid = p.m_tiles < h->sm_count - h->sm_reserve ? p.m_tiles : h->sm_count - h->sm_reserve;
+  const int grid = p.m_tiles < sms ? p.m_tiles : sms;
   if (f16) {
     auto kern = k_mlp_p<__half, 45>;
     { const int rc_ = arx_func_smem(h, kern, (int)SMEM_BYTES); if (rc_) return rc_; }

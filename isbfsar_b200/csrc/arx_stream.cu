@@ -235,15 +235,6 @@ __global__ void __launch_bounds__(256) k_form_windows(const float *__restrict__ 
   }
 }
 
-// explicit windows (n_win, T, J3) from a frame stream: the generic route for shapes on the fp32 kernels
-__global__ void k_make_windows(const float *__restrict__ frames, float *__restrict__ win, int64_t n_win, int T, int J3) {
-  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= n_win * T * J3) return;
-  const int64_t w = idx / ((int64_t)T * J3);
-  const int64_t r = idx - w * T * J3;
-  win[idx] = frames[w * J3 + r];
-}
-
 }  // namespace
 
 int arx_stream_frame_launch(arx_handle *h, const ArxTransformer &tr, const float *x_dev, float *ring, int *slot_next, cudaStream_t st) {
@@ -279,13 +270,6 @@ int arx_form_windows_launch(arx_handle *h, const ArxTransformer &tr, const float
   const int NO = 2 * tr.c * h->D;
   const int64_t total = n_win * h->T * (NO / 4 + (U ? 8 : 0));
   k_form_windows<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(P, U, tr.bp, tr.tcomp, G, uab, n_win, h->T, NO, chunked ? 1 : 0);
-  ARX_LAUNCH_CHECK(h);
-  return ARX_OK;
-}
-
-int arx_make_windows_launch(arx_handle *h, const float *frames, float *win, int64_t n_win, cudaStream_t st) {
-  const int64_t total = n_win * h->T * h->J3;
-  k_make_windows<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(frames, win, n_win, h->T, h->J3);
   ARX_LAUNCH_CHECK(h);
   return ARX_OK;
 }

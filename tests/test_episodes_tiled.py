@@ -192,3 +192,20 @@ def test_pair_pipeline_unchanged():
             counts[b] = m.launch_count() - l0
             assert m.last_path() == 2
     assert counts[28] == counts[256], counts
+
+
+# ---- 8. the pair pipeline with a pass larger than one chunk scores episode by episode ----------------------------------
+def test_pair_pipeline_past_one_chunk_equals_loop():
+    cfg = Cfg()
+    m, _ = make_model(cfg, 0, max_chunk=100)                     # 256 episodes per pass do not fit one chunk
+    support, query = episodes(cfg, 256, 5, 29)
+    S, Q = torch.from_numpy(support).cuda(), torch.from_numpy(query).cuda()
+    loop(m, S[:1], Q[:1])                                        # one-time tables of the handle's first scoring pass
+    l0 = m.launch_count()
+    lg, it = m.score_episodes(Q, poses=S)
+    l1 = m.launch_count()
+    assert m.last_path() == 2
+    rl, ri = loop(m, S, Q)
+    l2 = m.launch_count()
+    assert torch.equal(lg, rl) and torch.equal(it, ri)
+    assert l1 - l0 == l2 - l1, (l1 - l0, l2 - l1)

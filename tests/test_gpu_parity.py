@@ -993,6 +993,8 @@ def test_frame_stream_scoring_equals_explicit_windows(cfg, n_frames, path, force
     lo_w, it_w = m.score(windows)
     tol = tol_for(m)
     assert rel_err(lo_s.cpu(), lo_w.cpu()).max() < tol and rel_err(it_s.cpu(), it_w.cpu()).max() < tol
+    if path == 1:       # k_linear adds the positional table after the accumulation, like k_form_windows: the same bits
+        assert torch.equal(lo_s, lo_w) and torch.equal(it_s, it_w)
     k = min(48, windows.shape[0])
     lo, it = TrxOracle(cfg, sd).score(support[None], np.arange(cfg.way)[None], windows[:k].cpu().numpy(), chunk=16)
     assert rel_err(lo_s[:k].cpu(), lo).max() < tol and rel_err(it_s[:k].cpu(), it).max() < tol
@@ -1001,3 +1003,37 @@ def test_frame_stream_scoring_equals_explicit_windows(cfg, n_frames, path, force
     # fewer than seq_len frames: nothing to score
     e_lo, e_it = m.score_frames(F[:T - 1])
     assert e_lo.shape == (0, cfg.way)
+
+
+@pytest.mark.parametrize("cfg,path,force", [(Cfg(), 1, 1), (Cfg(way=3, seq_len=8), 3, 0), (Cfg(), 2, 0)], ids=["fp32", "tiled", "pair"])
+def test_frame_stream_chunks_are_bit_identical(cfg, path, force):
+    """arx_score_frames split into passes of 7 windows: every pass starts at its own frame, same bits as one pass."""
+    T = cfg.seq_len
+    rng = np.random.default_rng(31)
+    support = torch.from_numpy((0.17 * rng.standard_normal((cfg.way, T, 90))).astype(np.float32)).cuda()
+    frames = torch.from_numpy((0.17 * rng.standard_normal((T + 40, 90))).astype(np.float32)).cuda()
+    res = []
+    for mc in (0, 7):
+        m, _ = make_model(cfg, 0, force_path=force, max_chunk=mc)
+        m.set_support(poses=support)
+        res.append(m.score_frames(frames))
+        assert m.last_path() == path
+    assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1], res[1][1])
+
+
+@pytest.mark.parametrize("cfg,B,max_chunk,path", [(Cfg(), 600, 0, 2), (Cfg(way=20, seq_len=32, temp_set=[2, 3]), 40, 7, 3)],
+                         ids=["pair", "tiled_chunked"])
+def test_fp16_and_fp32_host_rows_alternate_on_one_handle(cfg, B, max_chunk, path):
+    """fp32 and fp16 rows of the same values, alternating on one handle: the first call of each runs eagerly, the second is
+    captured, the third replayed (pair pipeline), and a pass never reads the other precision's rows or graph."""
+    m, _ = make_model(cfg, 0, max_chunk=max_chunk)
+    support, _, query, _ = make_episode(cfg, B, 143, "structured")
+    q16 = torch.from_numpy(query).to(torch.float16).pin_memory()
+    q32 = q16.to(torch.float32).pin_memory()
+    m.set_support(poses=torch.from_numpy(support[0]).cuda())
+    ref = m.score_host(q32)
+    for _ in range(3):
+        for q in (q32, q16):
+            for r in (m.score_host(q), m.score_host_async(q).result()):
+                assert m.last_path() == path
+                assert torch.equal(r[0], ref[0]) and torch.equal(r[1], ref[1])
