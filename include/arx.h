@@ -48,7 +48,11 @@ typedef enum arx_status {
 /* Mirror of the TRXConfig fields the path reads (utils/params.py:50-95). */
 typedef struct arx_config {
   int32_t seq_len;        /* T; 16 (utils/params.py:8)                                   */
-  int32_t n_joints;       /* J; MLP input = 3*J, hidden = 6*J (model.py:269)             */
+  int32_t n_joints;       /* J; MLP input = 3*J, hidden = 6*J (model.py:269).  Any J > 0:
+                             J <= 32 runs the frame MLP on the tensor-core linears (the fused
+                             k_mlp_p at J = 30 only), J >= 33 on the fp32 CUDA cores, and T=16
+                             pairs then score on the tiled route.  The resident streaming scorer
+                             (arx_stream_push) serves J <= 42, the fp16 host rows J <= 32.   */
   int32_t feat_dim;       /* F = trans_linear_in_dim = MLP output = 256                  */
   int32_t out_dim;        /* D = trans_linear_out_dim = 128                              */
   int32_t n_transformers; /* len(temp_set) (model.py:279)                                */

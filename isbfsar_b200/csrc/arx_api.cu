@@ -193,13 +193,15 @@ int embed_frames(arx_handle *h, const float *X, int64_t rows, float *H1, float *
 }
 
 // the same on tensor cores, three launches: frames (fp32, or fp16 when `f16`) -> fp16 image x_img -> fc1 -> h_img -> fc2 ->
-// feature image f_img (f_nk sub-tiles; f_onehot: the one-hot sub-tile of the positional table, or -1)
+// feature image f_img (f_nk sub-tiles; f_onehot: the one-hot sub-tile of the positional table, or -1).  h_img keeps fc1's
+// whole column tile per row tile (3 sub-tiles), not the ceil(6J/64) fc2 reads: fc1 writes its pad columns too.
 int embed_frames_tc(arx_handle *h, const void *X, bool f16, int64_t rows, __half *x_img, __half *h_img, __half *f_img, int f_nk, int f_onehot,
                     cudaStream_t st) {
   int rc;
+  const int h_nk = arx_tc_img_nk(h->tl_fc1);
   if ((rc = arx_tc_rows_to_img(h, X, f16, h->J3, h->J3, rows, x_img, h->tl_fc1.nk, -1, st))) return rc;
-  if ((rc = arx_tc_linear_img(h, h->tl_fc1, x_img, rows, ARX_ACT_RELU, h_img, h->tl_fc2.nk, -1, st))) return rc;
-  return arx_tc_linear_img(h, h->tl_fc2, h_img, rows, ARX_ACT_RELU, f_img, f_nk, f_onehot, st);
+  if ((rc = arx_tc_linear_img(h, h->tl_fc1, x_img, h->tl_fc1.nk, rows, ARX_ACT_RELU, h_img, h_nk, -1, st))) return rc;
+  return arx_tc_linear_img(h, h->tl_fc2, h_img, h_nk, rows, ARX_ACT_RELU, f_img, f_nk, f_onehot, st);
 }
 
 // discriminator MLP on the CUDA cores: head input y (n, N*T) -> d1 -> d2 -> d3 + sigmoid   (model.py:183-204)
@@ -213,7 +215,7 @@ int disc_tail_fp32(arx_handle *h, const ArxTransformer &tr, const float *y, floa
 
 // the same on tensor cores from the head input image y_img: d1 -> h1_img, then d2 + d3 + sigmoid in one launch
 int disc_tail_tc(arx_handle *h, const __half *y_img, __half *h1_img, int64_t n, float *is_true, cudaStream_t st) {
-  const int rc = arx_tc_linear_img(h, h->tl_d1, y_img, n, ARX_ACT_RELU, h1_img, h->tl_d2.nk, -1, st);
+  const int rc = arx_tc_linear_img(h, h->tl_d1, y_img, h->tl_d1.nk, n, ARX_ACT_RELU, h1_img, h->tl_d2.nk, -1, st);
   if (rc) return rc;
   return arx_tc_linear_sigmoid_dot(h, h->tl_d2, h1_img, n, h->d3_w, h->d3_b, is_true, st);
 }
@@ -1055,8 +1057,9 @@ static int score_gen3(arx_handle *h, int ti, const Query &q, int64_t n_windows, 
         if ((rc = arx_mlp_fused(h, xq, q.f16, rows, w.f_img, f_nk, f_onehot, sms, st))) return rc;      // one launch: poses -> feature image
       } else if (p_embed) {
         if ((rc = arx_tc_rows_to_img(h, xq, q.f16, h->J3, h->J3, rows, w.x_img, h->tl_fc1.nk, -1, st))) return rc;
-        if ((rc = arx_tcp_linear_img(h, h->tl_fc1, w.x_img, rows, ARX_ACT_RELU, w.h_img, h->tl_fc2.nk, -1, sms, st))) return rc;
-        if ((rc = arx_tcp_linear_img(h, h->tl_fc2, w.h_img, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, sms, st))) return rc;
+        const int h_nk = arx_tc_img_nk(h->tl_fc1);          // as in embed_frames_tc
+        if ((rc = arx_tcp_linear_img(h, h->tl_fc1, w.x_img, h->tl_fc1.nk, rows, ARX_ACT_RELU, w.h_img, h_nk, -1, sms, st))) return rc;
+        if ((rc = arx_tcp_linear_img(h, h->tl_fc2, w.h_img, h_nk, rows, ARX_ACT_RELU, w.f_img, f_nk, f_onehot, sms, st))) return rc;
       } else if ((rc = embed_frames_tc(h, xq, q.f16, rows, w.x_img, w.h_img, w.f_img, f_nk, f_onehot, st))) return rc;
       if ((rc = prof_mark(h, 1, st))) return rc;
       if ((rc = arx_tcp_linear_chunked(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, sms, st))) return rc;

@@ -329,10 +329,14 @@ template <int BN, int OUT, int NSTG> int launch_p(arx_handle *h, GemmPParams &p,
 bool arx_tcp_supported(const ArxTcLinear &L) { return (L.BN == 256 || L.BN == 192) && (size_t)L.nk * L.BN * 128 + 2 * A_SUB + 4 * 4096 + 4096 <= 232448; }
 
 // act(A.W^T + b) -> fp16 activation image with c_nk K-sub-tiles per row tile (persistent kernel on `sms` SMs)
-int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                       int sms, cudaStream_t st) {
+int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, int act, __half *c_img, int c_nk,
+                       int onehot_sub, int sms, cudaStream_t st) {
+  // the epilogue writes every sub-tile of every column tile, pad columns included
+  if (a_nk < L.nk || c_nk < arx_tc_img_nk(L))
+    return arx_fail(h, ARX_ERR_INVALID, "tcp_linear_img: image layout too narrow (a_nk %d < nk %d, or c_nk %d < %d sub-tiles written)", a_nk, L.nk,
+                    c_nk, arx_tc_img_nk(L));
   GemmPParams p{};
-  p.a_img = a_img; p.w_img = L.w_img; p.bias = L.bias; p.nk = L.nk; p.a_nk = L.nk; p.m_tiles = (int)((M + 127) / 128); p.n_tiles = L.n_tiles;
+  p.a_img = a_img; p.w_img = L.w_img; p.bias = L.bias; p.nk = L.nk; p.a_nk = a_nk; p.m_tiles = (int)((M + 127) / 128); p.n_tiles = L.n_tiles;
   p.act = act; p.c_img = c_img; p.c_nk = c_nk; p.onehot_sub = onehot_sub;
   if (L.BN == 192) return launch_p<192, POUT_IMG16, 4>(h, p, sms, st);
   if (L.BN == 256) return launch_p<256, POUT_IMG16, 4>(h, p, sms, st);

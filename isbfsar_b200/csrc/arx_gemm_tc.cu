@@ -300,10 +300,14 @@ int arx_tc_rows_to_img(arx_handle *h, const void *X, bool f16, int lda, int K, i
 }
 
 // act(A.W^T + b) -> fp16 activation image with c_nk K-sub-tiles per row tile
-int arx_tc_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                      cudaStream_t st) {
+int arx_tc_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, int act, __half *c_img, int c_nk,
+                      int onehot_sub, cudaStream_t st) {
+  // the epilogue writes every sub-tile of every column tile, pad columns included
+  if (a_nk < L.nk || c_nk < arx_tc_img_nk(L))
+    return arx_fail(h, ARX_ERR_INVALID, "tc_linear_img: image layout too narrow (a_nk %d < nk %d, or c_nk %d < %d sub-tiles written)", a_nk, L.nk,
+                    c_nk, arx_tc_img_nk(L));
   GemmParams p{};
-  p.a_img = a_img; p.w_img = L.w_img; p.bias = L.bias; p.nk = L.nk; p.a_nk = L.nk; p.M = M; p.act = act; p.c_img = c_img; p.c_nk = c_nk;
+  p.a_img = a_img; p.w_img = L.w_img; p.bias = L.bias; p.nk = L.nk; p.a_nk = a_nk; p.M = M; p.act = act; p.c_img = c_img; p.c_nk = c_nk;
   p.onehot_sub = onehot_sub;
   if (L.BN == 192) return launch_gemm<192, OUT_IMG16>(h, p, L.n_tiles, st);
   if (L.BN == 256) return launch_gemm<256, OUT_IMG16>(h, p, L.n_tiles, st);

@@ -267,10 +267,14 @@ int arx_tc_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_i
 
 // ---- tcgen05 GEMM (arx_gemm_tc.cu) ------------------------------------------------
 int arx_tc_linear_prepare(arx_handle *h, ArxTcLinear &L, const float *W, int ldw, const float *bias, int N, int K, int BN, cudaStream_t st);
+// 64-column sub-tiles per row tile that the fp16 image epilogues of layer L write: every column of its n_tiles column tiles
+inline int arx_tc_img_nk(const ArxTcLinear &L) { return L.n_tiles * L.BN / 64; }
 // rows X (M, K; fp32, or fp16 when `f16`) -> fp16 operand image
 int arx_tc_rows_to_img(arx_handle *h, const void *X, bool f16, int lda, int K, int64_t M, __half *img, int nk, int onehot_sub, cudaStream_t st);
-int arx_tc_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                      cudaStream_t st);
+// Activation image of one layer for the next: a_img has a_nk >= L.nk sub-tiles per row tile; c_img gets c_nk sub-tiles per row
+// tile, at least the n_tiles * BN / 64 this layer writes (arx_tc_img_nk), or a row tile's pad columns land in the next one
+int arx_tc_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, int act, __half *c_img, int c_nk,
+                      int onehot_sub, cudaStream_t st);
 int arx_tc_linear_f32(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *C, int ldc, const float *table, int T,
                       cudaStream_t st, bool with_bias = false);
 int arx_tc_linear_sigmoid_dot(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, const float *w3, const float *b3, float *out,
@@ -315,8 +319,8 @@ bool arx_tcp_supported(const ArxTcLinear &L);
 // fused frame MLP (arx_mlp_p.cu)
 bool arx_mlp_fused_supported(const arx_handle *h, const void *x);
 int arx_mlp_fused(arx_handle *h, const void *x, bool f16, int64_t rows, __half *f_img, int c_nk, int onehot_sub, int sms, cudaStream_t st);
-int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int64_t M, int act, __half *c_img, int c_nk, int onehot_sub,
-                       int sms, cudaStream_t st);
+int arx_tcp_linear_img(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, int act, __half *c_img, int c_nk,
+                       int onehot_sub, int sms, cudaStream_t st);
 int arx_tcp_linear_chunked(arx_handle *h, const ArxTcLinear &L, const __half *a_img, int a_nk, int64_t M, float *gc, int sms, cudaStream_t st);
 int arx_tuple_img(arx_handle *h, const ArxTransformer &tr, const float *gc, int n_chunks, int64_t n_win, __half *kq_img, float alpha,
                   int sms, cudaStream_t st);
