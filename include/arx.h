@@ -56,7 +56,12 @@ typedef struct arx_config {
   int32_t feat_dim;       /* F = trans_linear_in_dim = MLP output = 256                  */
   int32_t out_dim;        /* D = trans_linear_out_dim = 128                              */
   int32_t n_transformers; /* len(temp_set) (model.py:279)                                */
-  int32_t cardinality[ARX_MAX_TRANSFORMERS]; /* temp_set entries, 2 or 3                 */
+  int32_t cardinality[ARX_MAX_TRANSFORMERS]; /* temp_set entries c, 1..min(4, seq_len).
+                             With N = C(T,c) tuples: T=16 pairs take the pair pipeline, other
+                             c = 2 or 3 with N >= 28 the tiled tcgen05 kernels, and c = 1 or 4,
+                             or N < 28 (pairs up to T=7, triples up to T=6), the fp32 CUDA-core
+                             kernels.  A handle with no transformer of N >= 28 runs its frame MLP
+                             and projections on the fp32 CUDA cores as well (DESIGN 4).    */
   int32_t has_discriminator; /* 1 for model="DISC" (model.py:282-285)                    */
   int32_t max_chunk;      /* windows processed per internal pass (0 = default)           */
   int32_t force_path;     /* 0 = auto, 1 = fp32 CUDA-core kernels, 2 = tcgen05 kernels   *
@@ -124,9 +129,11 @@ ARX_API int arx_import_support(arx_handle *h, const void *blob_dev, int32_t way,
  *   query_dev (B,T,3J) -> logits_dev (B,W) [= -distance], is_true_dev (B) in (0,1)
  *   [may be NULL / ignored without discriminator], chosen_dev (B) int32 argmax
  *   (first maximum on ties, model.py:323) [may be NULL].
- * The discriminator is sized for pair tuples (model.py:282-285): is_true needs temp_set[0] = 2.  On the tiled tcgen05
- * kernels the open-set head covers every seq_len the handle accepts (2..64); the head's T columns are accumulator lanes
- * of the attention kernel's head mode. */
+ * The discriminator is sized for pair tuples (model.py:282-285): is_true needs temp_set[0] = 2, and other cardinalities
+ * with the discriminator are refused (ARX_ERR_INVALID).  On the tiled tcgen05 kernels the open-set head covers every
+ * seq_len from 8 to 64; the head's T columns are accumulator lanes of the attention kernel's head mode.  Below 28 query
+ * tuples (T <= 7) the fp32 kernels score pairs, head included: there the fp16 / bf16 operands of the tiled kernels miss the
+ * 1e-3 tolerance.  Which (T, c) take which kernels: arx_config.cardinality. */
 ARX_API int arx_score(arx_handle *h, const float *query_dev, int64_t n_windows,
               float *logits_dev, float *is_true_dev, int32_t *chosen_dev, void *stream);
 
@@ -145,7 +152,8 @@ ARX_API int arx_score_frames(arx_handle *h, const float *frames_dev, int64_t n_f
  * episodes go through the batched kernels a pass at a time: the support operands of the pass's episodes*way classes
  * form one pool, and window i attends classes [i*way, (i+1)*way) of it.  A pass holds 256 episodes on the pair
  * pipeline; on the tiled kernels as many as keep the pool within 1 GiB (at least one, at most 256).  The fp32 route
- * (force_path = 1, LayerNorm affines past the accuracy bound, D != 128) scores one episode at a time.
+ * (force_path = 1, LayerNorm affines past the accuracy bound, D != 128, c = 1 or 4, fewer than 28 tuples) scores one
+ * episode at a time.
  * The pool holds the support operands of transformers[0] only, the transformer that scores episodes (model.py:320).
  *   support_dev (n_episodes, way, T, 3J) poses, or (n_episodes, way, T, F) frame features when is_features != 0
  *   (the ss_features argument); query_dev (n_episodes, T, 3J); outputs as arx_score.
@@ -195,7 +203,8 @@ ARX_API int arx_score_host_wait(arx_handle *h, int64_t ticket);
  * (transformers[0] + discriminator) and returns result_host[0..way) = softmax(logits) (ar.py:77), result_host[way] = is_true
  * (ar.py:78).  *valid = 0 until seq_len frames have been pushed since the last reset (ar.py:43-44).  One H2D (the frame),
  * one CUDA-graph launch and one D2H per call; synchronises the handle's internal stream.  Pair tuples only (with or
- * without the discriminator, any seq_len up to 64), on the tiled tcgen05 kernels.
+ * without the discriminator, seq_len 8..64), on the tiled tcgen05 kernels; ARX_ERR_INVALID for shapes that score on the
+ * fp32 kernels (seq_len <= 7 among them), where ActionRecognizer scores each window through arx_score instead.
  * arx_stream_reset forgets the window (previous_frames = []). */
 ARX_API int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, int32_t *valid);
 ARX_API int arx_stream_reset(arx_handle *h);

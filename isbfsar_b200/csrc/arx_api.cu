@@ -397,9 +397,13 @@ int arx_load_weights(arx_handle *h, const arx_weights *w, void *stream) {
     UP(h->d3_w, w->d3_w, 64); UP(h->d3_b, w->d3_b, 1);
   }
 #undef UP
-  // tensor-core images of the linear layers (fp16, pre-swizzled); shapes outside these bounds stay on the fp32 kernels
+  // tensor-core images of the linear layers (fp16, pre-swizzled); shapes outside these bounds stay on the fp32 kernels, and so
+  // do handles whose transformers all have fewer than ARX_TC_MIN_TUPLES tuples: with the attention on the fp32 kernels the
+  // fp16 support features alone would cost them the tolerance (1.0e-3 at T = 4, c = 4, N = 1)
+  bool enough_tuples = h->cfg.force_path == 2;
+  for (int i = 0; i < h->cfg.n_transformers; ++i) enough_tuples |= h->tr[i].N >= ARX_TC_MIN_TUPLES;
   h->tc_linears = false;
-  if (h->cfg.force_path != 1 && h->F == 256 && h->H <= 192 && h->J3 <= 128) {
+  if (h->cfg.force_path != 1 && enough_tuples && h->F == 256 && h->H <= 192 && h->J3 <= 128) {
     if ((rc = arx_tc_linear_prepare(h, h->tl_fc1, h->fc1_w, h->J3, h->fc1_b, h->H, h->J3, 192, st))) return rc;
     if ((rc = arx_tc_linear_prepare(h, h->tl_fc2, h->fc2_w, h->H, h->fc2_b, h->F, h->H, 256, st))) return rc;
     for (int i = 0; i < h->cfg.n_transformers; ++i) {
@@ -585,10 +589,10 @@ static int support_scratch_reserve(arx_handle *h, int way, SupportScratch *out) 
 static float accuracy_bound(const ArxTransformer &tr) {
   return tr.N < ARX_TC_FEW_TUPLES ? ARX_TC_ACCURACY_BOUND_FEW_TUPLES : ARX_TC_ACCURACY_BOUND;
 }
-// The tensor-core routes may score transformer `tr`: its LayerNorm affine is inside the accuracy bound, or the caller
-// forced them (force_path = 2) and accepts the reduced accuracy.
+// The tensor-core routes may score transformer `tr`: it has enough query tuples to average the operand rounding and its
+// LayerNorm affine is inside the accuracy bound, or the caller forced them (force_path = 2) and accepts the reduced accuracy.
 static bool tc_admitted(const arx_handle *h, const ArxTransformer &tr) {
-  return h->cfg.force_path == 2 || tr.softmax_bound < accuracy_bound(tr);
+  return h->cfg.force_path == 2 || (tr.N >= ARX_TC_MIN_TUPLES && tr.softmax_bound < accuracy_bound(tr));
 }
 
 // Which kernels score transformer `tr`:  the T=16 pair pipeline (arx_tc3.cu and friends: fused tuple images, head by
@@ -606,7 +610,9 @@ static ArxRoute support_route(const arx_handle *h, const ArxTransformer &tr) {
 }
 static void warn_fp32_fallback(arx_handle *h, int ti) {
   const ArxTransformer &tr = h->tr[ti];
-  if (h->cfg.force_path == 1 || (h->warned & (1u << ti)) || !arx_tcn_supported(h, tr) || tc_admitted(h, tr)) return;
+  // (fewer than ARX_TC_MIN_TUPLES query tuples take the fp32 kernels silently: at that size they cost next to nothing)
+  if (h->cfg.force_path == 1 || (h->warned & (1u << ti)) || !arx_tcn_supported(h, tr) || tr.N < ARX_TC_MIN_TUPLES || tc_admitted(h, tr))
+    return;
   h->warned |= 1u << ti;
   fprintf(stderr, "libarx: transformers[%d].norm_k has a LayerNorm affine outside the fp16 tensor-core bound (|S| <= %.1f; accuracy "
                   "bound %.1f, overflow bound %.1f): scoring on the fp32 CUDA-core kernels (about 30x slower) to stay within the "

@@ -24,6 +24,11 @@
 #define ARX_TC_ACCURACY_BOUND 19.0f
 #define ARX_TC_ACCURACY_BOUND_FEW_TUPLES 12.0f
 #define ARX_TC_FEW_TUPLES 120
+// Below this many query tuples nothing averages the operand rounding at all, whatever the affine: at gamma = 1 the tiled
+// route errs 1.05e-3 at N = 21 (T=7 pairs), 2.5e-3 at N = 10 and 1.3e-2 at N = 1, against 7.2e-4 at N = 28 (T=8 pairs)
+// (B200, 1000 W power limit; profiles/r04_few_tuples_accuracy.txt, DESIGN 4).  Such transformers score on the fp32 kernels by default, and a handle none of
+// whose transformers reaches it runs its front end (support side included) on the fp32 CUDA cores too.
+#define ARX_TC_MIN_TUPLES 28
 
 // A linear layer prepared for the tcgen05 GEMM: fp16 weight image [n_tiles][nk][BN x 64] + zero-padded bias
 struct ArxTcLinear {
