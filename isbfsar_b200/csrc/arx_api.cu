@@ -77,11 +77,9 @@ void free_support(arx_handle *h) {
   h->support_gen++;      // operand pointers change: cached score graphs no longer match
   for (int i = 0; i < h->cfg.n_transformers; ++i) {
     cudaFree(h->tr[i].ks); cudaFree(h->tr[i].vs);
-    cudaFree(h->tr[i].ks_img); cudaFree(h->tr[i].vs_img); cudaFree(h->tr[i].vs_img_bf); cudaFree(h->tr[i].uc_img);
-    cudaFree(h->tr[i].kc_tiles); cudaFree(h->tr[i].vct_tiles); cudaFree(h->tr[i].uc_tiles);
+    cudaFree(h->tr[i].kc_tiles); cudaFree(h->tr[i].vct_tiles); cudaFree(h->tr[i].uc_img); cudaFree(h->tr[i].uc_tiles);
     h->tr[i].ks = h->tr[i].vs = nullptr;
-    h->tr[i].ks_img = h->tr[i].vs_img = h->tr[i].vs_img_bf = h->tr[i].uc_img = nullptr;
-    h->tr[i].kc_tiles = h->tr[i].vct_tiles = h->tr[i].uc_tiles = nullptr;
+    h->tr[i].kc_tiles = h->tr[i].vct_tiles = h->tr[i].uc_img = h->tr[i].uc_tiles = nullptr;
     h->tr[i].route = ARX_ROUTE_NONE;
   }
   cudaFree(h->ss_feat);
@@ -624,20 +622,21 @@ static void warn_fp32_fallback(arx_handle *h, int ti) {
 static bool tiled_head(const arx_handle *h, int i) { return i == 0 && h->cfg.has_discriminator && arx_tcn_head_supported(h, h->tr[i]); }
 
 // Decides transformer i's route and builds the support operands it reads: the tuple tensors ks/vs from the per-frame
-// projections G (or, with G == nullptr, ks/vs are already in place: arx_import_support), the operand images and the
-// head's Uc of the pair pipeline, the class tiles of the tiled kernels.
+// projections G (or, with G == nullptr, ks/vs are already in place: arx_import_support), the Kc / Vc^T class tiles of
+// both tensor-core routes, the head's Uc of the route, and the tiled route's tables.
 static int support_operands(arx_handle *h, int i, const float *G, int way, cudaStream_t st) {
   ArxTransformer &tr = h->tr[i];
   tr.route = support_route(h, tr);
-  const bool imgs = tr.route == ARX_ROUTE_PAIR;
+  const bool pair = tr.route == ARX_ROUTE_PAIR, tiled = tr.route == ARX_ROUTE_TILED;
+  const bool fused_tiles = G && pair;              // k_support_build writes the single class tile of the pair pipeline
   int rc = ARX_OK;
-  if (G && h->D == 128) rc = arx_tc_support_build(h, tr, G, way, imgs, st);      // tuples + LayerNorm + operand images, one launch
+  if (G && h->D == 128) rc = arx_tc_support_build(h, tr, G, way, fused_tiles, st);      // tuples + LayerNorm (+ class tiles), one launch
   else if (G) rc = arx_fp32_build_tuples(h, tr, G, way, tr.ks, tr.vs, st);
-  else if (imgs) rc = arx_tc_prep_support(h, tr, way, st);
   if (rc) return rc;
-  if (imgs && i == 0 && h->cfg.has_discriminator && (rc = arx_tc2_support_uc(h, tr, way, st))) return rc;
-  if (tr.route == ARX_ROUTE_TILED) {
-    if ((rc = arx_tcn_prep_support(h, tr, way, tiled_head(h, i), st))) return rc;
+  if ((pair || tiled) && !fused_tiles && (rc = arx_tc_class_tiles(h, tr, way, st))) return rc;
+  if (pair && i == 0 && h->cfg.has_discriminator && (rc = arx_tc2_support_uc(h, tr, way, st))) return rc;
+  if (tiled) {
+    if ((rc = arx_tcn_prep_extras(h, tr, way, tiled_head(h, i), st))) return rc;
     h->tiles_gen[i] = h->support_seq + 1;
   }
   return ARX_OK;
@@ -663,24 +662,40 @@ static int support_from_features(arx_handle *h, const __half *f_img, const float
   return ARX_OK;
 }
 
-static int set_support_features(arx_handle *h, const float *feats_dev, int32_t way, int n_tr, cudaStream_t st) {
+// Support set of `way` classes from fp32 frame features (way, T, F) or poses (way, T, 3J) on the device, for transformers
+// [0, n_tr)
+static int set_support(arx_handle *h, const float *src_dev, bool is_features, int32_t way, int n_tr, cudaStream_t st) {
   int rc;
   if ((rc = support_alloc(h, way, n_tr, st))) return rc;
   SupportScratch sc;
   if ((rc = support_scratch_reserve(h, way, &sc))) return rc;
-  if ((rc = support_wait(h, st))) return rc;                       // a previous chain may still be writing ss_feat
-  if (feats_dev != h->ss_feat)
-    ARX_CUDA(h, cudaMemcpyAsync(h->ss_feat, feats_dev, (size_t)way * h->T * h->F * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  h->ss_feat_valid = true;
+  const int64_t rows = (int64_t)way * h->T;
+  if ((rc = support_wait(h, st))) return rc;                       // a previous chain may still be reading ss_feat / ss_poses
+  if (is_features) {
+    if (src_dev != h->ss_feat)
+      ARX_CUDA(h, cudaMemcpyAsync(h->ss_feat, src_dev, (size_t)rows * h->F * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    h->ss_feat_valid = true;
+  } else {
+    ARX_CUDA(h, cudaMemcpyAsync(h->ss_poses, src_dev, (size_t)rows * h->J3 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    h->ss_poses_valid = true;
+    if (h->tc_linears) {
+      h->ss_feat_valid = false;                                    // the fp32 'support_features' are derived lazily on request
+    } else {
+      // general path: arx_embed stages through the shared workspace, so it stays on the caller's stream
+      if ((rc = arx_embed(h, h->ss_poses, rows, h->ss_feat, st))) return rc;
+      h->ss_feat_valid = true;
+    }
+  }
   cudaStream_t ss;
   if ((rc = support_fork(h, st, &ss))) return rc;                  // the caller's buffer is not touched past this point
-  if (h->tc_linears) {
-    if ((rc = arx_tc_rows_to_img(h, h->ss_feat, false, h->F, h->F, (int64_t)way * h->T, sc.f_img, h->tr[0].tl_proj.nk,
-                                 h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
-      return rc;
-    rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
-  } else {
+  if (!h->tc_linears) {
     rc = support_from_features(h, nullptr, h->ss_feat, way, n_tr, sc.G, ss);
+  } else {
+    // same tensor-core pipeline as the query frames
+    const int nk = h->tr[0].tl_proj.nk, onehot = h->tr[0].table_in_gemm ? nk - 1 : -1;
+    rc = is_features ? arx_tc_rows_to_img(h, h->ss_feat, false, h->F, h->F, rows, sc.f_img, nk, onehot, ss)
+                     : embed_frames_tc(h, h->ss_poses, false, rows, sc.x_img, sc.h_img, sc.f_img, nk, onehot, ss);
+    if (rc == ARX_OK) rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
   }
   if (rc) return rc;
   return support_join_record(h);
@@ -689,42 +704,13 @@ static int set_support_features(arx_handle *h, const float *feats_dev, int32_t w
 int arx_set_support_features(arx_handle *h, const float *feats_dev, int32_t way, void *stream) {
   if (!h || !feats_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
   if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "set_support: weights not loaded");
-  return set_support_features(h, feats_dev, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
-}
-
-static int set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, int n_tr, cudaStream_t st) {
-  int rc;
-  if ((rc = support_alloc(h, way, n_tr, st))) return rc;
-  SupportScratch sc;
-  if ((rc = support_scratch_reserve(h, way, &sc))) return rc;
-  const int64_t rows = (int64_t)way * h->T;
-  if ((rc = support_wait(h, st))) return rc;                       // a previous chain may still be reading ss_poses
-  ARX_CUDA(h, cudaMemcpyAsync(h->ss_poses, poses_dev, (size_t)rows * h->J3 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  h->ss_poses_valid = true;
-  cudaStream_t ss;
-  if ((rc = support_fork(h, st, &ss))) return rc;                  // the caller's buffer is not touched past this point
-  if (h->tc_linears) {
-    // same tensor-core pipeline as the query frames; the fp32 'support_features' are derived lazily on request
-    h->ss_feat_valid = false;
-    if ((rc = embed_frames_tc(h, h->ss_poses, false, rows, sc.x_img, sc.h_img, sc.f_img, h->tr[0].tl_proj.nk,
-                              h->tr[0].table_in_gemm ? h->tr[0].tl_proj.nk - 1 : -1, ss)))
-      return rc;
-    rc = support_from_features(h, sc.f_img, nullptr, way, n_tr, sc.G, ss);
-  } else {
-    // general path: arx_embed stages through the shared workspace, so it stays on the caller's stream
-    if ((rc = arx_embed(h, h->ss_poses, rows, h->ss_feat, st))) return rc;
-    h->ss_feat_valid = true;
-    if ((rc = support_fork(h, st, &ss))) return rc;
-    rc = support_from_features(h, nullptr, h->ss_feat, way, n_tr, sc.G, ss);
-  }
-  if (rc) return rc;
-  return support_join_record(h);
+  return set_support(h, feats_dev, true, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
 }
 
 int arx_set_support_poses(arx_handle *h, const float *poses_dev, int32_t way, void *stream) {
   if (!h || !poses_dev || way < 1) return arx_fail(h, ARX_ERR_INVALID, "set_support: bad argument");
   if (!h->weights_loaded) return arx_fail(h, ARX_ERR_STATE, "set_support: weights not loaded");
-  return set_support_poses(h, poses_dev, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
+  return set_support(h, poses_dev, false, way, h->cfg.n_transformers, static_cast<cudaStream_t>(stream));
 }
 
 static int support_features_materialise(arx_handle *h, cudaStream_t st) {
@@ -1070,9 +1056,11 @@ static int score_gen3(arx_handle *h, int ti, const Query &q, int64_t n_windows, 
       if ((rc = prof_mark(h, 1, st))) return rc;
       if ((rc = arx_tcp_linear_chunked(h, tr.tl_proj, w.f_img, f_nk, rows, w.G, sms, st))) return rc;
       if ((rc = prof_mark(h, 2, st))) return rc;
-      if ((h->tc_variant & 64) == 0 && (rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, sms, st))) return rc;   // bit 6: timing only
       if (disc) {
-        // only the head pass reads these 32 columns: run them on a second stream, beside the tuple build + attention
+        // only the head pass reads these 32 columns: run them on a second stream, beside the tuple build.  Forked before the
+        // tuple build, not after it: a GEMM that starts when the attention kernel becomes ready holds every SM with its CTAs,
+        // and the persistent attention CTAs, each with a fixed share of the windows, start one by one as SMs drain (B200, 1000 W
+        // power limit: the step took 3-4 us longer whenever the support chain joined before the tuple build ended)
         const bool aux = (h->tc_variant & 2048) == 0 && !h->prof_on && !sg;      // (a graph segment must end joined)
         cudaStream_t us = st;
         if (aux) {
@@ -1088,6 +1076,7 @@ static int score_gen3(arx_handle *h, int ti, const Query &q, int64_t n_windows, 
         if ((rc = arx_tc_linear_f32_small(h, tr.tl_uab, w.f_img, f_nk, rows, w.uab, 32, tr.tcomp, h->T, us))) return rc;
         if (aux) { ARX_CUDA(h, cudaEventRecord(h->ev_aux_done, us)); aux_pending = true; }
       }
+      if ((h->tc_variant & 64) == 0 && (rc = arx_tuple_img(h, tr, w.G, g_ld / 32, n, w.kq_img, alpha, sms, st))) return rc;   // bit 6: timing only
       return ARX_OK;
     });
     if (rc) return rc;
@@ -1208,16 +1197,12 @@ int arx_score_episodes(arx_handle *h, const float *support_dev, int32_t is_featu
   if (!h->cfg.has_discriminator) is_true_dev = nullptr;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const size_t per_class = (size_t)h->T * (is_features ? h->F : h->J3);
-  // support operands of transformers[0] only: episodes are scored by it alone (model.py:320)
-  auto set_support = [&](int64_t e0, int64_t n_classes) -> int {
-    const float *sup = support_dev + (size_t)e0 * way * per_class;
-    return is_features ? set_support_features(h, sup, (int32_t)n_classes, 1, st) : set_support_poses(h, sup, (int32_t)n_classes, 1, st);
-  };
   const Query q{query_dev, Query::WINDOWS, false};
   // episodes [e0, e0 + m) against a pool of m*way support classes (ep_way = way), or one at a time against a support set of
-  // their own (ep_way = 0: the same kernels as set_support + arx_score)
+  // their own (ep_way = 0: the same kernels as set_support + arx_score).  Support operands of transformers[0] only: episodes
+  // are scored by it alone (model.py:320)
   auto score = [&](int64_t e0, int64_t m, int ep_way) -> int {
-    const int rc = set_support(e0, m * way);
+    const int rc = set_support(h, support_dev + (size_t)e0 * way * per_class, is_features != 0, (int32_t)(m * way), 1, st);
     if (rc) return rc;
     return score_impl(h, 0, {q.at(h, e0), Query::WINDOWS, false}, m,
                       {logits_dev + e0 * way, is_true_dev ? is_true_dev + e0 : nullptr, chosen_dev ? chosen_dev + e0 : nullptr},
@@ -1499,10 +1484,12 @@ int arx_stream_push(arx_handle *h, const float *frame_host, float *result_host, 
       ARX_CUDA(h, cudaMalloc(&s.ws, need));
       s.ws_bytes = need;
     }
-    // the tiled class operands (the T=16 pair pipeline of arx_score builds its own images): from the fp32 tuple tensors
+    // the class tiles come with every tensor-core support set; what the T=16 pair pipeline does not build are the tiled
+    // route's tables and, with the discriminator, its Uc tiles.  The class tiles are not rewritten here: an arx_score on
+    // another stream may be reading them.
     if (h->tiles_gen[0] != h->support_seq + 1) {
       if ((rc = support_wait(h, s.st))) return rc;
-      if ((rc = arx_tcn_prep_support(h, tr, way, disc, s.st))) return rc;
+      if ((rc = arx_tcn_prep_extras(h, tr, way, disc, s.st))) return rc;
       h->tiles_gen[0] = h->support_seq + 1;
     }
     s.way = way; s.sgen = h->support_seq; s.wgen = h->weights_gen;

@@ -62,17 +62,17 @@ struct ArxTransformer {
   ArxRoute route = ARX_ROUTE_NONE;   // the route the support operands below were built for
   // support operands, fp32 generic path: (W,N,D) each
   float *ks = nullptr, *vs = nullptr;
-  // support operands, tcgen05 path: fp16 UMMA smem images, see arx_tc.cu
-  __half *ks_img = nullptr, *vs_img = nullptr;
-  __half *vs_img_bf = nullptr;   // Vc^T as bf16 (prototype MMA of arx_tc2.cu)
+  // class operands of both tensor-core routes (arx_tc.cu): [way_cap][Npad/128] 32 KB K-major SW128 tiles, Kc fp16 (rows =
+  // support tuples) and Vc^T bf16 (rows = d); the T=16 pair pipeline has one tile per class
+  __half *kc_tiles = nullptr, *vct_tiles = nullptr;
   float softmax_bound = 0.f; // static |S| bound from LayerNorm affine (SURVEY 7.2-1)
   ArxTcLinear tl_proj;       // K/V projection (2cD x F) on tensor cores
   ArxTcLinear tl_proj_nt;    // the same without the positional-table columns (frame streams: the table is added per window position)
   ArxTcLinear tl_uab;        // 32 composite columns Wdr.Wv of the second-generation head pass
   float *wc = nullptr, *tcomp = nullptr;   // composite weights (32,F) and table (T,32)
-  __half *uc_img = nullptr;  // per class Wdr.Vc^T (16 x 128 fp16 B operand)
-  // tiled operands of the any-N kernel (arx_tcn.cu): [way][Npad/128] 32 KB tiles
-  __half *kc_tiles = nullptr, *vct_tiles = nullptr, *uc_tiles = nullptr;
+  __half *uc_img = nullptr;  // pair pipeline's head: per class Wdr.Vc^T (16 x 128 fp16 B operand)
+  // operands of the tiled any-N kernels only (arx_tcn.cu)
+  __half *uc_tiles = nullptr;       // head: per class Wdr.Vc^T, [way_cap][Npad/128] 32 KB bf16 tiles
   uint32_t *tup_packed = nullptr;   // (N) tuple frames packed one byte each
   __half *sel_tiles = nullptr;      // one-hot frame-selection operand of every query tile (selection MMA of arx_tcn.cu)
 };
@@ -191,7 +191,7 @@ struct arx_handle {
   float *zscratch = nullptr;        // softmax normaliser partials of the tiled attention kernel (arx_tcn.cu), per CTA
   size_t zscratch_bytes = 0;
   ArxStream stream;
-  uint64_t tiles_gen[ARX_MAX_TRANSFORMERS] = {0, 0, 0, 0};   // support generation the tiled operands were built for (+1)
+  uint64_t tiles_gen[ARX_MAX_TRANSFORMERS] = {0, 0, 0, 0};   // support generation the tiled route's extras (tables, Uc tiles) were built for (+1)
   float mlp_bias_host[192 + 256] = {};   // host copies of the (zero padded) fc1 / fc2 biases: kernel-parameter operands of k_mlp_p
   bool mlp_bias_host_ok = false;
   bool support_inflight = false;    // a support chain was forked onto the side stream and no scoring pass has joined it yet
@@ -265,8 +265,12 @@ int arx_fp32_attention(arx_handle *h, const ArxTransformer &tr, const float *Kq,
 
 // ---- tcgen05 kernels (arx_tc.cu) -------------------------------------------------
 bool arx_tc_supported(const arx_handle *h, const ArxTransformer &tr);
-int arx_tc_prep_support(arx_handle *h, ArxTransformer &tr, int way, cudaStream_t st);
-int arx_tc_support_build(arx_handle *h, ArxTransformer &tr, const float *G, int way, bool with_images, cudaStream_t st);
+// Kc / Vc^T class tiles of `way` classes from the fp32 tuple tensors ks / vs
+int arx_tc_class_tiles(arx_handle *h, ArxTransformer &tr, int way, cudaStream_t st);
+// ks / vs (and with_tiles: the single class tile of every class) from the per-frame projections G, one launch
+int arx_tc_support_build(arx_handle *h, ArxTransformer &tr, const float *G, int way, bool with_tiles, cudaStream_t st);
+// logits (n_win, way) and chosen (n_win) from the squared-distance partials (n_win*way, 4) of either tensor-core route
+int arx_tc_finish(arx_handle *h, const float *partial, float *logits, int32_t *chosen, int64_t n_win, int way, int N, bool pdl, cudaStream_t st);
 int arx_tc_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_img, const float *G, int64_t n_win, int way, float *partial,
                      float *logits, int32_t *chosen, int g_ld, int g_voff, bool g_chunked, bool episodes, cudaStream_t st);
 
@@ -337,7 +341,8 @@ bool arx_tcn_needs_rowmax(const ArxTransformer &tr);
 bool arx_tcn_head_supported(const arx_handle *h, const ArxTransformer &tr);
 // columns per frame part of the head table UAB (row stride 2x this): 32 for T <= 32, 64 above
 int arx_tcn_head_cols(int T);
-int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st);
+// the tiled route's own support-side operands: packed tuples and selection tiles (once per handle), with_head the Uc tiles
+int arx_tcn_prep_extras(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st);
 int arx_tcn_prep_query(arx_handle *h, const ArxTransformer &tr, const float *G, int ldg, int64_t n_win, __half *kq_tiles, cudaStream_t st);
 int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_tiles, const float *G, int ldg, int64_t n_win, int way,
                       float *partial, float *logits, int32_t *chosen, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st);

@@ -1,9 +1,10 @@
 // Thin inline-PTX wrappers for the sm_100a features the tensor-core kernels use:
 // mbarrier, bulk async copy (TMA engine, 1-D), tcgen05 (alloc / mma / commit / ld / fences),
-// and the shared-memory matrix / instruction descriptors of tcgen05.mma.
+// the shared-memory matrix / instruction descriptors of tcgen05.mma, and the SW128 operand-tile format the kernels share.
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 
 namespace ptx {
@@ -150,6 +151,20 @@ __host__ __device__ constexpr uint32_t idesc_bf16(uint32_t M, uint32_t N, uint32
 // row r at r*128, 16-byte chunk j stored at position j ^ (r & 7).
 __host__ __device__ constexpr uint32_t sw128_offset(uint32_t row, uint32_t col /* 0..63 */) {
   return row * 128u + ((((col >> 3) ^ (row & 7u)) << 4) | ((col & 7u) << 1));
+}
+
+// The 128 x 128 operand tile of the attention kernels (Kq, Kc, Vc^T, Uc): two 16 KB SW128 sub-tiles of 64 columns
+constexpr int DD = 128;
+constexpr uint32_t IMG_BYTES = 128 * DD * 2;
+constexpr uint32_t SUB_BYTES = 128 * 64 * 2;
+
+__device__ __forceinline__ uint32_t pack_half2(float lo, float hi) {
+  __half2 h = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<uint32_t *>(&h);
+}
+__device__ __forceinline__ uint32_t pack_bf162(float lo, float hi) {
+  __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<uint32_t *>(&h);
 }
 
 }  // namespace ptx

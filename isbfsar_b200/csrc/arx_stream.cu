@@ -6,8 +6,10 @@
 // encoding through the projection, arx_load_weights), and the window is scored by the tiled tcgen05 kernels.
 // Three small kernels live here; the orchestration (CUDA graph per frame, pinned staging) is in arx_api.cu.
 #include "arx_internal.cuh"
+#include "arx_ptx.cuh"
 
 namespace {
+using namespace ptx;
 
 constexpr int SF_THREADS = 512;
 
@@ -64,13 +66,6 @@ __global__ void __launch_bounds__(SF_THREADS) k_stream_frame(const float *__rest
   warp_matvec4(wp, F, nullptr, f_s, ring + (size_t)(*slot_next) * NO, o0, o1, F, false);
 }
 
-__device__ __forceinline__ uint32_t pack_half2(float lo, float hi) {
-  __half2 h = __floats2half2_rn(lo, hi);
-  return *reinterpret_cast<uint32_t *>(&h);
-}
-__host__ __device__ constexpr uint32_t sw128(uint32_t row, uint32_t col) {          // byte offset in a [rows x 64]-fp16 K-major SW128 sub-tile
-  return row * 128u + ((((col >> 3) ^ (row & 7u)) << 4) | ((col & 7u) << 1));
-}
 
 // Window formation + query tiles in one launch.  The window's frame t lives in ring slot (newest + 1 + t) mod T (newest =
 // *slot_next, just written); its per-frame projections are ring + table[t] (table = positional encoding through the
@@ -87,7 +82,7 @@ __global__ void __launch_bounds__(256) k_stream_tiles(const float *__restrict__ 
   }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int q = blockIdx.x * 8 + warp;                       // row of the tiled image: tile q / 128, row q % 128
-  uint8_t *out = reinterpret_cast<uint8_t *>(kq) + (size_t)(q >> 7) * 32768;
+  uint8_t *out = reinterpret_cast<uint8_t *>(kq) + (size_t)(q >> 7) * IMG_BYTES;
   const int r = q & 127, d0 = lane * 4;
   uint2 packed = make_uint2(0u, 0u);
   if (q < N) {
@@ -112,7 +107,7 @@ __global__ void __launch_bounds__(256) k_stream_tiles(const float *__restrict__ 
     packed.x = pack_half2((dl.x * rstd * g.x + be.x) * alpha, (dl.y * rstd * g.y + be.y) * alpha);
     packed.y = pack_half2((dl.z * rstd * g.z + be.z) * alpha, (dl.w * rstd * g.w + be.w) * alpha);
   }
-  *reinterpret_cast<uint2 *>(out + (d0 >> 6) * 16384 + sw128(r, d0 & 63)) = packed;
+  *reinterpret_cast<uint2 *>(out + (d0 >> 6) * SUB_BYTES + sw128_offset(r, d0 & 63)) = packed;
 }
 
 // logits / argmax of ONE window from the distance partials (model.py:131-135,323: first maximum wins), then discriminator

@@ -9,10 +9,6 @@
 namespace {
 using namespace ptx;
 
-constexpr int TILE = 128;
-constexpr int DD = 128;
-constexpr uint32_t IMG_BYTES = TILE * DD * 2;
-constexpr uint32_t SUB_BYTES = TILE * 64 * 2;
 constexpr int NTHREADS2 = 512;
 
 }  // namespace
@@ -23,10 +19,6 @@ __device__ __forceinline__ uint32_t ex2_bits(uint32_t x) {
   uint32_t y;
   asm volatile("ex2.approx.ftz.f32 %0, %1;" : "=r"(y) : "r"(x));
   return y;
-}
-__device__ __forceinline__ uint32_t pack_half2(float lo, float hi) {
-  __half2 h = __floats2half2_rn(lo, hi);
-  return *reinterpret_cast<uint32_t *>(&h);
 }
 
 template <int... Is> __device__ __forceinline__ void zero_pads(uint32_t (&r)[128], std::integer_sequence<int, Is...>) {
@@ -384,7 +376,7 @@ int arx_tc2_support_uc(arx_handle *h, ArxTransformer &tr, int way, cudaStream_t 
 int arx_tc2_head_launch(arx_handle *h, const ArxTransformer &tr, const __half *kq_img, const float *uab, int64_t n_win, const int32_t *chosen,
                         __half *y_img, int y_nk, int cls_stride, cudaStream_t st) {
   Head2Params p{};
-  p.kq_img = kq_img; p.kc_img = tr.ks_img; p.uc_img = tr.uc_img; p.uab = uab; p.chosen = chosen; p.y_img = y_img; p.n_win = (int)n_win; p.y_nk = y_nk; p.cls_stride = cls_stride;
+  p.kq_img = kq_img; p.kc_img = tr.kc_tiles; p.uc_img = tr.uc_img; p.uab = uab; p.chosen = chosen; p.y_img = y_img; p.n_win = (int)n_win; p.y_nk = y_nk; p.cls_stride = cls_stride;
   p.l2_ahead = (h->tc_variant & 16384) ? 1 << 30 : 4;
   p.trace = h->trace_sel == 3 ? h->trace_buf : nullptr;
   const int grid = n_win < h->sm_count ? (int)n_win : h->sm_count;

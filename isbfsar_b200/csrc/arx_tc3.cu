@@ -17,9 +17,6 @@
 namespace {
 using namespace ptx;
 
-constexpr int DD = 128;
-constexpr uint32_t IMG_BYTES = 128 * DD * 2;
-constexpr uint32_t SUB_BYTES = 128 * 64 * 2;
 constexpr int NTHREADS3 = 512;
 
 constexpr uint32_t OFF_KQ = 0;                       // 64 KB: [sub0: w0 rows | w1 rows][sub1: w0 rows | w1 rows]
@@ -387,7 +384,7 @@ __global__ void __launch_bounds__(NTHREADS3, 1) k_attn_tc3(const Attn3Params p) 
 int arx_tc3_attention_launch(arx_handle *h, const ArxTransformer &tr, const __half *kq_img, const float *G, int64_t n_win, int way,
                              float *partial, int g_ld, int g_voff, bool g_chunked, bool episodes, cudaStream_t st) {
   Attn3Params p{};
-  p.kq_img = kq_img; p.kc_img = tr.ks_img; p.vct_img = tr.vs_img_bf; p.G = G; p.partial = partial;
+  p.kq_img = kq_img; p.kc_img = tr.kc_tiles; p.vct_img = tr.vct_tiles; p.G = G; p.partial = partial;
   p.n_win = (int)n_win; p.way = way; p.ldg = g_ld; p.voff = g_voff; p.trace = h->trace_sel == 1 ? h->trace_buf : nullptr;
   p.gchunk = g_chunked ? 1 : 0;
   p.ep = episodes ? 1 : 0;

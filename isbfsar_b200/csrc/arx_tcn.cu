@@ -30,17 +30,15 @@
 // [cls_base + w*way, cls_base + (w+1)*way) of one pool of class tiles; the query side and the head are per window as always.
 // Work unit = (window, class), round-robin over one persistent CTA per SM; 16 warps, warp-specialised; every
 // mbarrier wait carries a watchdog (a protocol bug traps instead of hanging the GPU).
+// The Kc / Vc^T class tiles are those of arx_tc.cu, shared with the T=16 pair pipeline; this file builds the tiled route's
+// own operands: query tiles, the selection operands, the head's Uc tiles and head table.
 #include "arx_internal.cuh"
 #include "arx_ptx.cuh"
-#include <cuda_bf16.h>
 #include <stdlib.h>
 
 namespace {
 using namespace ptx;
 
-constexpr int DD = 128;
-constexpr uint32_t IMG_BYTES = 128 * DD * 2;
-constexpr uint32_t SUB_BYTES = 128 * 64 * 2;
 constexpr int NTHREADS = 512;
 
 constexpr uint32_t OFF_KQ = 0;                       // 64 KB: [sub0: t0 rows | t1 rows][sub1: t0 rows | t1 rows]
@@ -547,16 +545,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_attn_tcn(const AttnNParams p) {
   if (warp == 3) { tc_fence_after(); tmem_dealloc(tmem, 512); }
 }
 
-// ---- operand image builders (tiled) ---------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t pack_half2(float lo, float hi) {
-  __half2 h = __floats2half2_rn(lo, hi);
-  return *reinterpret_cast<uint32_t *>(&h);
-}
-__device__ __forceinline__ uint32_t pack_bf162(float lo, float hi) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t *>(&h);
-}
-
+// ---- operand image builders (tiled; the Kc / Vc^T class tiles are built in arx_tc.cu) --------------------------------
 // Query K tiles: one warp per tuple row; K = LayerNorm(sum_p Gk_p[frame_p]) * alpha -> fp16, K-major SW128.  grid (n_win, nq)
 __global__ void __launch_bounds__(256) k_prep_kq_tiles(const float *__restrict__ G, const uint32_t *__restrict__ tup, const float *__restrict__ ln_g,
                                                        const float *__restrict__ ln_b, __half *__restrict__ img, int T, int c, int N, int nq, int ldg,
@@ -592,46 +581,6 @@ __global__ void __launch_bounds__(256) k_prep_kq_tiles(const float *__restrict__
       packed.y = pack_half2((dl.z * rstd * g.z + be.z) * alpha, (dl.w * rstd * g.w + be.w) * alpha);
     }
     *reinterpret_cast<uint2 *>(out + (d0 >> 6) * SUB_BYTES + sw128_offset(r, d0 & 63)) = packed;
-  }
-}
-
-// Support K tiles from fp32 ks (way, N, D): rows = s, cols = d.  grid (way, ns)
-__global__ void __launch_bounds__(256) k_prep_kc_tiles(const float *__restrict__ ks, __half *__restrict__ img, int N, int ns) {
-  const size_t cls = blockIdx.x;
-  const int st = blockIdx.y;
-  const float *k = ks + cls * (size_t)N * DD;
-  uint8_t *out = reinterpret_cast<uint8_t *>(img) + (cls * ns + st) * IMG_BYTES;
-  for (int e = threadIdx.x; e < 128 * 16; e += 256) {
-    const int dc = e & 15, r = e >> 4, s = st * 128 + r;
-    uint4 pk = make_uint4(0, 0, 0, 0);
-    if (s < N) {
-      const float4 x0 = *reinterpret_cast<const float4 *>(k + (size_t)s * DD + dc * 8);
-      const float4 x1 = *reinterpret_cast<const float4 *>(k + (size_t)s * DD + dc * 8 + 4);
-      pk.x = pack_half2(x0.x, x0.y); pk.y = pack_half2(x0.z, x0.w); pk.z = pack_half2(x1.x, x1.y); pk.w = pack_half2(x1.z, x1.w);
-    }
-    const int d0 = dc * 8;
-    *reinterpret_cast<uint4 *>(out + (d0 >> 6) * SUB_BYTES + sw128_offset(r, d0 & 63)) = pk;
-  }
-}
-
-// Support V^T tiles (bf16): rows = d, cols = support tuple of tile st (zero beyond N).  grid (way, ns)
-__global__ void __launch_bounds__(256) k_prep_vct_tiles(const float *__restrict__ vs, __half *__restrict__ img, int N, int ns) {
-  const size_t cls = blockIdx.x;
-  const int st = blockIdx.y;
-  const float *v = vs + cls * (size_t)N * DD;
-  uint8_t *out = reinterpret_cast<uint8_t *>(img) + (cls * ns + st) * IMG_BYTES;
-  for (int e = threadIdx.x; e < DD * 16; e += 256) {
-    const int d = e & 127, sc = e >> 7;          // consecutive threads -> consecutive d (coalesced reads)
-    float x[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int s = st * 128 + sc * 8 + i;
-      x[i] = s < N ? v[(size_t)s * DD + d] : 0.f;
-    }
-    uint4 pk;
-    pk.x = pack_bf162(x[0], x[1]); pk.y = pack_bf162(x[2], x[3]); pk.z = pack_bf162(x[4], x[5]); pk.w = pack_bf162(x[6], x[7]);
-    const int s0 = sc * 8;
-    *reinterpret_cast<uint4 *>(out + (s0 >> 6) * SUB_BYTES + sw128_offset(d, s0 & 63)) = pk;
   }
 }
 
@@ -771,21 +720,6 @@ __global__ void k_pack_tuples(const int32_t *__restrict__ tuples, uint32_t *__re
   out[q] = v;
 }
 
-__global__ void k_finish_n(const float *__restrict__ partial, float *__restrict__ logits, int32_t *__restrict__ chosen, int64_t n_win, int way,
-                           int N) {
-  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= n_win) return;
-  float best = -INFINITY;
-  int bi = 0;
-  for (int c = 0; c < way; ++c) {
-    const float4 t = *reinterpret_cast<const float4 *>(partial + (b * way + c) * 4);
-    const float lg = -(((t.x + t.y) + (t.z + t.w)) / (float)N);
-    logits[b * way + c] = lg;
-    if (lg > best) { best = lg; bi = c; }        // strict '>': the first maximum wins (torch.argmax, model.py:323)
-  }
-  if (chosen) chosen[b] = bi;
-}
-
 }  // namespace
 
 bool arx_tcn_supported(const arx_handle *h, const ArxTransformer &tr) {
@@ -797,13 +731,8 @@ int arx_tcn_head_cols(int T) { return T <= 32 ? 32 : 64; }
 // variant runs.  Only force_path = 2 gets there: by default weights past the tighter accuracy bound score on the fp32 kernels.
 bool arx_tcn_needs_rowmax(const ArxTransformer &tr) { return !(tr.softmax_bound * ARX_SOFTMAX_LOG2E < 100.0f); }
 
-int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st) {
+int arx_tcn_prep_extras(arx_handle *h, ArxTransformer &tr, int way, bool with_head, cudaStream_t st) {
   const int ns = tr.Npad / 128;
-  const size_t bytes = (size_t)h->way_cap * ns * IMG_BYTES;
-  if (!tr.kc_tiles) {
-    ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.kc_tiles), bytes));
-    ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.vct_tiles), bytes));
-  }
   if (!tr.tup_packed) {
     ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.tup_packed), (size_t)tr.N * sizeof(uint32_t)));
     k_pack_tuples<<<(tr.N + 127) / 128, 128, 0, st>>>(tr.tuples, tr.tup_packed, tr.N, tr.c);
@@ -813,12 +742,8 @@ int arx_tcn_prep_support(arx_handle *h, ArxTransformer &tr, int way, bool with_h
     k_prep_sel_tiles<<<dim3(ns, nsel), 256, 0, st>>>(tr.tup_packed, tr.N, h->T, tr.c, nsel, tr.sel_tiles);
     ARX_LAUNCH_CHECK(h);
   }
-  k_prep_kc_tiles<<<dim3(way, ns), 256, 0, st>>>(tr.ks, tr.kc_tiles, tr.N, ns);
-  ARX_LAUNCH_CHECK(h);
-  k_prep_vct_tiles<<<dim3(way, ns), 256, 0, st>>>(tr.vs, tr.vct_tiles, tr.N, ns);
-  ARX_LAUNCH_CHECK(h);
   if (with_head) {
-    if (!tr.uc_tiles) ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.uc_tiles), bytes));
+    if (!tr.uc_tiles) ARX_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&tr.uc_tiles), (size_t)h->way_cap * ns * IMG_BYTES));
     auto kern = arx_tcn_head_cols(h->T) == 32 ? k_prep_uc_tiles<32> : k_prep_uc_tiles<64>;
     kern<<<dim3(way, ns), 128, h->T * 128 * sizeof(float), st>>>(tr.vs, h->dr_w, tr.uc_tiles, tr.N, ns, h->T);
     ARX_LAUNCH_CHECK(h);
@@ -925,9 +850,7 @@ int arx_tcn_attention(arx_handle *h, const ArxTransformer &tr, const __half *kq_
                       float *partial, float *logits, int32_t *chosen, __half *vq_ws, bool episodes, int64_t cls_base, cudaStream_t st) {
   int rc = arx_tcn_attention_partial(h, tr, kq_tiles, G, ldg, n_win, way, partial, vq_ws, episodes, cls_base, st);
   if (rc) return rc;
-  k_finish_n<<<(unsigned)((n_win + 127) / 128), 128, 0, st>>>(partial, logits, chosen, n_win, way, tr.N);
-  ARX_LAUNCH_CHECK(h);
-  return ARX_OK;
+  return arx_tc_finish(h, partial, logits, chosen, n_win, way, tr.N, false, st);
 }
 
 // streaming: the head input of EVERY class of ONE window at once (y_all (way, N*L) fp32), so that it can run beside the main

@@ -523,6 +523,33 @@ def test_export_import_support_roundtrip():
         m2.support_features()
 
 
+def test_pair_route_class_tiles_shared_with_stream_push():
+    """At T=16 pairs with the discriminator the pair pipeline (arx_score) and the resident streaming scorer read the same
+    Kc / Vc^T class tiles.  A handle whose tiles were built from an imported support set (k_prep_kc_tiles /
+    k_prep_vct_tiles) scores and streams bit-identically to the handle whose fused support build wrote them, and scores
+    after pushing frames equal those before.  (A rewrite of the tiles with the same bytes would pass the latter: it guards
+    against stream_push changing them, not against a race.)"""
+    cfg = Cfg()
+    m1, _ = make_model(cfg, 0)
+    m2, _ = make_model(cfg, 0)
+    support, labels, query, _ = make_episode(cfg, 200, 111, "structured")
+    Q = torch.from_numpy(query).cuda()
+    m1.set_support(poses=torch.from_numpy(support[0]).cuda())
+    m2.import_support(m1.export_support(), 5)
+    lo, it = m1.score(Q)
+    assert m1.last_path() == 2
+    frames = (0.17 * np.random.default_rng(5).standard_normal((20, 90))).astype(np.float32)
+    for f in frames:
+        p1, t1, v1 = m1.stream_push(f)
+        p2, t2, v2 = m2.stream_push(f)
+        assert np.array_equal(p1, p2) and np.array_equal(t1, t2) and v1 == v2
+    assert v1 and m1.last_path() == 3
+    lo1, it1 = m1.score(Q)
+    lo2, it2 = m2.score(Q)
+    assert m1.last_path() == 2 and m2.last_path() == 2
+    assert torch.equal(lo, lo1) and torch.equal(it, it1) and torch.equal(lo, lo2) and torch.equal(it, it2)
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 # Round 2: the acceptance criteria at FULL size (SURVEY 8d), ties, hooks, cache round trip, episodes, API races
 # ----------------------------------------------------------------------------------------------------------------------
